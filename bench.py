@@ -72,7 +72,11 @@ def parse(argv=None):
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the short runs of BASELINE configs[2..4]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the row batch of the last timed step as DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.cap is None:
         # slot capacity per env and species: large enough that no env of the rollout ever fills it (`status_envs` 0 —
         # a full list would suppress births the reference allows); measured maxima: BASE 26 / 83, ECO 13 / 65,
@@ -244,6 +248,61 @@ def load_peak():
         return 6650.0, "fallback 6650 GB/s (of fallback)"
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(pipe, out_dir, stats):
+    """Writes what the timed path handed out in its last step, as out_dir/<name>.npy (integers as float64, observations and
+    rewards as float32), so that two builds run with the same arguments can be compared array for array:
+
+      stats                                 the statistics vector of the timed steps (config.STAT_NAMES)
+      env_flags, env_status, env_step, env_count
+      {pred,prey}_old_off, _new_off, _new_cnt  row offsets per env (new_off is 0 where new_cnt is 0, as include/ppg.h leaves it undefined)
+      {pred,prey}_row_index                 which valid rows the per-row arrays below hold
+      {pred,prey}_obs, _reward, _row_env, _row_agent, _flags
+
+    With several env groups every array is the concatenation of the groups' arrays in group order (offsets and row_env stay
+    relative to the group), and a row index counts the valid rows of all groups in that order.  When the valid rows do not fit
+    in DUMP_BYTES, the per-row arrays hold a sample: a sorted draw without replacement from a fixed-seed generator."""
+    import numpy as np
+    import torch
+
+    outs = [e.out for e in pipe.envs]
+    f64 = lambda ts: torch.cat([t.to(torch.float64) for t in ts]).cpu().numpy()  # noqa: E731
+    arrays = {"stats": stats.to(torch.float64).cpu().numpy()}
+    for name in ("env_flags", "env_status", "env_step", "env_count"):
+        arrays[name] = f64([getattr(o, name) for o in outs])
+    for s, sp in enumerate(("pred", "prey")):
+        arrays[f"{sp}_old_off"] = f64([o.old_off[s] for o in outs])
+        arrays[f"{sp}_new_off"] = f64([torch.where(o.new_cnt[s] > 0, o.new_off[s], 0) for o in outs])
+        arrays[f"{sp}_new_cnt"] = f64([o.new_cnt[s] for o in outs])
+    budget = (DUMP_BYTES - sum(a.nbytes for a in arrays.values())) // 2  # per species
+    for s, sp in enumerate(("pred", "prey")):
+        n = [o.counts()[s] for o in outs]
+        total = sum(n)
+        row_bytes = 4 * pipe.C * pipe.R[s] ** 2 + 4 + 4 * 8  # obs + reward (f32), row index, env, agent, flags (f64)
+        m = min(total, budget // row_bytes)
+        idx = np.arange(total) if m == total else np.sort(np.random.default_rng(s).choice(total, m, replace=False))
+        parts = {k: [] for k in ("obs", "reward", "row_env", "row_agent", "flags")}
+        first = 0
+        for o, k in zip(outs, n):
+            sel = idx[(idx >= first) & (idx < first + k)] - first
+            sel = torch.from_numpy(sel).to(o.obs[s].device)
+            for name in parts:
+                parts[name].append(getattr(o, name)[s].index_select(0, sel))
+            first += k
+        arrays[f"{sp}_row_index"] = idx.astype(np.float64)
+        arrays[f"{sp}_obs"] = torch.cat(parts["obs"]).cpu().numpy()
+        arrays[f"{sp}_reward"] = torch.cat(parts["reward"]).cpu().numpy()
+        for name in ("row_env", "row_agent", "flags"):
+            arrays[f"{sp}_{name}"] = f64(parts[name])
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(arrays)
+
+
 class Rollout:
     """`groups` handles of envs / groups env instances each, every group on its own CUDA stream."""
 
@@ -310,6 +369,8 @@ def measure(args, rank, local_rank, world, K, W, full):
     clocks = sampler.stop() if full else None
     launches = ro.launches() - launches0
     stats1 = ro.stats()
+    if full and args.dump_outputs and rank == 0:
+        dump_outputs(pipe, args.dump_outputs, stats1 - stats0)
     d = (stats1 - stats0).to(torch.float64)  # this rank's env/agent steps, rows, births... in the timed region
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
