@@ -393,6 +393,21 @@ int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, 
                  double* energy_pred, int32_t* ids_prey, int32_t* xy_prey, double* energy_prey,
                  int32_t* xy_grass, double* energy_grass);
 
+/* `grid_world_state` (BASE:311; ECO, STAG and the trait variants alike) of the envs [env_begin, env_begin + n_envs):
+ * out (DEVICE, [n_envs][num_obs_channels][grid_size][grid_size] fp32, index order [c][x][y] like the rows) receives the
+ * grid as the reference holds it after step(), rounded to fp32 the way the observation rows round it (BASE keeps its
+ * grid in float64: this is its fp32 rounding).  Channels as in the rows: BASE wall, predator, prey, grass; ECO
+ * family predator, prey, grass; STAG walls, predators, mammoths, rabbits, grass.  ECO's own-speed plane is row-only.
+ * The result is the world of the handle's last output (ppg_step / full ppg_reset): for an env reset by that call
+ * (autoreset, scheduled masked reset, full reset) the world after the reset; for an env whose episode ended in it the
+ * world after the final step; an idle env (autoreset off) keeps the world of its final step.  A masked ppg_reset only
+ * schedules resets and changes nothing here.  Stream-ordered, no synchronisation; one kernel launch.
+ * PPG_ERR_INVALID: NULL handle or out, n_envs < 1 or the range not inside [0, n_envs of the handle).
+ * PPG_ERR_STATE: no output since ppg_create; no output since ppg_restore (a snapshot does not carry the world image),
+ * or no full ppg_reset since a ppg_restore that left envs idle (their image is never rewritten by a step); the one-kernel
+ * step (PPG_OBS_SPLIT=0) keeps no image. */
+int ppg_world_state(ppg_handle h, int32_t env_begin, int32_t n_envs, float* out, void* cuda_stream);
+
 /* ECO extras of one env (ECO attributes agent_ages, agent_genomes[..].speed, dead_prey,
  * active_num_predators/prey), in the list order of ppg_read_env.  Any pointer may be NULL. Synchronises. */
 int ppg_read_env_eco(ppg_handle h, int32_t env, int32_t* age_pred, double* speed_pred, int32_t* age_prey,

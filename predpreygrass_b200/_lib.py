@@ -17,6 +17,7 @@ SYMBOLS = [
     "ppg_step_ordered", "ppg_step_host", "ppg_random_actions", "ppg_get_buffers", "ppg_snapshot_size", "ppg_snapshot", "ppg_restore",
     "ppg_read_env", "ppg_read_env_eco", "ppg_read_env_stag", "ppg_stats", "ppg_stats_device", "ppg_stats_clear", "ppg_launch_count", "ppg_last_error",
     "ppg_profile_begin", "ppg_profile_end", "ppg_profile_env_cycles", "ppg_rollout_random", "ppg_selftest_pow", "ppg_read_episode_eco", "ppg_read_episode_events_eco", "ppg_read_env_acc", "ppg_set_pdl_chain",
+    "ppg_world_state",
 ]
 
 _lib = None
@@ -65,6 +66,7 @@ def load():
     L.ppg_read_episode_eco.argtypes = [vp, i32, vp, vp]
     L.ppg_read_episode_events_eco.argtypes = [vp, i32, vp]
     L.ppg_read_env_acc.argtypes = [vp, i32, vp, vp]
+    L.ppg_world_state.argtypes = [vp, i32, i32, vp, vp]
     L.ppg_stats.argtypes = [vp, vp, vp]
     L.ppg_stats_device.argtypes = [vp, C.POINTER(vp), vp]
     L.ppg_stats_clear.argtypes = [vp, vp]

@@ -249,6 +249,23 @@ class BatchedPredPreyGrass:
         _lib.check(self.L.ppg_profile_end(self.h, C.byref(a), C.byref(b), C.byref(n)), self.h)
         return a.value, b.value, n.value
 
+    def world_state(self, env_begin=0, n=None, out=None):
+        """`grid_world_state` of envs [env_begin, env_begin + n) after the last output (include/ppg.h ppg_world_state):
+        float32 CUDA tensor [n, num_obs_channels, G, G], written on the current stream without synchronising.  Without
+        `out` it is a view of a buffer this object owns and reuses: valid until the next world_state() call."""
+        n = self.n_envs - int(env_begin) if n is None else int(n)
+        G, C = self.cfg.grid_size, self.cfg.num_obs_channels
+        shape = (n, C, G, G)
+        if out is None:
+            if getattr(self, "_world", None) is None:
+                self._world = torch.empty((self.n_envs, C, G, G), dtype=torch.float32, device=self.device)
+            out = self._world[: max(n, 0)]
+        elif out.dtype != torch.float32 or out.device != self.device or not out.is_contiguous() or tuple(out.shape) != shape:
+            raise ValueError(f"world_state: out must be a contiguous float32 tensor of shape {shape} on {self.device}, got "
+                             f"{out.dtype} {tuple(out.shape)} on {out.device} (contiguous={out.is_contiguous()})")
+        _lib.check(self.L.ppg_world_state(self.h, int(env_begin), n, out.data_ptr(), self._stream()), self.h)
+        return out
+
     def snapshot(self):
         n = self.L.ppg_snapshot_size(self.h)
         blob = np.empty(n, np.uint8)

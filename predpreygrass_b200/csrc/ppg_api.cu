@@ -40,6 +40,9 @@ cudaError_t launch_set_tape_reals_stag(StagHdr* shdr, int B, const long long* re
 cudaError_t launch_random_actions_stag(const int32_t* n_rows, const int32_t* re0, const int32_t* ra0, const int32_t* re1, const int32_t* ra1,
                                        int32_t* a0, int32_t* a1, unsigned long long seed, unsigned call, unsigned env_base, int t2_pred,
                                        int t2_prey, int ar0, int ar1, int blocks, cudaStream_t s);
+// ppg_world.cu
+cudaError_t launch_world_state(const WorldStateParams& p, int map_bytes, int n_cta, cudaStream_t stream);
+cudaError_t world_state_occupancy(const WorldStateParams& p, int map_bytes, int* blocks_per_sm);
 }  // namespace ppg
 
 namespace ppg { int g_pdl_chain = -1; }
@@ -67,6 +70,9 @@ struct ppg_handle_s {
   bool profiling = false;
   std::vector<cudaEvent_t> prof_events;  // triples: before the step kernel, between the kernels, after the observation kernel
   unsigned long long calls = 0;          // ppg_reset(all)/ppg_step calls (ppg_random_actions key)
+  // do the env images in obs_img show the world of the last output (ppg_world_state)?
+  enum { IMG_NONE, IMG_VALID, IMG_RESTORED, IMG_RESTORED_IDLE } img = IMG_NONE;
+  int n_cta_ws = 0;                      // ppg_world_state grid (0: not computed yet)
   int64_t launch_count = 0;
   std::vector<void*> allocs;
   unsigned long long* d_stats = nullptr;
@@ -104,6 +110,22 @@ static cudaError_t dalloc(ppg_handle h, T** p, size_t n) {
   h->allocs.push_back(q);
   *p = static_cast<T*>(q);
   return e;
+}
+
+// Which owner map and which value table show grid channel `ch` (so_* offsets): the observation rows (obs_rel) and
+// ppg_world_state both take their sources from here.
+//   BASE: 0 walls (predator map: its halo holds the wall entry of the wall table), 1 predators, 2 prey, 3 grass
+//   ECO:  0 predators, 1 prey, 2 grass (channel 3, the own-speed plane, is not a gather)
+//   STAG (STAG:112-117): 0 walls (wall cells are wall entries of the predator map), 1 predators, 2 mammoths, 3 rabbits,
+//         4 grass; further channels read the wall table through the predator map (all zero off the walls)
+struct ChannelSource { int map, tbl; };
+static ChannelSource channel_source(const StepParams& P, int ch) {
+  if (P.variant == PPG_VARIANT_STAG) {
+    static const int map_of[5] = {0, 0, 1, 3, 2};
+    return {P.so_map[ch < 5 ? map_of[ch] : 0], ch == 1 ? P.so_vt[0] : (ch == 2 || ch == 3) ? P.so_vt[1] : ch == 4 ? P.so_vt[2] : P.so_wt};
+  }
+  if (P.variant == PPG_VARIANT_ECO) return {P.so_map[ch], P.so_vt[ch]};
+  return {P.so_map[ch == 0 ? 0 : ch - 1], ch == 0 ? P.so_wt : P.so_vt[ch - 1]};
 }
 
 static int str_cmp_ids(const void* a, const void* b) {
@@ -440,22 +462,10 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
           const int ch = q / RR, i = (q % RR) / R, jj = q % R;
           const int cellrel = (i - P.off[s]) * P.PS + (jj - P.off[s]);
           const size_t at = ((size_t)(s * PPG_MAX_NJ + j) * 32 + lane) * 2;
-          if (stag) {  // STAG channels (STAG:112-117): 0 walls (none: an all-zero table), 1 predators, 2 mammoths, 3 rabbits, 4 grass
-            static const int map_of[5] = {0, 0, 1, 3, 2};
-            const int m = ch < 5 ? map_of[ch] : 0;
-            rel[at] = (P.so_map[m] - P.so_map[0]) + cellrel * P.map_bytes;
-            rel[at + 1] = ch == 1 ? P.so_vt[0] : (ch == 2 || ch == 3) ? P.so_vt[1] : ch == 4 ? P.so_vt[2] : P.so_wt;
-            continue;
-          }
-          if (eco) {  // ECO channels: 0 predators, 1 prey, 2 grass, 3 the agent's own speed (a constant plane, not a gather)
-            if (ch >= 3) { selfm[(size_t)s * 32 + lane] |= 1u << j; continue; }
-            rel[at] = (P.so_map[ch] - P.so_map[0]) + cellrel * P.map_bytes;
-            rel[at + 1] = P.so_vt[ch];
-            continue;
-          }
-          const int m = ch == 0 ? 0 : ch - 1;
-          rel[at] = (P.so_map[m] - P.so_map[0]) + cellrel * P.map_bytes;
-          rel[at + 1] = ch == 0 ? P.so_wt : P.so_vt[ch - 1];
+          if (eco && ch >= 3) { selfm[(size_t)s * 32 + lane] |= 1u << j; continue; }  // ECO's own-speed plane
+          const ChannelSource src = channel_source(P, ch);
+          rel[at] = (src.map - P.so_map[0]) + cellrel * P.map_bytes;
+          rel[at + 1] = src.tbl;
         }
     }
     int* d_rel = nullptr;
@@ -690,6 +700,9 @@ static int run_step_kernel(ppg_handle h, const int32_t* a0, const int32_t* a1, c
     h->launch_count++;
   }
   if (h->profiling) CK(cudaEventRecord(pe[2], st));
+  // the images now hold this output's world, except that an env idle since a ppg_restore still has the pre-restore one:
+  // after restoring idle envs only a full reset (a0 == NULL, every env dumps its image) makes them valid again
+  if (a0 == nullptr || h->img != ppg_handle_s::IMG_RESTORED_IDLE) h->img = ppg_handle_s::IMG_VALID;
   h->calls++;
   h->h_n_rows_valid = false;
   return PPG_OK;
@@ -928,6 +941,16 @@ int ppg_restore(ppg_handle h, const void* blob, size_t bytes, void* cuda_stream)
   }
   h->calls = head[0];
   q += SNAP_HEAD;
+  {
+    // the blob starts with the env headers; an env restored idle is never re-imaged by a step (header-only dump)
+    bool idle = false;
+    for (int e = 0; e < h->B && !idle; ++e) {
+      EnvHdr hd;
+      memcpy(&hd, q + (size_t)e * sizeof(EnvHdr), sizeof hd);
+      idle = hd.state == ST_IDLE;
+    }
+    h->img = idle ? ppg_handle_s::IMG_RESTORED_IDLE : ppg_handle_s::IMG_RESTORED;
+  }
   for (const Seg& s : state_segments(h)) { CK(cudaMemcpyAsync(s.p, q, s.bytes, cudaMemcpyHostToDevice, st)); q += s.bytes; }
   {
     int rc = prepare_offsets(h, st);
@@ -938,6 +961,46 @@ int ppg_restore(ppg_handle h, const void* blob, size_t bytes, void* cuda_stream)
   }
   CK(cudaStreamSynchronize(st));
   h->h_n_rows_valid = false;
+  return PPG_OK;
+}
+
+int ppg_world_state(ppg_handle h, int32_t env_begin, int32_t n_envs, float* out, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (env_begin < 0 || n_envs < 1 || env_begin > h->B - n_envs) { h->err = "ppg_world_state: env range outside [0, n_envs)"; return PPG_ERR_INVALID; }
+  if (!out) { h->err = "ppg_world_state: NULL out"; return PPG_ERR_INVALID; }
+  const StepParams& P = h->P;
+  if (!P.obs_split) { h->err = "ppg_world_state: the one-kernel step (PPG_OBS_SPLIT=0) keeps no env images"; return PPG_ERR_STATE; }
+  switch (h->img) {
+    case ppg_handle_s::IMG_NONE: h->err = "ppg_world_state: no output since ppg_create"; return PPG_ERR_STATE;
+    case ppg_handle_s::IMG_RESTORED: h->err = "ppg_world_state: no output since ppg_restore"; return PPG_ERR_STATE;
+    case ppg_handle_s::IMG_RESTORED_IDLE: h->err = "ppg_world_state: envs were restored idle; no full ppg_reset since"; return PPG_ERR_STATE;
+    default: break;
+  }
+  CK(cudaSetDevice(h->device));
+  WorldStateParams w;
+  memset(&w, 0, sizeof w);
+  w.img = P.obs_img; w.out = out; w.env_begin = env_begin; w.n_envs = n_envs;
+  w.img_stride = P.img_stride; w.img_bytes = P.img_bytes;
+  w.G = P.G; w.C = h->cfg.num_obs_channels; w.P = P.P; w.PS = P.PS;
+  for (int c = 0; c < PPG_WS_SRC; ++c) {
+    const ChannelSource src = channel_source(P, c < w.C ? c : w.C - 1);
+    w.map_off[c] = src.map - P.so_img; w.tbl_off[c] = src.tbl - P.so_img;
+  }
+  for (int c = PPG_WS_SRC; c < w.C; ++c) {
+    const ChannelSource src = channel_source(P, c);
+    if (src.map - P.so_img != w.map_off[PPG_WS_SRC - 1] || src.tbl - P.so_img != w.tbl_off[PPG_WS_SRC - 1]) {
+      h->err = "ppg_world_state: internal: channel sources past PPG_WS_SRC differ"; return PPG_ERR_STATE;
+    }
+  }
+  if (h->n_cta_ws == 0) {
+    int per_sm = 0, n_sm = 0;
+    CK(world_state_occupancy(w, P.map_bytes, &per_sm));
+    CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device));
+    if (per_sm < 1) { h->err = "ppg_world_state: kernel does not fit on an SM"; return PPG_ERR_INVALID; }
+    h->n_cta_ws = per_sm * n_sm;
+  }
+  CK(launch_world_state(w, P.map_bytes, std::min(n_envs, h->n_cta_ws), static_cast<cudaStream_t>(cuda_stream)));
+  h->launch_count++;
   return PPG_OK;
 }
 

@@ -241,6 +241,19 @@ struct StepParams {
                         //                       (so_map[m] + rel * map_bytes), y = byte offset of the value table; x = INT_MAX: no element
 };
 
+// ppg_world_state (ppg_world.cu): grid channel c of env e is table_c[map_c[P + (x + P) * PS + y]] of the env's image.
+// Channels >= PPG_WS_SRC share the source of channel PPG_WS_SRC - 1 (STAG's channels past grass: walls table, all zero).
+#define PPG_WS_SRC 8
+struct WorldStateParams {
+  const unsigned char* img;  // StepParams::obs_img
+  float* out;                // [n_envs][C][G][G]
+  int env_begin, n_envs;
+  int img_stride, img_bytes; // image pitch in HBM, bytes brought into shared memory (a multiple of 16)
+  int G, C, P, PS;
+  int map_off[PPG_WS_SRC];   // byte offset of channel c's owner map inside the image
+  int tbl_off[PPG_WS_SRC];   // byte offset of channel c's fp32 value table inside the image
+};
+
 // Launch with programmatic stream serialization (PDL): the grid's CTAs may be scheduled as soon as every CTA of the kernel
 // before it in the stream has executed griddepcontrol.launch_dependents (or exited), which hides the launch ramp of the 2960
 // one-warp CTAs of a step kernel behind the tail of the observation kernel.  The kernel MUST execute griddepcontrol.wait before

@@ -253,6 +253,12 @@ class _RowDictEnv(_Base):
         st = self._read()
         return {f"grass_{k}": float(e) for k, e in enumerate(st["grass_energy"])}
 
+    @property
+    def grid_world_state(self):
+        """the reference's `grid_world_state` (float32 [num_obs_channels, G, G], ECO / STAG / trait variants): the world
+        after the last reset() / step().  After restore_state_snapshot() it is available again after the next step()."""
+        return self._batch.world_state(0, 1)[0].cpu().numpy()
+
     def get_state_snapshot(self):
         return {"blob": self._batch.snapshot(), "current_step": self.current_step, "agents": list(self.agents),
                 "agents_just_ate": set(self.agents_just_ate), "done": self._done}
