@@ -408,6 +408,84 @@ int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, 
  * step (PPG_OBS_SPLIT=0) keeps no image. */
 int ppg_world_state(ppg_handle h, int32_t env_begin, int32_t n_envs, float* out, void* cuda_stream);
 
+/*
+ * Episode returns and agent lifetimes on the device (RLlib's episode_return_mean, episode_len_mean,
+ * module_episode_returns_mean; the per-life records the evolutionary analyses read).  Off by default: while off nothing is
+ * launched, allocated or changed.  While on, every output (ppg_reset without a mask, ppg_step, ppg_step_ordered,
+ * ppg_step_host, every step of ppg_rollout_random) is followed by one more kernel on the same stream that updates:
+ *
+ *   Row columns, per species, indexed like the rows of the output they belong to:
+ *     row_return[s][r] (f64): the agent's return so far in this life: the sum, in f64, of the fp32 reward[s] of every row
+ *       the agent has had in the current episode, this one included (the rewards the rows hand out, not the reference's
+ *       internal float64 ones);
+ *     row_life[s][r] (int32): the number of rows the agent has had in this episode, this one included.
+ *     A row flagged PPG_ROW_FOUNDER or PPG_ROW_NEWBORN starts a new life (row_return = reward, row_life = 1); any other row
+ *     continues the life of the same (env, numeric id) of the previous output.  On a row flagged TERMINATED or TRUNCATED
+ *     they are the agent's lifetime return and lifetime rows.
+ *   Per env:
+ *     env_return[e][2] (f64): the running episode return per species after this output.  An output with PPG_ENV_RESET
+ *       starts it from 0 before adding its own rows.  An output with PPG_ENV_TERMINATED | PPG_ENV_TRUNCATED ends the
+ *       episode, which is folded into the env's accumulators env_acc[e][PPG_EP_*]: one episode, its length env_step[e],
+ *       its return per species and in total, the square of the total, the max and -min of the total.  A masked reset
+ *       abandons a running episode: it is not counted.  Idle envs (PPG_ENV_IDLE) change nothing.
+ *     For every row flagged TERMINATED or TRUNCATED the env's per-species accumulators add one life ended, one death
+ *       (TERMINATED only), its row_return and its row_life.
+ *   Validity: env_valid[e] is cleared when tracking is switched on and by ppg_restore (the tracking state is not part of
+ *     the snapshot blob), and set again by the env's next output with PPG_ENV_RESET.  An invalid env writes NaN / 0 into
+ *     its rows' columns, keeps env_return at NaN and accumulates nothing.  Switched on before the first full reset,
+ *     tracking sees every episode; envs part-way through an episode are counted from their next episode on.
+ *
+ * Kernel: one warp per env.  Per species it first updates the env's old rows (lanes in parallel, the old rows of an env
+ * have distinct ids), then, after __syncwarp, its newborn rows, so an old TERMINATED row finishes its id's life before a
+ * newborn row could restart that id (every variant hands newborns never-used ids today, so no id is reused within an
+ * episode; the order keeps the tables right should one ever be reused in the step that freed it).  The per-step
+ * sums (the step reward per species, the returns of the lives ended) are formed in one fixed order: lane l adds, in f64 and
+ * in row order, old rows l, l+32, ... and then newborn rows l, l+32, ... to a partial starting at 0.0; the 32 partials are
+ * combined by an xor-butterfly (v += shfl_xor(v, k), k = 16, 8, 4, 2, 1).  Per-agent state lives in tables indexed by
+ * (env, numeric id; STAG: the flat id): 12 bytes x n_envs x (n_possible[0] + n_possible[1]), allocated with the row
+ * columns and the per-env state when tracking is first switched on.  The kernel is launched after the observation kernel
+ * with plain stream order and never triggers dependent launches, so with the launch chain on the next step's kernels do
+ * not start while it still reads reward, flags and row_agent.
+ */
+#define PPG_N_EP_STATS 16
+enum {
+  PPG_EP_EPISODES = 0,       /* episodes finished */
+  PPG_EP_LENGTH_SUM = 1,     /* sum of their lengths (env_step at the end) */
+  PPG_EP_RETURN_SUM = 2,     /* sum of their total returns (predator + prey) */
+  PPG_EP_RETURN_SQ_SUM = 3,  /* sum of the squares of their total returns */
+  PPG_EP_RETURN_PRED = 4,    /* sum of their predator returns */
+  PPG_EP_RETURN_PREY = 5,    /* sum of their prey returns */
+  PPG_EP_RETURN_MAX = 6,     /* max total return (-inf: no episode); reduces with MAX */
+  PPG_EP_RETURN_NEG_MIN = 7, /* -(min total return) (-inf: no episode); reduces with MAX */
+  PPG_EP_LIVES = 8,          /* per species, slot + 4 * s: lives ended (rows flagged TERMINATED or TRUNCATED) */
+  PPG_EP_DEATHS = 9,         /* ... of them TERMINATED */
+  PPG_EP_LIFE_RETURN = 10,   /* ... sum of their lifetime returns (row_return) */
+  PPG_EP_LIFE_ROWS = 11      /* ... sum of their lifetime rows (row_life) */
+};
+#define PPG_EP_SPECIES_STRIDE 4
+
+/* Device pointers of the tracking state; valid while tracking is on, until ppg_destroy. */
+typedef struct ppg_returns {
+  double* row_return[2]; /* [row_capacity[s]] */
+  int32_t* row_life[2];  /* [row_capacity[s]] */
+  double* env_return;    /* [n_envs][2] */
+  uint8_t* env_valid;    /* [n_envs] */
+  double* env_acc;       /* [n_envs][PPG_N_EP_STATS]: each env's share of the aggregate vector */
+} ppg_returns;
+
+/* Switches tracking on (on != 0) or off.  The first switch-on allocates the state and clears the accumulators; every
+ * switch-on marks all envs invalid until their next reset (stream-ordered on cuda_stream).  Switching off keeps the state
+ * and the accumulators.  PPG_ERR_CUDA if the allocation fails. */
+int ppg_track_returns(ppg_handle h, int32_t on, void* cuda_stream);
+/* The device pointers of the tracking state.  PPG_ERR_STATE while tracking is off. */
+int ppg_get_returns(ppg_handle h, ppg_returns* out);
+/* The aggregate vector: env_acc summed over the envs whose env_valid is set (slots 6 and 7: max), PPG_N_EP_STATS doubles
+ * left in a device buffer of the handle (valid until the next call).  Reduced in a fixed order, so it is bit-identical from
+ * run to run.  Stream-ordered, no synchronisation; two kernel launches.  PPG_ERR_STATE before tracking was first on. */
+int ppg_episode_stats_device(ppg_handle h, double** dev_out, void* cuda_stream);
+/* Clears every env's accumulators (stream-ordered, one kernel launch).  PPG_ERR_STATE before tracking was first on. */
+int ppg_episode_stats_clear(ppg_handle h, void* cuda_stream);
+
 /* ECO extras of one env (ECO attributes agent_ages, agent_genomes[..].speed, dead_prey,
  * active_num_predators/prey), in the list order of ppg_read_env.  Any pointer may be NULL. Synchronises. */
 int ppg_read_env_eco(ppg_handle h, int32_t env, int32_t* age_pred, double* speed_pred, int32_t* age_prey,

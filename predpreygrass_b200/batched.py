@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .config import N_STATS, STAT_NAMES, VARIANT_ECO, PpgBuffers, PpgConfig, PpgTape
+from .config import N_EP_STATS, N_STATS, STAT_NAMES, VARIANT_ECO, PpgBuffers, PpgConfig, PpgReturns, PpgTape
 
 
 class _DevPtr:
@@ -24,7 +24,7 @@ class _DevPtr:
         self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 3}
 
 
-_TYPESTR = {torch.float32: "<f4", torch.int32: "<i4", torch.uint8: "|u1", torch.int64: "<i8"}
+_TYPESTR = {torch.float32: "<f4", torch.float64: "<f8", torch.int32: "<i4", torch.uint8: "|u1", torch.int64: "<i8"}
 
 
 def _view(ptr, shape, dtype, device):
@@ -55,6 +55,44 @@ class StepOutput:
         """(n_pred_rows, n_prey_rows) — synchronises (device -> host read of 16 bytes)."""
         n = self.n_rows.tolist()
         return n[0] + n[2], n[1] + n[3]
+
+
+@dataclass
+class Returns:
+    """Views of the episode-returns state (include/ppg.h ppg_track_returns); the row columns belong to the last output."""
+
+    row_return: tuple   # (pred, prey) f64 [cap]: return so far of the row's agent in this life
+    row_life: tuple     # (pred, prey) int32 [cap]: rows so far of the row's agent in this life
+    env_return: torch.Tensor  # f64 [B, 2]: running episode return per species (NaN: env not valid)
+    env_valid: torch.Tensor   # uint8 [B]: 1 once the env has been reset since tracking was switched on / a restore
+    env_acc: torch.Tensor     # f64 [B, N_EP_STATS]: each env's share of episode_stats_device()
+
+
+def episode_metrics_from_stats(v):
+    """The PPG_N_EP_STATS vector (summed over envs and ranks) -> RLlib's episode metric names, plus per-species lifetimes.
+    Means are nan when their count is 0; with no episode, episode_return_max is -inf and episode_return_min +inf."""
+    v = np.asarray(v, np.float64)
+    if v.shape != (N_EP_STATS,):
+        raise ValueError(f"expected the {N_EP_STATS}-slot episode statistics vector, got shape {v.shape}")
+
+    def mean(total, count):
+        return float(total / count) if count > 0 else float("nan")
+
+    n = v[0]
+    sp = ("predator", "prey")
+    life = [v[8 + 4 * s: 12 + 4 * s] for s in range(2)]  # lives, deaths, return sum, rows sum
+    return {
+        "num_episodes": int(n),
+        "episode_return_mean": mean(v[2], n),
+        "episode_return_min": float(-v[7]),
+        "episode_return_max": float(v[6]),
+        "episode_len_mean": mean(v[1], n),
+        "module_episode_returns_mean": {"predator": mean(v[4], n), "prey": mean(v[5], n)},
+        "agent_lifetime_return_mean": {sp[s]: mean(life[s][2], life[s][0]) for s in range(2)},
+        "agent_lifetime_rows_mean": {sp[s]: mean(life[s][3], life[s][0]) for s in range(2)},
+        "agent_deaths": {sp[s]: int(life[s][1]) for s in range(2)},
+        "agent_lives_ended": {sp[s]: int(life[s][0]) for s in range(2)},
+    }
 
 
 class BatchedPredPreyGrass:
@@ -229,6 +267,40 @@ class BatchedPredPreyGrass:
 
     def stats_clear(self):
         _lib.check(self.L.ppg_stats_clear(self.h, self._stream()), self.h)
+
+    # ------------------------------------------------------------------ episode returns (include/ppg.h ppg_track_returns)
+    def track_returns(self, on=True):
+        """Switch episode-return tracking on or off.  Switching on marks every env invalid until its next reset, so call
+        it before reset() to see every episode."""
+        _lib.check(self.L.ppg_track_returns(self.h, 1 if on else 0, self._stream()), self.h)
+
+    def returns(self):
+        """Zero-copy views of the tracking state (a `Returns`); PpgError while tracking is off."""
+        r = PpgReturns()
+        _lib.check(self.L.ppg_get_returns(self.h, C.byref(r)), self.h)
+        d, B, cap = self.device, self.n_envs, self.row_capacity
+        return Returns(row_return=tuple(_view(r.row_return[s], (cap[s],), torch.float64, d) for s in range(2)),
+                       row_life=tuple(_view(r.row_life[s], (cap[s],), torch.int32, d) for s in range(2)),
+                       env_return=_view(r.env_return, (B, 2), torch.float64, d),
+                       env_valid=_view(r.env_valid, (B,), torch.uint8, d),
+                       env_acc=_view(r.env_acc, (B, N_EP_STATS), torch.float64, d))
+
+    def episode_stats_device(self):
+        """The N_EP_STATS float64 vector reduced over the valid envs, on the current stream without synchronising: a view of
+        a buffer of the handle, valid until the next call."""
+        p = C.c_void_p()
+        _lib.check(self.L.ppg_episode_stats_device(self.h, C.byref(p), self._stream()), self.h)
+        return _view(p.value, (N_EP_STATS,), torch.float64, self.device)
+
+    def episode_stats_clear(self):
+        _lib.check(self.L.ppg_episode_stats_clear(self.h, self._stream()), self.h)
+
+    def episode_metrics(self, group=None):
+        """RLlib's episode metrics over this handle's envs (and over the ranks of `group` when torch.distributed is
+        initialised): episode_stats_device() all-reduced and converted by episode_metrics_from_stats.  Synchronises."""
+        from .sharding import allreduce_episode_stats
+
+        return episode_metrics_from_stats(allreduce_episode_stats(self.episode_stats_device().clone(), group).cpu().numpy())
 
     def launch_count(self):
         return int(self.L.ppg_launch_count(self.h))

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libppg_b200.so")
-SOURCES = ["ppg_base.cu", "ppg_eco.cu", "ppg_stag.cu", "ppg_obs.cu", "ppg_world.cu", "ppg_api.cu"]
+SOURCES = ["ppg_base.cu", "ppg_eco.cu", "ppg_stag.cu", "ppg_obs.cu", "ppg_world.cu", "ppg_returns.cu", "ppg_api.cu"]
 HEADERS = ["ppg_device.cuh", "ppg_step_common.cuh", os.path.join("..", "..", "include", "ppg.h"), os.path.join("..", "..", "include", "ppg_philox.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

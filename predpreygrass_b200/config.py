@@ -33,6 +33,13 @@ STAT_NAMES = [
     "starved_prey", "eaten_prey", "grass_eaten", "truncated", "rows_pred", "rows_prey", "spawn_fallback",
     "status_envs", "capture_attempts",
 ]
+# include/ppg.h PPG_EP_*: the episode-returns vector (ppg_episode_stats_device); slots 6 and 7 reduce with MAX, the others with SUM
+N_EP_STATS = 16
+EP_STAT_NAMES = [
+    "episodes", "length_sum", "return_sum", "return_sq_sum", "return_pred", "return_prey", "return_max", "return_neg_min",
+    "lives_pred", "deaths_pred", "life_return_pred", "life_rows_pred", "lives_prey", "deaths_prey", "life_return_prey", "life_rows_prey",
+]
+EP_MAX_SLOTS = (6, 7)
 
 
 class PpgConfig(C.Structure):
@@ -158,6 +165,16 @@ class PpgBuffers(C.Structure):
         ("row_capacity", C.c_int64 * 2),
         ("obs_row_elems", C.c_int32 * 2),
         ("n_envs", C.c_int32),
+    ]
+
+
+class PpgReturns(C.Structure):
+    _fields_ = [
+        ("row_return", C.c_void_p * 2),
+        ("row_life", C.c_void_p * 2),
+        ("env_return", C.c_void_p),
+        ("env_valid", C.c_void_p),
+        ("env_acc", C.c_void_p),
     ]
 
 

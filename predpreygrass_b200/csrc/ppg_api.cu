@@ -43,6 +43,11 @@ cudaError_t launch_random_actions_stag(const int32_t* n_rows, const int32_t* re0
 // ppg_world.cu
 cudaError_t launch_world_state(const WorldStateParams& p, int map_bytes, int n_cta, cudaStream_t stream);
 cudaError_t world_state_occupancy(const WorldStateParams& p, int map_bytes, int* blocks_per_sm);
+// ppg_returns.cu
+cudaError_t launch_returns(const ReturnsParams& p, cudaStream_t stream);
+int episode_stats_partials(int B);
+cudaError_t launch_episode_stats(const double* env_acc, const uint8_t* env_valid, int B, double* partial, double* out, cudaStream_t stream);
+cudaError_t launch_episode_stats_clear(double* env_acc, int B, cudaStream_t stream);
 }  // namespace ppg
 
 namespace ppg { int g_pdl_chain = -1; }
@@ -73,6 +78,12 @@ struct ppg_handle_s {
   // do the env images in obs_img show the world of the last output (ppg_world_state)?
   enum { IMG_NONE, IMG_VALID, IMG_RESTORED, IMG_RESTORED_IDLE } img = IMG_NONE;
   int n_cta_ws = 0;                      // ppg_world_state grid (0: not computed yet)
+  // episode returns (ppg_track_returns): allocated at the first switch-on
+  bool track_on = false;
+  ReturnsParams R;
+  bool R_alloc = false;
+  double* d_ep_partial = nullptr;        // ppg_episode_stats_device scratch and result
+  double* d_ep_stats = nullptr;
   int64_t launch_count = 0;
   std::vector<void*> allocs;
   unsigned long long* d_stats = nullptr;
@@ -700,6 +711,10 @@ static int run_step_kernel(ppg_handle h, const int32_t* a0, const int32_t* a1, c
     h->launch_count++;
   }
   if (h->profiling) CK(cudaEventRecord(pe[2], st));
+  if (h->track_on) {  // after pe[2]: the per-kernel timing of the step is the same with tracking on
+    CK(launch_returns(h->R, st));
+    h->launch_count++;
+  }
   // the images now hold this output's world, except that an env idle since a ppg_restore still has the pre-restore one:
   // after restoring idle envs only a full reset (a0 == NULL, every env dumps its image) makes them valid again
   if (a0 == nullptr || h->img != ppg_handle_s::IMG_RESTORED_IDLE) h->img = ppg_handle_s::IMG_VALID;
@@ -959,8 +974,75 @@ int ppg_restore(ppg_handle h, const void* blob, size_t bytes, void* cuda_stream)
     CK(launch_relabel_rows(h->P, h->P.cntA[q], h->P.sum1[q], h->P.sum2[q], h->P.totals + 4 * q, st));
     h->launch_count++;
   }
+  if (h->track_on) {  // the tracking state is not in the blob: every env is invalid until its next reset
+    CK(cudaMemsetAsync(h->R.env_valid, 0, (size_t)h->B, st));
+    CK(cudaMemsetAsync(h->R.env_return, 0xFF, (size_t)h->B * 2 * sizeof(double), st));  // all-ones bits: NaN
+  }
   CK(cudaStreamSynchronize(st));
   h->h_n_rows_valid = false;
+  return PPG_OK;
+}
+
+int ppg_track_returns(ppg_handle h, int32_t on, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (!on) { h->track_on = false; return PPG_OK; }
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  CK(cudaSetDevice(h->device));
+  ReturnsParams& R = h->R;
+  const StepParams& P = h->P;
+  if (!h->R_alloc) {
+    memset(&R, 0, sizeof R);
+    for (int s = 0; s < 2; ++s) {
+      R.row_agent[s] = P.row_agent[s]; R.reward[s] = P.reward[s]; R.flags[s] = P.flags[s];
+      R.old_off[s] = P.old_off[s]; R.new_off[s] = P.new_off[s]; R.new_cnt[s] = P.new_cnt[s];
+      R.n_possible[s] = P.n_possible[s];
+      CK(dalloc(h, &R.row_return[s], (size_t)h->bufs.row_capacity[s]));
+      CK(dalloc(h, &R.row_life[s], (size_t)h->bufs.row_capacity[s]));
+      CK(dalloc(h, &R.tab_ret[s], (size_t)h->B * P.n_possible[s]));
+      CK(dalloc(h, &R.tab_life[s], (size_t)h->B * P.n_possible[s]));
+    }
+    R.env_flags = P.env_flags; R.env_step = P.env_step; R.B = h->B;
+    CK(dalloc(h, &R.env_return, (size_t)h->B * 2));
+    CK(dalloc(h, &R.env_valid, (size_t)h->B));
+    CK(dalloc(h, &R.env_acc, (size_t)h->B * PPG_N_EP_STATS));
+    CK(dalloc(h, &h->d_ep_partial, (size_t)episode_stats_partials(h->B) * PPG_N_EP_STATS));
+    CK(dalloc(h, &h->d_ep_stats, PPG_N_EP_STATS));
+    h->R_alloc = true;
+    CK(launch_episode_stats_clear(R.env_acc, h->B, st));
+    h->launch_count++;
+  }
+  if (!h->track_on) {
+    CK(cudaMemsetAsync(R.env_valid, 0, (size_t)h->B, st));
+    CK(cudaMemsetAsync(R.env_return, 0xFF, (size_t)h->B * 2 * sizeof(double), st));  // all-ones bits: NaN
+  }
+  h->track_on = true;
+  return PPG_OK;
+}
+
+int ppg_get_returns(ppg_handle h, ppg_returns* out) {
+  if (!h || !out) return PPG_ERR_INVALID;
+  if (!h->track_on) { h->err = "ppg_get_returns: tracking is off (ppg_track_returns)"; return PPG_ERR_STATE; }
+  for (int s = 0; s < 2; ++s) { out->row_return[s] = h->R.row_return[s]; out->row_life[s] = h->R.row_life[s]; }
+  out->env_return = h->R.env_return; out->env_valid = h->R.env_valid; out->env_acc = h->R.env_acc;
+  return PPG_OK;
+}
+
+int ppg_episode_stats_device(ppg_handle h, double** dev_out, void* cuda_stream) {
+  if (!h || !dev_out) return PPG_ERR_INVALID;
+  if (!h->R_alloc) { h->err = "ppg_episode_stats_device: tracking was never switched on (ppg_track_returns)"; return PPG_ERR_STATE; }
+  CK(cudaSetDevice(h->device));
+  CK(launch_episode_stats(h->R.env_acc, h->R.env_valid, h->B, h->d_ep_partial, h->d_ep_stats, static_cast<cudaStream_t>(cuda_stream)));
+  h->launch_count += 2;
+  *dev_out = h->d_ep_stats;
+  return PPG_OK;
+}
+
+int ppg_episode_stats_clear(ppg_handle h, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (!h->R_alloc) { h->err = "ppg_episode_stats_clear: tracking was never switched on (ppg_track_returns)"; return PPG_ERR_STATE; }
+  CK(cudaSetDevice(h->device));
+  CK(launch_episode_stats_clear(h->R.env_acc, h->B, static_cast<cudaStream_t>(cuda_stream)));
+  h->launch_count++;
   return PPG_OK;
 }
 

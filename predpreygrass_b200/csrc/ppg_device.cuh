@@ -254,6 +254,28 @@ struct WorldStateParams {
   int tbl_off[PPG_WS_SRC];   // byte offset of channel c's fp32 value table inside the image
 };
 
+// ppg_returns_kernel (ppg_returns.cu): episode returns and agent lifetimes, updated from the rows of the last output
+// (include/ppg.h ppg_track_returns).
+struct ReturnsParams {
+  const int32_t* row_agent[2];
+  const float* reward[2];
+  const uint8_t* flags[2];
+  const int32_t* old_off[2];
+  const int32_t* new_off[2];
+  const int32_t* new_cnt[2];
+  const uint8_t* env_flags;
+  const int32_t* env_step;
+  double* row_return[2];  // [row_capacity[s]]
+  int32_t* row_life[2];
+  double* tab_ret[2];     // [B][n_possible[s]]: return so far of the life of (env, id)
+  int32_t* tab_life[2];   // [B][n_possible[s]]: rows so far of that life
+  double* env_return;     // [B][2]
+  uint8_t* env_valid;     // [B]
+  double* env_acc;        // [B][PPG_N_EP_STATS]
+  int n_possible[2];
+  int B;
+};
+
 // Launch with programmatic stream serialization (PDL): the grid's CTAs may be scheduled as soon as every CTA of the kernel
 // before it in the stream has executed griddepcontrol.launch_dependents (or exited), which hides the launch ramp of the 2960
 // one-warp CTAs of a step kernel behind the tail of the observation kernel.  The kernel MUST execute griddepcontrol.wait before

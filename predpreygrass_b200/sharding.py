@@ -7,7 +7,7 @@ The only exchange is the small all-reduce of the episode / population statistics
 import torch
 import torch.distributed as dist
 
-from .config import N_STATS, STAT_NAMES
+from .config import EP_MAX_SLOTS, N_EP_STATS, N_STATS, STAT_NAMES
 
 
 def shard_range(n_envs_total, rank, world_size):
@@ -56,6 +56,21 @@ def allreduce_stats(stats, group=None):
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.all_reduce(stats, op=dist.ReduceOp.SUM, group=group)
     return dict(zip(STAT_NAMES, stats.tolist()))
+
+
+def allreduce_episode_stats(vec, group=None):
+    """All-reduce the N_EP_STATS float64 episode-returns vector (`BatchedPredPreyGrass.episode_stats_device()`) in place:
+    SUM over every slot except the max and -min of the episode return (slots 6 and 7), which reduce with MAX.  Returns it."""
+    if vec.dtype != torch.float64 or vec.numel() != N_EP_STATS:
+        raise ValueError("vec must be the float64 PPG_N_EP_STATS vector")
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        lo, hi = EP_MAX_SLOTS[0], EP_MAX_SLOTS[1] + 1
+        extremes = vec[lo:hi].clone()
+        vec[lo:hi] = 0.0
+        dist.all_reduce(vec, op=dist.ReduceOp.SUM, group=group)
+        dist.all_reduce(extremes, op=dist.ReduceOp.MAX, group=group)
+        vec[lo:hi] = extremes
+    return vec
 
 
 def max_over_ranks(value, device, group=None):
