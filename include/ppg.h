@@ -486,6 +486,70 @@ int ppg_episode_stats_device(ppg_handle h, double** dev_out, void* cuda_stream);
 /* Clears every env's accumulators (stream-ordered, one kernel launch).  PPG_ERR_STATE before tracking was first on. */
 int ppg_episode_stats_clear(ppg_handle h, void* cuda_stream);
 
+/*
+ * Advantages and value targets of a rollout (RLlib PPO's GAE: `advantages` are the lambda-returns minus `vf_preds`).
+ * A rollout is T+1 consecutive outputs 0..T of one handle, copied by the caller into slabs (slot t = output t).  For every
+ * output the caller supplies value[s][t][r] (fp32), the value estimate of row r of output t, for every row, including rows
+ * flagged TERMINATED or TRUNCATED.
+ *
+ *   Successor link: row r of output t < T has a successor when output t+1 holds a row of the same (env, row_agent) (STAG: the
+ *     flat id) that is flagged neither FOUNDER nor NEWBORN; next_row[s][t][r] is its row, else -1.  Rows flagged TERMINATED
+ *     or TRUNCATED, rows of an env whose output t+1 has PPG_ENV_RESET (a masked or automatic reset: the step did not happen
+ *     for them) and the rows of output T have none.  A row with a successor is exactly a transition: the rows of output t
+ *     with a successor are as many as the rows of output t+1 that are old and not FOUNDER.
+ *   End of a life: a successor row r' of output t+1, with row flags f and env flags ef of output t+1, is
+ *     terminal  when (f & TERMINATED) or ((ef & PPG_ENV_TERMINATED) and not (f & TRUNCATED));
+ *     truncated when it is not terminal and (f & TRUNCATED) or (ef & PPG_ENV_TRUNCATED).
+ *     So each variant's own flags decide: BASE leaves the survivors of an extinction unflagged and ECO flags them
+ *     TERMINATED, both are terminal (RLlib's `__all__` ends every agent); STAG flags them TRUNCATED (STAG:587-591), they
+ *     bootstrap.
+ *   Recursion, in fp32, each expression evaluated exactly as written (no fused multiply-add), gl = fp32(gamma) * fp32(lambda)
+ *   computed once; for every transition (t, r) -> (t+1, r'):
+ *     vn    = terminal(r') ? 0 : value[t+1][r']
+ *     cont  = t+1 < T && !terminal(r') && !truncated(r') && next_row[t+1][r'] >= 0
+ *     An    = cont ? adv[t+1][r'] : 0
+ *     delta = (reward[t+1][r'] + gamma * vn) - value[t][r]
+ *     adv[t][r]          = delta + gl * An
+ *     value_target[t][r] = adv[t][r] + value[t][r]
+ *   A live agent at the end of the rollout bootstraps from V(output T); so does an agent whose next output is a masked reset
+ *   (its last row has no successor) and a truncated life (from the value of its final row).  Rows of output t without a
+ *   successor get adv = value_target = NaN; rows at or beyond the output's row count are not written.
+ *
+ * Slabs, [s] = species, C = row_capacity[s] of the handle, B = n_envs; slot t of a slab starts at element t * C (rows) or
+ * t * B, t * (B + 1) (per-env columns), every slab is a DEVICE array.  The env's rows of output t are
+ * [old_off[t][e], old_off[t][e+1]) and [new_off[t][e], new_off[t][e] + new_cnt[t][e]) as in ppg_buffers.
+ */
+#define PPG_GAE_ERR_ID 0x1u    /* a row's id is outside [0, n_possible[s]) */
+#define PPG_GAE_ERR_LINK 0x2u  /* an old, non-FOUNDER row of output t+1 has no live row of the same id in output t */
+#define PPG_GAE_ERR_RANGE 0x4u /* an env's row range lies outside [0, C), or it holds more old rows than fit the link table */
+typedef struct ppg_gae_args {
+  int32_t T;                  /* steps of the rollout (>= 1): outputs 0..T */
+  float gamma, lam;            /* discount and GAE lambda, each in [0, 1] */
+  const int32_t* row_agent[2]; /* [T+1][C] */
+  const uint8_t* flags[2];     /* [T+1][C] PPG_ROW_* */
+  const float* reward[2];      /* [T+1][C] */
+  const float* value[2];       /* [T+1][C] */
+  const int32_t* old_off[2];   /* [T+1][B+1] */
+  const int32_t* new_off[2];   /* [T+1][B] */
+  const int32_t* new_cnt[2];   /* [T+1][B] */
+  const uint8_t* env_flags;    /* [T+1][B] PPG_ENV_* */
+  float* adv[2];               /* [T][C] out */
+  float* value_target[2];      /* [T][C] out */
+  int32_t* next_row[2];        /* [T][C] out */
+  uint32_t* error;             /* [1] out: cleared by the call, then PPG_GAE_ERR_* bits ORed in by the kernel */
+} ppg_gae_args;
+
+/* Links the rows of the rollout and runs the recursion above: one kernel launch on cuda_stream (after a 4-byte memset of
+ * a->error), one warp per env and species walking backward from t = T-1 to 0.  The links are matched per env in a hash table
+ * of the env's old rows in shared memory (2 x 4 bytes x the next power of two >= 2 * max(cap_live) per warp): the memory
+ * does not grow with n_possible.  It reads only the caller's slabs, never the handle's live outputs, keeps no state in the
+ * handle, does not synchronise and never triggers dependent launches.  The result is deterministic: every value is one chain
+ * of fp32 operations.  Malformed slabs do not fault: the kernel sets PPG_GAE_ERR_* in *a->error (a device word the caller
+ * reads when it synchronises, as it reads the step kernels' status words) and leaves the affected rows unlinked.
+ * PPG_ERR_INVALID: NULL handle, args or pointer, T < 1, gamma or lambda outside [0, 1], max(cap_live) > 8192 (the two tables
+ * of one warp would not fit in shared memory). */
+int ppg_gae(ppg_handle h, const ppg_gae_args* a, void* cuda_stream);
+
 /* ECO extras of one env (ECO attributes agent_ages, agent_genomes[..].speed, dead_prey,
  * active_num_predators/prey), in the list order of ppg_read_env.  Any pointer may be NULL. Synchronises. */
 int ppg_read_env_eco(ppg_handle h, int32_t env, int32_t* age_pred, double* speed_pred, int32_t* age_prey,

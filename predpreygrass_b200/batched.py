@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .config import N_EP_STATS, N_STATS, STAT_NAMES, VARIANT_ECO, PpgBuffers, PpgConfig, PpgReturns, PpgTape
+from .config import N_EP_STATS, N_STATS, STAT_NAMES, VARIANT_ECO, PpgBuffers, PpgConfig, PpgGaeArgs, PpgReturns, PpgTape
 
 
 class _DevPtr:
@@ -337,6 +337,42 @@ class BatchedPredPreyGrass:
                              f"{out.dtype} {tuple(out.shape)} on {out.device} (contiguous={out.is_contiguous()})")
         _lib.check(self.L.ppg_world_state(self.h, int(env_begin), n, out.data_ptr(), self._stream()), self.h)
         return out
+
+    def gae(self, gamma, lam, row_agent, flags, reward, value, old_off, new_off, new_cnt, env_flags, adv, value_target, next_row,
+            error):
+        """GAE advantages and value targets of a recorded rollout (include/ppg.h ppg_gae): one kernel launch on the current
+        stream, no synchronisation.  Per-species arguments are (pred, prey) pairs of contiguous CUDA tensors on this device:
+        row_agent int32, flags uint8, reward and value float32 [T+1, cap]; old_off int32 [T+1, B+1]; new_off, new_cnt int32
+        [T+1, B]; env_flags uint8 [T+1, B]; outputs adv, value_target float32 and next_row int32 [T, cap]; error int32 [1]
+        receives the PPG_GAE_ERR_* bits.  `connector.RolloutBuffer` owns such slabs."""
+        T = int(env_flags.shape[0]) - 1 if env_flags.dim() == 2 else -1
+        B, cap = self.n_envs, self.row_capacity
+
+        def chk(name, t, dtype, shape):
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != self.device or not t.is_contiguous()
+                    or tuple(t.shape) != tuple(shape)):
+                got = f"{t.dtype} {tuple(t.shape)} on {t.device}" if isinstance(t, torch.Tensor) else type(t).__name__
+                raise ValueError(f"gae: {name} must be a contiguous {dtype} tensor of shape {tuple(shape)} on {self.device}, got {got}")
+            return t.data_ptr()
+
+        if T < 1:
+            raise ValueError(f"gae: env_flags must be [T+1, {B}] with T >= 1, got {tuple(env_flags.shape)}")
+        a = PpgGaeArgs()
+        a.T, a.gamma, a.lam = T, float(gamma), float(lam)
+        for s in range(2):
+            a.row_agent[s] = chk(f"row_agent[{s}]", row_agent[s], torch.int32, (T + 1, cap[s]))
+            a.flags[s] = chk(f"flags[{s}]", flags[s], torch.uint8, (T + 1, cap[s]))
+            a.reward[s] = chk(f"reward[{s}]", reward[s], torch.float32, (T + 1, cap[s]))
+            a.value[s] = chk(f"value[{s}]", value[s], torch.float32, (T + 1, cap[s]))
+            a.old_off[s] = chk(f"old_off[{s}]", old_off[s], torch.int32, (T + 1, B + 1))
+            a.new_off[s] = chk(f"new_off[{s}]", new_off[s], torch.int32, (T + 1, B))
+            a.new_cnt[s] = chk(f"new_cnt[{s}]", new_cnt[s], torch.int32, (T + 1, B))
+            a.adv[s] = chk(f"adv[{s}]", adv[s], torch.float32, (T, cap[s]))
+            a.value_target[s] = chk(f"value_target[{s}]", value_target[s], torch.float32, (T, cap[s]))
+            a.next_row[s] = chk(f"next_row[{s}]", next_row[s], torch.int32, (T, cap[s]))
+        a.env_flags = chk("env_flags", env_flags, torch.uint8, (T + 1, B))
+        a.error = chk("error", error, torch.int32, (1,))
+        _lib.check(self.L.ppg_gae(self.h, C.byref(a), self._stream()), self.h)
 
     def snapshot(self):
         n = self.L.ppg_snapshot_size(self.h)

@@ -178,6 +178,31 @@ class PpgReturns(C.Structure):
     ]
 
 
+class PpgGaeArgs(C.Structure):
+    """include/ppg.h ppg_gae_args: [s] = species, every pointer a device slab"""
+
+    _fields_ = [
+        ("T", C.c_int32),
+        ("gamma", C.c_float),
+        ("lam", C.c_float),
+        ("row_agent", C.c_void_p * 2),
+        ("flags", C.c_void_p * 2),
+        ("reward", C.c_void_p * 2),
+        ("value", C.c_void_p * 2),
+        ("old_off", C.c_void_p * 2),
+        ("new_off", C.c_void_p * 2),
+        ("new_cnt", C.c_void_p * 2),
+        ("env_flags", C.c_void_p),
+        ("adv", C.c_void_p * 2),
+        ("value_target", C.c_void_p * 2),
+        ("next_row", C.c_void_p * 2),
+        ("error", C.c_void_p),
+    ]
+
+
+GAE_ERR_ID, GAE_ERR_LINK, GAE_ERR_RANGE = 0x1, 0x2, 0x4  # include/ppg.h PPG_GAE_ERR_*
+
+
 def _round32(n):
     return max(32, (int(n) + 31) // 32 * 32)
 

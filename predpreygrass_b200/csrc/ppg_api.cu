@@ -48,6 +48,9 @@ cudaError_t launch_returns(const ReturnsParams& p, cudaStream_t stream);
 int episode_stats_partials(int B);
 cudaError_t launch_episode_stats(const double* env_acc, const uint8_t* env_valid, int B, double* partial, double* out, cudaStream_t stream);
 cudaError_t launch_episode_stats_clear(double* env_acc, int B, cudaStream_t stream);
+// ppg_gae.cu
+cudaError_t launch_gae(const GaeParams& p, cudaStream_t stream);
+int gae_warps(int log2_h);
 }  // namespace ppg
 
 namespace ppg { int g_pdl_chain = -1; }
@@ -1042,6 +1045,41 @@ int ppg_episode_stats_clear(ppg_handle h, void* cuda_stream) {
   if (!h->R_alloc) { h->err = "ppg_episode_stats_clear: tracking was never switched on (ppg_track_returns)"; return PPG_ERR_STATE; }
   CK(cudaSetDevice(h->device));
   CK(launch_episode_stats_clear(h->R.env_acc, h->B, static_cast<cudaStream_t>(cuda_stream)));
+  h->launch_count++;
+  return PPG_OK;
+}
+
+int ppg_gae(ppg_handle h, const ppg_gae_args* a, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (!a) { h->err = "ppg_gae: NULL args"; return PPG_ERR_INVALID; }
+  if (a->T < 1) { h->err = "ppg_gae: T must be >= 1"; return PPG_ERR_INVALID; }
+  if (!(a->gamma >= 0.0f && a->gamma <= 1.0f) || !(a->lam >= 0.0f && a->lam <= 1.0f)) {
+    h->err = "ppg_gae: gamma and lambda must lie in [0, 1]"; return PPG_ERR_INVALID;
+  }
+  for (int s = 0; s < 2; ++s) {
+    if (!a->row_agent[s] || !a->flags[s] || !a->reward[s] || !a->value[s] || !a->old_off[s] || !a->new_off[s] || !a->new_cnt[s] ||
+        !a->adv[s] || !a->value_target[s] || !a->next_row[s]) {
+      h->err = "ppg_gae: NULL slab"; return PPG_ERR_INVALID;
+    }
+  }
+  if (!a->env_flags || !a->error) { h->err = "ppg_gae: NULL slab"; return PPG_ERR_INVALID; }
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  CK(cudaSetDevice(h->device));
+  GaeParams g;
+  memset(&g, 0, sizeof g);
+  g.a = *a;
+  g.B = h->B;
+  int cap = 1;
+  for (int s = 0; s < 2; ++s) {
+    g.cap[s] = h->bufs.row_capacity[s];
+    g.n_possible[s] = h->P.n_possible[s];
+    cap = std::max(cap, h->cfg.cap_live[s]);
+  }
+  g.log2_h = 1;
+  while ((1 << g.log2_h) < 2 * cap) ++g.log2_h;  // load factor <= 1/2 with cap_live old rows per env
+  if (gae_warps(g.log2_h) < 1) { h->err = "ppg_gae: cap_live too large for the link tables (max(cap_live) <= 8192)"; return PPG_ERR_INVALID; }
+  CK(cudaMemsetAsync(a->error, 0, sizeof(uint32_t), st));
+  CK(launch_gae(g, st));
   h->launch_count++;
   return PPG_OK;
 }

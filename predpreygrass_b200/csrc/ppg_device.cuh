@@ -276,6 +276,15 @@ struct ReturnsParams {
   int B;
 };
 
+// ppg_gae_kernel (ppg_gae.cu): links the rows of a rollout and runs the GAE recursion (include/ppg.h ppg_gae).
+struct GaeParams {
+  ppg_gae_args a;
+  long long cap[2];   // row_capacity[s]: pitch of the row slabs
+  int n_possible[2];
+  int B;
+  int log2_h;         // link table: 1 << log2_h entries per warp and buffer
+};
+
 // Launch with programmatic stream serialization (PDL): the grid's CTAs may be scheduled as soon as every CTA of the kernel
 // before it in the stream has executed griddepcontrol.launch_dependents (or exited), which hides the launch ramp of the 2960
 // one-warp CTAs of a step kernel behind the tail of the observation kernel.  The kernel MUST execute griddepcontrol.wait before
