@@ -409,6 +409,55 @@ int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, 
 int ppg_world_state(ppg_handle h, int32_t env_begin, int32_t n_envs, float* out, void* cuda_stream);
 
 /*
+ * Agent state aligned with the rows: for every row of the handle's last output (the rows of ppg_get_buffers after the last
+ * ppg_step, ppg_step_ordered, ppg_step_host, full ppg_reset or step of ppg_rollout_random), the state of the agent behind it,
+ * as ppg_read_env / ppg_read_env_eco / ppg_read_env_stag / ppg_read_env_acc report it after the same output.
+ *
+ *   Present: row r of species s, with e = row_env[s][r] and id = row_agent[s][r] (STAG: the flat id, which the rows and the
+ *     lists both carry), is present when env_flags[e] has neither PPG_ENV_TERMINATED nor PPG_ENV_TRUNCATED and env e's agent
+ *     list of species s holds an entry with that id.  Its columns are that entry's:
+ *       pos (x, y); energy (f64); age (ECO family, STAG); trait (f64: the ECO family's genome `speed` as ppg_read_env_eco
+ *       reports it, which holds the trait of the trait variants; STAG predators' cooperation trait); facing (STAG predators,
+ *       index into `_predator_facing_options`); acc (cadence variant: the move accumulator).
+ *   Absent rows get present = 0, pos = (-1, -1), energy = trait = acc = NaN, age = facing = -1.  That covers every row of an
+ *     env whose episode ended in this output (survivors and ECO newborn rows kept at birth included: an auto-resetting env
+ *     does not write its lists back on the step that ends its episode, so they are not its final state), and every row whose
+ *     agent left the list (BASE and STAG deaths, eaten ECO prey).  ECO carcasses stay in the list: their TERMINATED row is
+ *     present and flagged PPG_ROW_CARCASS.  Rows at or beyond the output's row count are not written.
+ *   Grass, per env: grass_pos and grass_energy as ppg_read_env reports them; -1 / NaN for an env whose episode ended in this
+ *     output.  An idle env (autoreset off) has no rows; its grass is that of its final step.
+ *
+ * The state of an ended env's final step is not reported (out of reach for auto-resetting envs, see above; one rule for
+ * every ended env).  The call describes the last output until the next one: a masked ppg_reset only schedules resets and
+ * changes nothing here.  It works with the two-kernel and the one-kernel step (PPG_OBS_SPLIT=0).
+ *
+ * Kernel: one warp per env.  Per species it writes the sentinels into the env's rows, then (after __syncwarp) each lane takes
+ * list entries k and writes entry k's columns into row ag_prow[k] when that row lies in the env's row ranges and carries the
+ * entry's id.  The ids of one env's rows are distinct, so every present row is written by exactly one entry; a list entry
+ * without a row in this output (an ECO carcass of an earlier output, whose recorded row is stale) writes nothing.  No atomics:
+ * the result does not depend on scheduling.  Launched after the observation kernel with plain stream order, it never triggers
+ * dependent launches, so with the launch chain on the next step's kernels do not start while it still reads the lists and rows.
+ */
+typedef struct ppg_agent_state_args {
+  uint8_t* present[2];   /* [row_capacity[s]] required: 1 = present */
+  int32_t* pos[2];       /* [row_capacity[s]][2] x, y */
+  double* energy[2];     /* [row_capacity[s]] */
+  double* trait[2];      /* [row_capacity[s]] ECO family both species, STAG predators */
+  double* acc[2];        /* [row_capacity[s]] cadence variant */
+  int32_t* age[2];       /* [row_capacity[s]] ECO family, STAG */
+  int8_t* facing[2];     /* [row_capacity[s]] STAG predators */
+  int32_t* grass_pos;    /* [n_envs][n_grass][2] x, y */
+  double* grass_energy;  /* [n_envs][n_grass] */
+} ppg_agent_state_args;
+
+/* Writes the columns above into the caller's DEVICE arrays: one kernel launch on cuda_stream, no synchronisation.  A NULL
+ * column pointer (other than present) is not written.
+ * PPG_ERR_INVALID: NULL handle or args, a NULL present[s], or a non-NULL column the variant or species does not have (age on
+ * BASE, trait on BASE or STAG prey, facing other than on STAG predators, acc other than on the cadence variant).
+ * PPG_ERR_STATE: no output since ppg_create, or no output since ppg_restore. */
+int ppg_agent_state(ppg_handle h, const ppg_agent_state_args* a, void* cuda_stream);
+
+/*
  * Episode returns and agent lifetimes on the device (RLlib's episode_return_mean, episode_len_mean,
  * module_episode_returns_mean; the per-life records the evolutionary analyses read).  Off by default: while off nothing is
  * launched, allocated or changed.  While on, every output (ppg_reset without a mask, ppg_step, ppg_step_ordered,

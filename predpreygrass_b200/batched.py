@@ -14,7 +14,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .config import N_EP_STATS, N_STATS, STAT_NAMES, VARIANT_ECO, PpgBuffers, PpgConfig, PpgGaeArgs, PpgReturns, PpgTape
+from .config import (N_EP_STATS, N_STATS, STAT_NAMES, TRAIT_CADENCE, VARIANT_ECO, VARIANT_STAG, PpgAgentStateArgs, PpgBuffers,
+                     PpgConfig, PpgGaeArgs, PpgReturns, PpgTape)
 
 
 class _DevPtr:
@@ -66,6 +67,35 @@ class Returns:
     env_return: torch.Tensor  # f64 [B, 2]: running episode return per species (NaN: env not valid)
     env_valid: torch.Tensor   # uint8 [B]: 1 once the env has been reset since tracking was switched on / a restore
     env_acc: torch.Tensor     # f64 [B, N_EP_STATS]: each env's share of episode_stats_device()
+
+
+@dataclass
+class AgentState:
+    """The state of the agent behind every row of the last output (include/ppg.h ppg_agent_state).  Per-species columns are
+    (pred, prey) pairs of CUDA tensors indexed like the rows; a column the variant or species lacks is None."""
+
+    present: tuple      # uint8 [cap]: 1 = the row's agent is in its env's list after this output
+    pos: tuple          # int32 [cap, 2]: x, y (-1 where absent)
+    energy: tuple       # f64 [cap] (NaN where absent)
+    age: tuple          # int32 [cap] ECO family, STAG (-1 where absent)
+    trait: tuple        # f64 [cap] ECO family (genome speed / the variant's trait), STAG predators (cooperation trait)
+    facing: tuple       # int8 [cap] STAG predators (-1 where absent)
+    acc: tuple          # f64 [cap] cadence variant: move accumulator
+    grass_pos: torch.Tensor     # int32 [B, n_grass, 2] (-1 for an env whose episode ended in this output)
+    grass_energy: torch.Tensor  # f64 [B, n_grass] (NaN for an env whose episode ended in this output)
+
+
+AGENT_STATE_COLUMNS = {"present": ((), torch.uint8), "pos": ((2,), torch.int32), "energy": ((), torch.float64),
+                       "age": ((), torch.int32), "trait": ((), torch.float64), "facing": ((), torch.int8),
+                       "acc": ((), torch.float64)}
+
+
+def agent_state_columns(cfg):
+    """{column: (pred, prey) booleans}: which per-species columns of AgentState the config's variant has"""
+    eco, stag = cfg.variant == VARIANT_ECO, cfg.variant == VARIANT_STAG
+    cad = eco and cfg.trait_mode == TRAIT_CADENCE
+    return {"present": (True, True), "pos": (True, True), "energy": (True, True), "age": (eco or stag, eco or stag),
+            "trait": (eco or stag, eco), "facing": (stag, False), "acc": (cad, cad)}
 
 
 def episode_metrics_from_stats(v):
@@ -336,6 +366,55 @@ class BatchedPredPreyGrass:
             raise ValueError(f"world_state: out must be a contiguous float32 tensor of shape {shape} on {self.device}, got "
                              f"{out.dtype} {tuple(out.shape)} on {out.device} (contiguous={out.is_contiguous()})")
         _lib.check(self.L.ppg_world_state(self.h, int(env_begin), n, out.data_ptr(), self._stream()), self.h)
+        return out
+
+    def new_agent_state(self):
+        """An AgentState of freshly allocated tensors, every column the variant has (for agent_state(out=...))"""
+        d, cap, cols = self.device, self.row_capacity, agent_state_columns(self.cfg)
+        per = {k: tuple(torch.empty((cap[s],) + AGENT_STATE_COLUMNS[k][0], dtype=AGENT_STATE_COLUMNS[k][1], device=d)
+                        if cols[k][s] else None for s in range(2)) for k in cols}
+        ng = self.cfg.n_grass
+        return AgentState(**per, grass_pos=torch.empty((self.n_envs, ng, 2), dtype=torch.int32, device=d),
+                          grass_energy=torch.empty((self.n_envs, ng), dtype=torch.float64, device=d))
+
+    def agent_state(self, out=None):
+        """The state of the agent behind every row of the last output (include/ppg.h ppg_agent_state): one kernel launch on the
+        current stream, no synchronisation.  Without `out` the result is an AgentState of views of buffers this object owns
+        and reuses: valid until the next agent_state() call.  `out` is an AgentState of contiguous CUDA tensors on this
+        device with the shapes and dtypes of new_agent_state(); a per-species column or a grass tensor may be None (not
+        written), except `present`."""
+        if out is None:
+            if getattr(self, "_agent_state", None) is None:
+                self._agent_state = self.new_agent_state()
+            out = self._agent_state
+        cap, cols = self.row_capacity, agent_state_columns(self.cfg)
+
+        def ptr(name, t, dtype, shape):
+            if t is None:
+                return None
+            if (not isinstance(t, torch.Tensor) or t.dtype != dtype or t.device != self.device or not t.is_contiguous()
+                    or tuple(t.shape) != tuple(shape)):
+                got = f"{t.dtype} {tuple(t.shape)} on {t.device} (contiguous={t.is_contiguous()})" if isinstance(t, torch.Tensor) \
+                    else type(t).__name__
+                raise ValueError(f"agent_state: {name} must be a contiguous {dtype} tensor of shape {tuple(shape)} on {self.device}, "
+                                 f"got {got}")
+            return t.data_ptr() or None
+
+        a = PpgAgentStateArgs()
+        for k, (extra, dtype) in AGENT_STATE_COLUMNS.items():
+            pair = getattr(out, k)
+            if not isinstance(pair, (tuple, list)) or len(pair) != 2:
+                raise ValueError(f"agent_state: {k} must be a (pred, prey) pair")
+            for s in range(2):
+                if pair[s] is not None and not cols[k][s]:
+                    raise ValueError(f"agent_state: this variant has no {k} column for species {s}")
+                if k == "present" and pair[s] is None:
+                    raise ValueError("agent_state: present is required")
+                getattr(a, k)[s] = ptr(f"{k}[{s}]", pair[s], dtype, (cap[s],) + extra)
+        ng = self.cfg.n_grass
+        a.grass_pos = ptr("grass_pos", out.grass_pos, torch.int32, (self.n_envs, ng, 2))
+        a.grass_energy = ptr("grass_energy", out.grass_energy, torch.float64, (self.n_envs, ng))
+        _lib.check(self.L.ppg_agent_state(self.h, C.byref(a), self._stream()), self.h)
         return out
 
     def gae(self, gamma, lam, row_agent, flags, reward, value, old_off, new_off, new_cnt, env_flags, adv, value_target, next_row,

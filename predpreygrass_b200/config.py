@@ -200,6 +200,22 @@ class PpgGaeArgs(C.Structure):
     ]
 
 
+class PpgAgentStateArgs(C.Structure):
+    """include/ppg.h ppg_agent_state_args: [s] = species, every pointer a device array (None: column not written)"""
+
+    _fields_ = [
+        ("present", C.c_void_p * 2),
+        ("pos", C.c_void_p * 2),
+        ("energy", C.c_void_p * 2),
+        ("trait", C.c_void_p * 2),
+        ("acc", C.c_void_p * 2),
+        ("age", C.c_void_p * 2),
+        ("facing", C.c_void_p * 2),
+        ("grass_pos", C.c_void_p),
+        ("grass_energy", C.c_void_p),
+    ]
+
+
 GAE_ERR_ID, GAE_ERR_LINK, GAE_ERR_RANGE = 0x1, 0x2, 0x4  # include/ppg.h PPG_GAE_ERR_*
 
 

@@ -51,6 +51,8 @@ cudaError_t launch_episode_stats_clear(double* env_acc, int B, cudaStream_t stre
 // ppg_gae.cu
 cudaError_t launch_gae(const GaeParams& p, cudaStream_t stream);
 int gae_warps(int log2_h);
+// ppg_agent_state.cu
+cudaError_t launch_agent_state(const AgentStateParams& p, cudaStream_t stream);
 }  // namespace ppg
 
 namespace ppg { int g_pdl_chain = -1; }
@@ -81,6 +83,9 @@ struct ppg_handle_s {
   // do the env images in obs_img show the world of the last output (ppg_world_state)?
   enum { IMG_NONE, IMG_VALID, IMG_RESTORED, IMG_RESTORED_IDLE } img = IMG_NONE;
   int n_cta_ws = 0;                      // ppg_world_state grid (0: not computed yet)
+  // do the agent lists and the output buffers describe the same output (ppg_agent_state)?  ppg_restore rewrites the lists
+  // and relabels the rows of an output it did not produce
+  enum { OUT_NONE, OUT_VALID, OUT_RESTORED } out_state = OUT_NONE;
   // episode returns (ppg_track_returns): allocated at the first switch-on
   bool track_on = false;
   ReturnsParams R;
@@ -721,6 +726,7 @@ static int run_step_kernel(ppg_handle h, const int32_t* a0, const int32_t* a1, c
   // the images now hold this output's world, except that an env idle since a ppg_restore still has the pre-restore one:
   // after restoring idle envs only a full reset (a0 == NULL, every env dumps its image) makes them valid again
   if (a0 == nullptr || h->img != ppg_handle_s::IMG_RESTORED_IDLE) h->img = ppg_handle_s::IMG_VALID;
+  h->out_state = ppg_handle_s::OUT_VALID;
   h->calls++;
   h->h_n_rows_valid = false;
   return PPG_OK;
@@ -968,6 +974,7 @@ int ppg_restore(ppg_handle h, const void* blob, size_t bytes, void* cuda_stream)
       idle = hd.state == ST_IDLE;
     }
     h->img = idle ? ppg_handle_s::IMG_RESTORED_IDLE : ppg_handle_s::IMG_RESTORED;
+    h->out_state = ppg_handle_s::OUT_RESTORED;
   }
   for (const Seg& s : state_segments(h)) { CK(cudaMemcpyAsync(s.p, q, s.bytes, cudaMemcpyHostToDevice, st)); q += s.bytes; }
   {
@@ -1120,6 +1127,46 @@ int ppg_world_state(ppg_handle h, int32_t env_begin, int32_t n_envs, float* out,
     h->n_cta_ws = per_sm * n_sm;
   }
   CK(launch_world_state(w, P.map_bytes, std::min(n_envs, h->n_cta_ws), static_cast<cudaStream_t>(cuda_stream)));
+  h->launch_count++;
+  return PPG_OK;
+}
+
+int ppg_agent_state(ppg_handle h, const ppg_agent_state_args* a, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (!a) { h->err = "ppg_agent_state: NULL args"; return PPG_ERR_INVALID; }
+  const StepParams& P = h->P;
+  const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
+  const bool cad = eco && P.trait_mode == PPG_TRAIT_CADENCE;
+  for (int s = 0; s < 2; ++s) {
+    if (!a->present[s]) { h->err = "ppg_agent_state: NULL present"; return PPG_ERR_INVALID; }
+    if (a->age[s] && !(eco || stag)) { h->err = "ppg_agent_state: age: BASE agents have no age"; return PPG_ERR_INVALID; }
+    if (a->trait[s] && !(eco || (stag && s == 0))) { h->err = "ppg_agent_state: trait: only the ECO family and STAG predators have one"; return PPG_ERR_INVALID; }
+    if (a->facing[s] && !(stag && s == 0)) { h->err = "ppg_agent_state: facing: only STAG predators have one"; return PPG_ERR_INVALID; }
+    if (a->acc[s] && !cad) { h->err = "ppg_agent_state: acc: only the cadence variant has a move accumulator"; return PPG_ERR_INVALID; }
+  }
+  switch (h->out_state) {
+    case ppg_handle_s::OUT_NONE: h->err = "ppg_agent_state: no output since ppg_create"; return PPG_ERR_STATE;
+    case ppg_handle_s::OUT_RESTORED: h->err = "ppg_agent_state: no output since ppg_restore"; return PPG_ERR_STATE;
+    default: break;
+  }
+  CK(cudaSetDevice(h->device));
+  AgentStateParams q;
+  memset(&q, 0, sizeof q);
+  q.a = *a;
+  q.hdr = P.hdr;
+  for (int s = 0; s < 2; ++s) {
+    q.ag_id[s] = P.ag_id[s]; q.ag_pos[s] = P.ag_pos[s]; q.ag_e[s] = P.ag_e[s]; q.ag_prow[s] = P.ag_prow[s];
+    if (eco || stag) q.ag_age[s] = P.ag_age[s];
+    q.ag_trait[s] = eco ? P.ag_spd[s] : (stag && s == 0) ? P.ag_trait : nullptr;
+    if (cad) q.ag_acc[s] = P.ag_acc[s];
+    q.row_agent[s] = P.row_agent[s]; q.old_off[s] = P.old_off[s]; q.new_off[s] = P.new_off[s]; q.new_cnt[s] = P.new_cnt[s];
+    q.cap[s] = P.cap[s];
+  }
+  if (stag) q.ag_face = P.ag_face;
+  q.env_flags = P.env_flags;
+  q.gr_pos = P.gr_pos; q.gr_e = P.gr_e;
+  q.n_grass = P.n_grass; q.B = h->B;
+  CK(launch_agent_state(q, static_cast<cudaStream_t>(cuda_stream)));
   h->launch_count++;
   return PPG_OK;
 }

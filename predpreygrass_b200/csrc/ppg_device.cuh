@@ -276,6 +276,30 @@ struct ReturnsParams {
   int B;
 };
 
+// ppg_agent_state_kernel (ppg_agent_state.cu): the state of the agent behind every row of the last output (include/ppg.h
+// ppg_agent_state).  The host resolves each column's source list (nullptr: the column is not written).
+struct AgentStateParams {
+  ppg_agent_state_args a;
+  const EnvHdr* hdr;
+  const uint16_t* ag_id[2];
+  const uint16_t* ag_pos[2];
+  const double* ag_e[2];
+  const int32_t* ag_prow[2];
+  const uint16_t* ag_age[2];    // ECO family, STAG
+  const double* ag_trait[2];    // ECO family: ag_spd[s]; STAG: ag_trait (predators)
+  const uint8_t* ag_face;       // STAG predators
+  const double* ag_acc[2];      // cadence variant
+  const int32_t* row_agent[2];
+  const int32_t* old_off[2];
+  const int32_t* new_off[2];
+  const int32_t* new_cnt[2];
+  const uint8_t* env_flags;
+  const uint16_t* gr_pos;
+  const double* gr_e;
+  int cap[2];
+  int n_grass, B;
+};
+
 // ppg_gae_kernel (ppg_gae.cu): links the rows of a rollout and runs the GAE recursion (include/ppg.h ppg_gae).
 struct GaeParams {
   ppg_gae_args a;
