@@ -105,7 +105,6 @@ struct ppg_handle_s {
   int32_t h_n_rows[4] = {0, 0, 0, 0};
   bool h_n_rows_valid = false;
   ppg_buffers bufs;
-  size_t state_bytes = 0;
   std::string err;
 };
 
@@ -120,15 +119,82 @@ static thread_local std::string g_err;
     }                                                                                        \
   } while (0)
 
+// n elements (at least one) owned by the handle, zeroed unless `clear` is false
 template <typename T>
-static cudaError_t dalloc(ppg_handle h, T** p, size_t n) {
+static cudaError_t dalloc(ppg_handle h, T** p, size_t n, bool clear = true) {
   void* q = nullptr;
   cudaError_t e = cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T));
   if (e != cudaSuccess) return e;
-  e = cudaMemset(q, 0, std::max<size_t>(n, 1) * sizeof(T));
+  if (clear) e = cudaMemset(q, 0, std::max<size_t>(n, 1) * sizeof(T));
   h->allocs.push_back(q);
   *p = static_cast<T*>(q);
   return e;
+}
+
+// a device copy of a host table, owned by the handle
+template <typename T>
+static cudaError_t upload(ppg_handle h, const T** p, const std::vector<T>& v) {
+  T* d = nullptr;
+  cudaError_t e = dalloc(h, &d, v.size());
+  if (e == cudaSuccess) e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+  *p = d;
+  return e;
+}
+
+// one column of a replay tape (include/ppg.h ppg_tape): its entries and the B + 1 offsets into them
+template <typename T>
+static cudaError_t upload_tape(int B, const T* entries, const int64_t* off, T** d, long long** d_off) {
+  const int64_t total = off[B];
+  cudaError_t e = cudaMalloc(d, sizeof(T) * (size_t)std::max<int64_t>(total, 1));
+  if (e == cudaSuccess) e = cudaMalloc(d_off, sizeof(long long) * ((size_t)B + 1));
+  if (e == cudaSuccess) e = cudaMemcpy(*d, entries, sizeof(T) * (size_t)total, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(*d_off, off, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice);
+  return e;
+}
+
+// the first n entries of env `env`'s agent list in column `col` ([B][cap_live[s]]), converted to the caller's type
+template <typename T, typename U>
+static cudaError_t read_list(U* to, const T* col, const StepParams& P, int32_t env, int s, int n) {
+  if (!n) return cudaSuccess;
+  std::vector<T> v((size_t)n);
+  cudaError_t e = cudaMemcpy(v.data(), col + (size_t)env * P.cap[s], sizeof(T) * (size_t)n, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) std::copy(v.begin(), v.end(), to);
+  return e;
+}
+
+// The handle's persistent state: every array a step carries over to the next call, in the order of the snapshot blob.
+// ppg_create allocates by this walk and ppg_snapshot / ppg_restore copy by it, so a new state array is added here and
+// only here.  add(p, n) is called with the pointer slot and the element count; the element size is sizeof *p.  n == 0
+// marks a placeholder the kernels take but never use (ag_par outside kickback): one element is allocated, none is
+// in the blob.  hdr stays first: ppg_restore reads the env headers at the start of the blob.
+template <typename F>
+static void for_each_state_array(ppg_handle h, F&& add) {
+  StepParams& P = h->P;
+  const size_t B = (size_t)h->B, n_grass = (size_t)std::max(1, P.n_grass);
+  const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
+  add(P.hdr, B);
+  for (int s = 0; s < 2; ++s) {
+    const size_t n = B * P.cap[s], m = B * P.n_possible[s];
+    add(P.ag_id[s], n); add(P.ag_pos[s], n); add(P.ag_e[s], n); add(P.ag_prow[s], n);
+    add(P.ag_par[s], P.reward_mode == PPG_REWARD_SPARSE_KICKBACK ? n : 0);
+    if (eco) {
+      add(P.ag_age[s], n); add(P.ag_seq[s], n); add(P.ag_spd[s], n); add(P.ag_dead[s], n);
+      if (P.trait_mode == PPG_TRAIT_CADENCE) add(P.ag_acc[s], n);
+      if (P.lin_on) { add(P.lin_parent[s], m); add(P.lin_live[s], m); add(P.lin_prev[s], m); add(P.lin_alive[s], m); }
+    }
+    if (stag) {
+      add(P.ag_age[s], n);
+      if (s == 0) { add(P.ag_face, n); add(P.ag_trait, n); }
+    }
+  }
+  if (stag) add(P.shdr, B);
+  if (eco) {
+    add(P.ehdr, B);
+    if (h->cfg.track_episode_sums) add(P.ep_sums, B * PPG_EP_STRIDE);
+    add(P.gh_n, B); add(P.gh_cell, B * PPG_MAX_GHOSTS); add(P.gh_val, B * PPG_MAX_GHOSTS);
+  }
+  add(P.gr_pos, B * n_grass); add(P.gr_e, B * n_grass);
+  add(P.counters, B * PPG_N_STATS);
 }
 
 // Which owner map and which value table show grid channel `ch` (so_* offsets): the observation rows (obs_rel) and
@@ -263,8 +329,6 @@ static int validate(const ppg_config* c, int32_t n_envs, std::string& err) {
     // STAG:408-412); the dict adapter appends it on the host, the batched row layout does not carry it
     if (c->include_visibility_channel) { err = "include_visibility_channel: a constant plane of ones in the reference; appended by the dict adapter (PredPreyGrassStag), not part of the batched rows"; return PPG_ERR_INVALID; }
   }
-  if (false) {
-  }
   for (int s = 0; s < 2; ++s) {
     if (c->obs_range[s] < 1 || (c->obs_range[s] & 1) == 0 || c->obs_range[s] > 255) { err = "obs_range must be odd"; return PPG_ERR_INVALID; }
     if ((c->num_obs_channels + (eco && c->include_speed_in_obs ? 1 : 0)) * c->obs_range[s] * c->obs_range[s] > 4 * 128) { err = "observation row too large for this build"; return PPG_ERR_INVALID; }
@@ -280,31 +344,15 @@ static int validate(const ppg_config* c, int32_t n_envs, std::string& err) {
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle* out) {
-  if (!out) return PPG_ERR_INVALID;
-  *out = nullptr;
-  int rc = validate(cfg, n_envs, g_err);
-  if (rc) return rc;
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { g_err = "no CUDA device"; return PPG_ERR_NO_DEVICE; }
-  if (device < 0 || device >= ndev) { g_err = "bad device index"; return PPG_ERR_INVALID; }
-  ppg_handle h = new ppg_handle_s();
-  h->cfg = *cfg;
-  h->walls.assign(cfg->wall_cells, cfg->wall_cells + (cfg->wall_cells ? cfg->n_walls : 0));  // the caller's list is copied
-  h->cfg.wall_cells = h->walls.empty() ? nullptr : h->walls.data();
-  h->B = n_envs;
-  h->device = device;
-  auto fail = [&](int code) { g_err = h->err; ppg_destroy(h); return code; };
-#define CKC(call)                                                                            \
-  do {                                                                                       \
-    cudaError_t _e = (call);                                                                 \
-    if (_e != cudaSuccess) { h->err = std::string(#call) + ": " + cudaGetErrorString(_e); return fail(PPG_ERR_CUDA); } \
-  } while (0)
-  CKC(cudaSetDevice(device));
+static const size_t smem_max = 227 * 1024;  // dynamic shared memory of one CTA on sm_100
+
+// ---- ppg_create, step by step ------------------------------------------------------------------------------------------
+// 1. the configuration's scalars in StepParams
+static void set_step_params(ppg_handle h) {
   const ppg_config& c = h->cfg;
   StepParams& P = h->P;
   memset(&P, 0, sizeof P);
-  const int B = n_envs, G = c.grid_size, GG = G * G;
+  const int B = h->B, G = c.grid_size, GG = G * G;
   const bool eco = c.variant == PPG_VARIANT_ECO, stag = c.variant == PPG_VARIANT_STAG;
   const int row_channels = c.num_obs_channels + (eco && c.include_speed_in_obs ? 1 : 0);
   P.B = B; P.G = G; P.GG = GG; P.C = row_channels; P.env_base = c.env_index_base;
@@ -355,10 +403,16 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
   P.init_e_grass = c.initial_energy_grass;
   P.r_catch = c.reward_predator_catch_prey; P.r_eat = c.reward_prey_eat_grass; P.r_pstep = c.reward_predator_step;
   P.r_qstep = c.reward_prey_step; P.pen_caught = c.penalty_prey_caught;
+}
 
-  const bool dense = c.reward_mode == PPG_REWARD_DENSE || c.reward_mode == PPG_REWARD_DENSE_ADDITIVE;
-  const bool kick = c.reward_mode == PPG_REWARD_SPARSE_KICKBACK;
-
+// 2. padded map geometry, row geometry and the shared-memory slice of one env (see EnvSmem in ppg_base.cu)
+static int layout_smem(ppg_handle h) {
+  StepParams& P = h->P;
+  const int G = P.G, GG = P.GG;
+  const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
+  const bool dense = P.reward_mode == PPG_REWARD_DENSE || P.reward_mode == PPG_REWARD_DENSE_ADDITIVE;
+  const bool kick = P.reward_mode == PPG_REWARD_SPARSE_KICKBACK;
+  // the one experiment switch read before the launch geometry: the slice holds row staging only for the bulk-copy writer
   P.obs_bulk = 0;
   if (const char* ev = getenv("PPG_OBS_BULK")) P.obs_bulk = atoi(ev) != 0;
   // padded map geometry (ppg_base.cu): halo as wide as the largest observation window
@@ -375,9 +429,8 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
     P.emit_kind[s] = (P.obs_vec[s] && P.nj[s] == 8) ? 1 : (P.obs_vec[s] && P.nj[s] == 12) ? 2 : (!P.obs_vec[s] && P.nj[s] == 13) ? 3
                      : (!P.obs_vec[s] && P.nj[s] == 5) ? 4 : (!P.obs_vec[s] && P.nj[s] == 8) ? 5 : 0;
   }
-  if (P.nj[0] > PPG_MAX_NJ || P.nj[1] > PPG_MAX_NJ) { h->err = "observation row too large for this build"; return fail(PPG_ERR_INVALID); }
+  if (P.nj[0] > PPG_MAX_NJ || P.nj[1] > PPG_MAX_NJ) { h->err = "observation row too large for this build"; return PPG_ERR_INVALID; }
 
-  // shared-memory layout of one env (see EnvSmem in ppg_base.cu)
   size_t o = 0;
   auto take = [&](size_t bytes, size_t al) { o = align_up(o, al); size_t r = o; o += bytes; return (int)r; };
   for (int s = 0; s < 2; ++s) { P.so_E[s] = take(8 * (size_t)P.cap[s], 8); P.so_E0[s] = take(dense ? 8 * (size_t)P.cap[s] : 0, 8); }
@@ -405,7 +458,7 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
   }
   // reset() stages its n_total cells in the value tables and a GG-entry claim table over the energy arrays
   if ((size_t)GG * 4 > (size_t)(P.so_vt[0] - P.so_E[0])) {
-    h->err = "internal: reset scratch does not fit (cap_live too small for this grid)"; return fail(PPG_ERR_INVALID);
+    h->err = "internal: reset scratch does not fit (cap_live too small for this grid)"; return PPG_ERR_INVALID;
   }
   // maps, wall table and touch counters are contiguous: their initial contents are one image copied by every warp
   P.so_map[0] = take((size_t)P.map_bytes * P.CH, 16);
@@ -435,69 +488,68 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
     P.so_face = take(P.cap[0], 1); P.so_join = take(P.cap[0], 1);
   }
   P.smem_per_env = (int)align_up(o, 128);
-  const size_t smem_max = 227 * 1024;
-  if ((size_t)P.smem_per_env > smem_max) { h->err = "cap_live/grid too large for shared memory"; return fail(PPG_ERR_INVALID); }
-  {
-    // per-lane gather constants: element q = lane + 32 j of a row is channel c, window cell (i, jj);
-    // BASE channels: 0 = outside the grid (predator map halo -> wall table), 1 predators, 2 prey, 3 grass
-    {
-      std::vector<unsigned char> img((size_t)P.init_bytes, 0);
-      for (int i = 0; i < P.CH; ++i) {
-        const int xx = i >= P.P ? (i - P.P) / P.PS - P.P : -1, yy = i >= P.P ? (i - P.P) % P.PS : 0;
-        const bool field = i >= P.P && xx >= 0 && xx < G && yy < G;
-        if (!field && !eco && !stag) {  // ECO has no wall channel; STAG's wall channel is empty (walls are rejected by the config layer): out-of-grid window cells stay 0 (ECO:700-706)
-          if (P.map_bytes == 1) img[(size_t)i] = (unsigned char)P.wall_idx;
-          else reinterpret_cast<uint16_t*>(img.data())[i] = (uint16_t)P.wall_idx;
-        }
-      }
-      if (!eco && !stag) reinterpret_cast<float*>(img.data() + (P.so_wt - P.so_map[0]))[P.wall_idx] = 1.0f;
-      if (stag && !h->walls.empty()) {  // STAG walls (STAG:2152-2159): static WALL entries of the predator map, shown by channel 0
-        for (int w : h->walls) {
-          const int i = P.P + (w / G + P.P) * P.PS + w % G;
-          if (P.map_bytes == 1) img[(size_t)i] = (unsigned char)P.wall_idx;
-          else reinterpret_cast<uint16_t*>(img.data())[i] = (uint16_t)P.wall_idx;
-        }
-        reinterpret_cast<float*>(img.data() + (P.so_wt - P.so_map[0]))[P.wall_idx] = 1.0f;
-        int32_t* d_w = nullptr;
-        CKC(dalloc(h, &d_w, h->walls.size()));
-        CKC(cudaMemcpy(d_w, h->walls.data(), h->walls.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-        P.wall_cells = d_w;
-      }
-      unsigned char* d_img = nullptr;
-      CKC(dalloc(h, &d_img, img.size()));
-      CKC(cudaMemcpy(d_img, img.data(), img.size(), cudaMemcpyHostToDevice));
-      P.init_image = d_img;
-    }
-    std::vector<int> rel((size_t)2 * PPG_MAX_NJ * 32 * 2, 0);
-    std::vector<unsigned> selfm(64, 0u);
-    for (int s = 0; s < 2; ++s) {
-      const int R = P.R[s], RR = R * R;
-      for (int j = 0; j < P.nj[s]; ++j)
-        for (int lane = 0; lane < 32; ++lane) {
-          const size_t at0 = ((size_t)(s * PPG_MAX_NJ + j) * 32 + lane) * 2;
-          rel[at0] = 0; rel[at0 + 1] = P.so_wt;  // lanes past the end of the row: a harmless in-range read, never stored
-          const int q = P.obs_vec[s] ? 4 * (lane + 32 * (j / 4)) + (j % 4) : j * 32 + lane;
-          if (q >= P.elems[s]) continue;
-          const int ch = q / RR, i = (q % RR) / R, jj = q % R;
-          const int cellrel = (i - P.off[s]) * P.PS + (jj - P.off[s]);
-          const size_t at = ((size_t)(s * PPG_MAX_NJ + j) * 32 + lane) * 2;
-          if (eco && ch >= 3) { selfm[(size_t)s * 32 + lane] |= 1u << j; continue; }  // ECO's own-speed plane
-          const ChannelSource src = channel_source(P, ch);
-          rel[at] = (src.map - P.so_map[0]) + cellrel * P.map_bytes;
-          rel[at + 1] = src.tbl;
-        }
-    }
-    int* d_rel = nullptr;
-    CKC(dalloc(h, &d_rel, rel.size()));
-    CKC(cudaMemcpy(d_rel, rel.data(), rel.size() * sizeof(int), cudaMemcpyHostToDevice));
-    P.obs_rel = reinterpret_cast<const int2*>(d_rel);
-    if (eco) {
-      unsigned* d_self = nullptr;
-      CKC(dalloc(h, &d_self, selfm.size()));
-      CKC(cudaMemcpy(d_self, selfm.data(), selfm.size() * sizeof(unsigned), cudaMemcpyHostToDevice));
-      P.obs_self = d_self;
+  if ((size_t)P.smem_per_env > smem_max) { h->err = "cap_live/grid too large for shared memory"; return PPG_ERR_INVALID; }
+  return PPG_OK;
+}
+
+// 3. the tables the kernels read: the initial image of a slice's maps, the per-lane gather constants of the observation
+//    rows, and the rank of every id string
+static int upload_tables(ppg_handle h) {
+  StepParams& P = h->P;
+  const int G = P.G;
+  const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
+  std::vector<unsigned char> img((size_t)P.init_bytes, 0);
+  for (int i = 0; i < P.CH; ++i) {
+    const int xx = i >= P.P ? (i - P.P) / P.PS - P.P : -1, yy = i >= P.P ? (i - P.P) % P.PS : 0;
+    const bool field = i >= P.P && xx >= 0 && xx < G && yy < G;
+    if (!field && !eco && !stag) {  // ECO has no wall channel; STAG's wall channel is empty (walls are rejected by the config layer): out-of-grid window cells stay 0 (ECO:700-706)
+      if (P.map_bytes == 1) img[(size_t)i] = (unsigned char)P.wall_idx;
+      else reinterpret_cast<uint16_t*>(img.data())[i] = (uint16_t)P.wall_idx;
     }
   }
+  if (!eco && !stag) reinterpret_cast<float*>(img.data() + (P.so_wt - P.so_map[0]))[P.wall_idx] = 1.0f;
+  if (stag && !h->walls.empty()) {  // STAG walls (STAG:2152-2159): static WALL entries of the predator map, shown by channel 0
+    for (int w : h->walls) {
+      const int i = P.P + (w / G + P.P) * P.PS + w % G;
+      if (P.map_bytes == 1) img[(size_t)i] = (unsigned char)P.wall_idx;
+      else reinterpret_cast<uint16_t*>(img.data())[i] = (uint16_t)P.wall_idx;
+    }
+    reinterpret_cast<float*>(img.data() + (P.so_wt - P.so_map[0]))[P.wall_idx] = 1.0f;
+    CK(upload(h, &P.wall_cells, h->walls));
+  }
+  const unsigned char* d_img = nullptr;
+  CK(upload(h, &d_img, img));
+  P.init_image = d_img;
+  // per-lane gather constants: element q = lane + 32 j of a row is channel c, window cell (i, jj)
+  std::vector<int2> rel((size_t)2 * PPG_MAX_NJ * 32, make_int2(0, 0));
+  std::vector<unsigned> selfm(64, 0u);
+  for (int s = 0; s < 2; ++s) {
+    const int R = P.R[s], RR = R * R;
+    for (int j = 0; j < P.nj[s]; ++j)
+      for (int lane = 0; lane < 32; ++lane) {
+        int2& r = rel[(size_t)(s * PPG_MAX_NJ + j) * 32 + lane];
+        r = make_int2(0, P.so_wt);  // lanes past the end of the row: a harmless in-range read, never stored
+        const int q = P.obs_vec[s] ? 4 * (lane + 32 * (j / 4)) + (j % 4) : j * 32 + lane;
+        if (q >= P.elems[s]) continue;
+        const int ch = q / RR, i = (q % RR) / R, jj = q % R;
+        const int cellrel = (i - P.off[s]) * P.PS + (jj - P.off[s]);
+        if (eco && ch >= 3) { selfm[(size_t)s * 32 + lane] |= 1u << j; continue; }  // ECO's own-speed plane
+        const ChannelSource src = channel_source(P, ch);
+        r = make_int2((src.map - P.so_map[0]) + cellrel * P.map_bytes, src.tbl);
+      }
+  }
+  CK(upload(h, &P.obs_rel, rel));
+  if (eco) CK(upload(h, &P.obs_self, selfm));
+  for (int s = 0; s < 2; ++s) CK(upload(h, &P.lexrank[s], lexrank_table(P.n_possible[s])));
+  return PPG_OK;
+}
+
+// 4. launch geometry of the step and observation kernels; every PPG_* experiment switch of a handle except PPG_OBS_BULK
+//    (layout_smem) is read here.  *env_order: the step kernel orders the envs of the next launch big-first (P.perm).
+static int launch_geometry(ppg_handle h, bool* env_order) {
+  StepParams& P = h->P;
+  const int B = h->B;
+  const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
   int W = 1;
   if (const char* ev = getenv("PPG_WARPS_PER_CTA")) W = atoi(ev);
   if (W != 1 && W != 4 && W != 8) W = 1;
@@ -509,91 +561,64 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
   if (W != 1 || P.obs_bulk || P.CH >= (int)DSC_COPY) P.obs_split = 0;
   h->warps_per_cta = W;
   h->smem_bytes = (size_t)W * P.smem_per_env;
-  {
-    // persistent warps: as many CTAs as fit on the device, never more than there are envs
-    int per_sm = 0, n_sm = 0;
-    if (eco) CKC(step_eco_occupancy(P.map_bytes, P.obs_split != 0, P.trait_mode != PPG_TRAIT_SPEED ? 1 : (P.lin_on ? 2 : 0), h->smem_bytes, &per_sm));
-    else if (stag) CKC(step_stag_occupancy(P.map_bytes, P.obs_split != 0, h->smem_bytes, &per_sm));
-    else CKC(step_base_occupancy(W, P.map_bytes, P.obs_bulk != 0, P.obs_split != 0, h->smem_bytes, &per_sm));
-    CKC(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
-    if (per_sm < 1) { h->err = "step kernel does not fit on an SM"; return fail(PPG_ERR_INVALID); }
-    h->n_cta = std::min((B + W - 1) / W, per_sm * n_sm);
-    if (const char* ev = getenv("PPG_MAX_CTAS")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev)));
-  }
-
-  // state
-  CKC(dalloc(h, &P.hdr, (size_t)B));
-  for (int s = 0; s < 2; ++s) {
-    const size_t n = (size_t)B * P.cap[s];
-    CKC(dalloc(h, &P.ag_id[s], n)); CKC(dalloc(h, &P.ag_pos[s], n)); CKC(dalloc(h, &P.ag_e[s], n));
-    CKC(dalloc(h, &P.ag_prow[s], n)); CKC(dalloc(h, &P.ag_par[s], c.reward_mode == PPG_REWARD_SPARSE_KICKBACK ? n : 1));
-    if (eco) {
-      CKC(dalloc(h, &P.ag_age[s], n)); CKC(dalloc(h, &P.ag_seq[s], n)); CKC(dalloc(h, &P.ag_spd[s], n)); CKC(dalloc(h, &P.ag_dead[s], n));
-      if (P.trait_mode == PPG_TRAIT_CADENCE) CKC(dalloc(h, &P.ag_acc[s], n));
-      if (P.lin_on) {
-        const size_t m = (size_t)B * P.n_possible[s];
-        CKC(dalloc(h, &P.lin_parent[s], m)); CKC(dalloc(h, &P.lin_live[s], m)); CKC(dalloc(h, &P.lin_prev[s], m)); CKC(dalloc(h, &P.lin_alive[s], m));
-      }
-    }
-    if (stag) {
-      CKC(dalloc(h, &P.ag_age[s], n));
-      if (s == 0) { CKC(dalloc(h, &P.ag_face, n)); CKC(dalloc(h, &P.ag_trait, n)); }
-    }
-    std::vector<uint16_t> lr = lexrank_table(c.n_possible[s]);
-    uint16_t* d = nullptr;
-    CKC(dalloc(h, &d, lr.size()));
-    CKC(cudaMemcpy(d, lr.data(), lr.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-    P.lexrank[s] = d;
-  }
-  {
-    const size_t n_blk = ((size_t)B + 31) / 32, n_grp = ((size_t)B + 1023) / 1024;
-    for (int q = 0; q < 2; ++q) {
-      CKC(dalloc(h, &P.cntA[q], (size_t)B)); CKC(dalloc(h, &P.cntB[q], (size_t)B));
-      CKC(dalloc(h, &P.sum1[q], n_blk * 4)); CKC(dalloc(h, &P.sum2[q], n_grp * 4));
-    }
-    CKC(dalloc(h, &P.acc1, n_blk * 2)); CKC(dalloc(h, &P.acc2, n_grp * 2)); CKC(dalloc(h, &P.acc3, 2));
-    CKC(dalloc(h, &P.totals, 8));
-    // big-envs-first order of the next launch: only where no env ever waits for another one (publish_begin)
-    bool lpt = !eco && P.obs_split;
-    if (const char* ev = getenv("PPG_ENV_ORDER")) lpt = lpt && atoi(ev) != 0;
-    if (lpt) { for (int q = 0; q < 2; ++q) CKC(dalloc(h, &P.perm[q], (size_t)B)); CKC(dalloc(h, &P.perm_tag, 2)); CKC(dalloc(h, &P.perm_cursor, 4)); CKC(cudaMemset(P.perm_tag, 0xFF, 2 * sizeof(unsigned))); }  // no epoch carries tag 0xFFFFFFFF
-  }
-  if (eco) {
-    CKC(dalloc(h, &P.ehdr, (size_t)B));
-    if (c.track_episode_sums) CKC(dalloc(h, &P.ep_sums, (size_t)B * PPG_EP_STRIDE));
-    CKC(dalloc(h, &P.gh_n, (size_t)B)); CKC(dalloc(h, &P.gh_cell, (size_t)B * PPG_MAX_GHOSTS)); CKC(dalloc(h, &P.gh_val, (size_t)B * PPG_MAX_GHOSTS));
-  }
-  if (stag) CKC(dalloc(h, &P.shdr, (size_t)B));
-  CKC(dalloc(h, &P.gr_pos, (size_t)B * std::max(1, P.n_grass)));
-  CKC(dalloc(h, &P.gr_e, (size_t)B * std::max(1, P.n_grass)));
-  CKC(dalloc(h, &P.counters, (size_t)B * PPG_N_STATS));
-  CKC(dalloc(h, &P.ticket, 1));
-  CKC(dalloc(h, &P.env_cycles, (size_t)B));
+  // persistent warps: as many CTAs as fit on the device, never more than there are envs
+  int per_sm = 0, n_sm = 0;
+  if (eco) CK(step_eco_occupancy(P.map_bytes, P.obs_split != 0, P.trait_mode != PPG_TRAIT_SPEED ? 1 : (P.lin_on ? 2 : 0), h->smem_bytes, &per_sm));
+  else if (stag) CK(step_stag_occupancy(P.map_bytes, P.obs_split != 0, h->smem_bytes, &per_sm));
+  else CK(step_base_occupancy(W, P.map_bytes, P.obs_bulk != 0, P.obs_split != 0, h->smem_bytes, &per_sm));
+  CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device));
+  if (per_sm < 1) { h->err = "step kernel does not fit on an SM"; return PPG_ERR_INVALID; }
+  h->n_cta = std::min((B + W - 1) / W, per_sm * n_sm);
+  if (const char* ev = getenv("PPG_MAX_CTAS")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev)));
+  // big-envs-first order of the next launch: only where no env ever waits for another one (publish_begin)
+  *env_order = !eco && P.obs_split;
+  if (const char* ev = getenv("PPG_ENV_ORDER")) *env_order = *env_order && atoi(ev) != 0;
   if (P.obs_split) {
-    void* q = nullptr;
-    CKC(cudaMalloc(&q, (size_t)B * (size_t)P.img_stride));  // not cleared: every launch writes every env's header
-    h->allocs.push_back(q);
-    P.obs_img = static_cast<unsigned char*>(q);
-    for (int s = 0; s < 2; ++s) CKC(dalloc(h, &P.nb_info[s], (size_t)B * P.cap[s]));
-    CKC(dalloc(h, &P.obs_ticket, 1));
-    CKC(dalloc(h, &P.queue, (size_t)B));
-    CKC(dalloc(h, &P.q_tail, 1));
     if (const char* ev = getenv("PPG_OBS_OVERLAP")) h->obs_overlap = atoi(ev) != 0;
-    if (eco)
-      for (int s = 0; s < 2; ++s) CKC(dalloc(h, &P.born_obs[s], (size_t)B * PPG_BORN_K * (size_t)P.elems[s]));
-    int per_sm = 0, n_sm = 0;
-    CKC(obs_occupancy(P, &per_sm));
-    CKC(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
-    if (per_sm < 1) { h->err = "observation kernel does not fit on an SM"; return fail(PPG_ERR_INVALID); }
+    CK(obs_occupancy(P, &per_sm));
+    if (per_sm < 1) { h->err = "observation kernel does not fit on an SM"; return PPG_ERR_INVALID; }
     h->n_cta_obs = std::min(B, per_sm * n_sm);
     if (const char* ev = getenv("PPG_OBS_CTAS_PER_SM")) h->n_cta_obs = std::max(1, std::min(h->n_cta_obs, atoi(ev) * n_sm));
     // overlap: leave room on every SM for observation CTAs next to the step kernel's persistent warps
     if (const char* ev = getenv("PPG_STEP_CTAS_PER_SM")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev) * n_sm));
   }
-  CKC(dalloc(h, &P.error, 1));
-  CKC(dalloc(h, &h->d_stats, PPG_N_STATS));
-  CKC(dalloc(h, &h->d_mask, (size_t)B));
-  CKC(dalloc(h, &h->d_seeds, (size_t)B));
+  return PPG_OK;
+}
+
+// 5. device memory: the persistent state, the step's scratch, the outputs
+static int allocate(ppg_handle h, bool env_order) {
+  StepParams& P = h->P;
+  const int B = h->B;
+  cudaError_t state = cudaSuccess;
+  for_each_state_array(h, [&](auto*& p, size_t n) { if (state == cudaSuccess) state = dalloc(h, &p, n); });
+  CK(state);
+  const size_t n_blk = ((size_t)B + 31) / 32, n_grp = ((size_t)B + 1023) / 1024;
+  for (int q = 0; q < 2; ++q) {
+    CK(dalloc(h, &P.cntA[q], (size_t)B)); CK(dalloc(h, &P.cntB[q], (size_t)B));
+    CK(dalloc(h, &P.sum1[q], n_blk * 4)); CK(dalloc(h, &P.sum2[q], n_grp * 4));
+  }
+  CK(dalloc(h, &P.acc1, n_blk * 2)); CK(dalloc(h, &P.acc2, n_grp * 2)); CK(dalloc(h, &P.acc3, 2));
+  CK(dalloc(h, &P.totals, 8));
+  if (env_order) {
+    for (int q = 0; q < 2; ++q) CK(dalloc(h, &P.perm[q], (size_t)B));
+    CK(dalloc(h, &P.perm_tag, 2)); CK(dalloc(h, &P.perm_cursor, 4));
+    CK(cudaMemset(P.perm_tag, 0xFF, 2 * sizeof(unsigned)));  // no epoch carries tag 0xFFFFFFFF
+  }
+  CK(dalloc(h, &P.ticket, 1));
+  CK(dalloc(h, &P.env_cycles, (size_t)B));
+  if (P.obs_split) {
+    CK(dalloc(h, &P.obs_img, (size_t)B * (size_t)P.img_stride, false));  // not cleared: every launch writes every env's header
+    for (int s = 0; s < 2; ++s) CK(dalloc(h, &P.nb_info[s], (size_t)B * P.cap[s]));
+    CK(dalloc(h, &P.obs_ticket, 1));
+    CK(dalloc(h, &P.queue, (size_t)B));
+    CK(dalloc(h, &P.q_tail, 1));
+    if (P.variant == PPG_VARIANT_ECO)
+      for (int s = 0; s < 2; ++s) CK(dalloc(h, &P.born_obs[s], (size_t)B * PPG_BORN_K * (size_t)P.elems[s]));
+  }
+  CK(dalloc(h, &P.error, 1));
+  CK(dalloc(h, &h->d_stats, PPG_N_STATS));
+  CK(dalloc(h, &h->d_mask, (size_t)B));
+  CK(dalloc(h, &h->d_seeds, (size_t)B));
   // outputs
   ppg_buffers& b = h->bufs;
   memset(&b, 0, sizeof b);
@@ -601,28 +626,62 @@ int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle
     const size_t rows = (size_t)B * P.cap[s];
     b.row_capacity[s] = (int64_t)rows;
     b.obs_row_elems[s] = P.elems[s];
-    void* q = nullptr;
-    CKC(cudaMalloc(&q, rows * (size_t)P.elems[s] * sizeof(float)));  // not cleared: only valid rows are ever read
-    h->allocs.push_back(q);
-    P.obs[s] = b.obs[s] = static_cast<float*>(q);
-    CKC(dalloc(h, &P.row_env[s], rows)); CKC(dalloc(h, &P.row_agent[s], rows));
-    CKC(dalloc(h, &P.reward[s], rows)); CKC(dalloc(h, &P.flags[s], rows));
-    CKC(dalloc(h, &P.old_off[s], (size_t)B + 1)); CKC(dalloc(h, &P.new_off[s], (size_t)B + 1));
-    CKC(dalloc(h, &P.new_cnt[s], (size_t)B + 1));
-    CKC(dalloc(h, &h->d_act[s], rows));
-    b.row_env[s] = P.row_env[s]; b.row_agent[s] = P.row_agent[s]; b.reward[s] = P.reward[s]; b.flags[s] = P.flags[s];
+    CK(dalloc(h, &P.obs[s], rows * (size_t)P.elems[s], false));  // not cleared: only valid rows are ever read
+    CK(dalloc(h, &P.row_env[s], rows)); CK(dalloc(h, &P.row_agent[s], rows));
+    CK(dalloc(h, &P.reward[s], rows)); CK(dalloc(h, &P.flags[s], rows));
+    CK(dalloc(h, &P.old_off[s], (size_t)B + 1)); CK(dalloc(h, &P.new_off[s], (size_t)B + 1));
+    CK(dalloc(h, &P.new_cnt[s], (size_t)B + 1));
+    CK(dalloc(h, &h->d_act[s], rows));
+    b.obs[s] = P.obs[s]; b.row_env[s] = P.row_env[s]; b.row_agent[s] = P.row_agent[s]; b.reward[s] = P.reward[s]; b.flags[s] = P.flags[s];
     b.old_off[s] = P.old_off[s]; b.new_off[s] = P.new_off[s]; b.new_cnt[s] = P.new_cnt[s];
   }
-  CKC(dalloc(h, &P.n_rows, 4)); CKC(dalloc(h, &P.env_flags, (size_t)B)); CKC(dalloc(h, &P.env_status, (size_t)B));
-  CKC(dalloc(h, &P.env_step, (size_t)B)); CKC(dalloc(h, &P.env_count, (size_t)B * 2));
+  CK(dalloc(h, &P.n_rows, 4)); CK(dalloc(h, &P.env_flags, (size_t)B)); CK(dalloc(h, &P.env_status, (size_t)B));
+  CK(dalloc(h, &P.env_step, (size_t)B)); CK(dalloc(h, &P.env_count, (size_t)B * 2));
   b.n_rows = P.n_rows; b.env_flags = P.env_flags; b.env_status = P.env_status; b.env_step = P.env_step; b.env_count = P.env_count;
   b.n_envs = B;
-  CKC(launch_init_hdr(P.hdr, B, c.seed, 0));
+  return PPG_OK;
+}
+
+static int init_handle(ppg_handle h) {
+  CK(cudaSetDevice(h->device));
+  set_step_params(h);
+  bool env_order = false;
+  int rc = layout_smem(h);
+  if (!rc) rc = upload_tables(h);
+  if (!rc) rc = launch_geometry(h, &env_order);
+  if (!rc) rc = allocate(h, env_order);
+  if (rc) return rc;
+  CK(launch_init_hdr(h->P.hdr, h->B, h->cfg.seed, 0));
   h->launch_count++;
-  CKC(cudaDeviceSynchronize());
+  CK(cudaDeviceSynchronize());
+  return PPG_OK;
+}
+
+int ppg_create(const ppg_config* cfg, int32_t n_envs, int32_t device, ppg_handle* out) {
+  if (!out) return PPG_ERR_INVALID;
+  *out = nullptr;
+  int rc = validate(cfg, n_envs, g_err);
+  if (rc) return rc;
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { g_err = "no CUDA device"; return PPG_ERR_NO_DEVICE; }
+  if (device < 0 || device >= ndev) { g_err = "bad device index"; return PPG_ERR_INVALID; }
+  ppg_handle h = new ppg_handle_s();
+  h->cfg = *cfg;
+  h->walls.assign(cfg->wall_cells, cfg->wall_cells + (cfg->wall_cells ? cfg->n_walls : 0));  // the caller's list is copied
+  h->cfg.wall_cells = h->walls.empty() ? nullptr : h->walls.data();
+  h->B = n_envs;
+  h->device = device;
+  rc = init_handle(h);
+  if (rc) { g_err = h->err; ppg_destroy(h); return rc; }
   *out = h;
   return PPG_OK;
-#undef CKC
+}
+
+// the replay tape lives outside `allocs`: ppg_load_tape replaces it
+static void free_tape(ppg_handle h) {
+  cudaFree(h->d_tape_cells); cudaFree(h->d_tape_off); cudaFree(h->d_tape_reals); cudaFree(h->d_tape_real_off);
+  h->d_tape_cells = nullptr; h->d_tape_off = nullptr; h->d_tape_reals = nullptr; h->d_tape_real_off = nullptr;
+  h->P.tape_cells = nullptr; h->P.tape_reals = nullptr;
 }
 
 int ppg_destroy(ppg_handle h) {
@@ -630,10 +689,7 @@ int ppg_destroy(ppg_handle h) {
   cudaSetDevice(h->device);
   for (void* p : h->allocs) cudaFree(p);
   for (cudaEvent_t e : h->prof_events) cudaEventDestroy(e);
-  if (h->d_tape_cells) cudaFree(h->d_tape_cells);
-  if (h->d_tape_off) cudaFree(h->d_tape_off);
-  if (h->d_tape_reals) cudaFree(h->d_tape_reals);
-  if (h->d_tape_real_off) cudaFree(h->d_tape_real_off);
+  free_tape(h);
   delete h;
   return PPG_OK;
 }
@@ -642,29 +698,16 @@ int ppg_load_tape(ppg_handle h, const ppg_tape* t) {
   if (!h) return PPG_ERR_INVALID;
   CK(cudaSetDevice(h->device));
   CK(cudaDeviceSynchronize());
-  if (h->d_tape_cells) { cudaFree(h->d_tape_cells); h->d_tape_cells = nullptr; }
-  if (h->d_tape_off) { cudaFree(h->d_tape_off); h->d_tape_off = nullptr; }
-  h->P.tape_cells = nullptr;
+  free_tape(h);
   if (t && t->cells && t->cell_off) {
-    const int64_t total = t->cell_off[h->B];
-    CK(cudaMalloc(&h->d_tape_cells, sizeof(int32_t) * (size_t)std::max<int64_t>(total, 1)));
-    CK(cudaMalloc(&h->d_tape_off, sizeof(long long) * ((size_t)h->B + 1)));
-    CK(cudaMemcpy(h->d_tape_cells, t->cells, sizeof(int32_t) * (size_t)total, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(h->d_tape_off, t->cell_off, sizeof(long long) * ((size_t)h->B + 1), cudaMemcpyHostToDevice));
+    CK(upload_tape(h->B, t->cells, t->cell_off, &h->d_tape_cells, &h->d_tape_off));
     h->P.tape_cells = h->d_tape_cells;
   }
   CK(launch_set_tape(h->P.hdr, h->B, h->d_tape_off, 0));
   h->launch_count++;
   if (h->P.variant == PPG_VARIANT_ECO || h->P.variant == PPG_VARIANT_STAG) {
-    if (h->d_tape_reals) { cudaFree(h->d_tape_reals); h->d_tape_reals = nullptr; }
-    if (h->d_tape_real_off) { cudaFree(h->d_tape_real_off); h->d_tape_real_off = nullptr; }
-    h->P.tape_reals = nullptr;
     if (t && t->reals && t->real_off) {
-      const int64_t total = t->real_off[h->B];
-      CK(cudaMalloc(&h->d_tape_reals, sizeof(double) * (size_t)std::max<int64_t>(total, 1)));
-      CK(cudaMalloc(&h->d_tape_real_off, sizeof(long long) * ((size_t)h->B + 1)));
-      CK(cudaMemcpy(h->d_tape_reals, t->reals, sizeof(double) * (size_t)total, cudaMemcpyHostToDevice));
-      CK(cudaMemcpy(h->d_tape_real_off, t->real_off, sizeof(long long) * ((size_t)h->B + 1), cudaMemcpyHostToDevice));
+      CK(upload_tape(h->B, t->reals, t->real_off, &h->d_tape_reals, &h->d_tape_real_off));
       h->P.tape_reals = h->d_tape_reals;
     }
     if (h->P.variant == PPG_VARIANT_ECO) CK(launch_set_tape_reals(h->P.ehdr, h->B, h->d_tape_real_off, 0));
@@ -887,36 +930,8 @@ int ppg_get_buffers(ppg_handle h, ppg_buffers* out) {
 // ---- snapshot / restore: the SoA slab as one host blob -----------------------------------------
 struct Seg { void* p; size_t bytes; };
 static std::vector<Seg> state_segments(ppg_handle h) {
-  const StepParams& P = h->P;
   std::vector<Seg> v;
-  v.push_back({P.hdr, sizeof(EnvHdr) * (size_t)h->B});
-  for (int s = 0; s < 2; ++s) {
-    const size_t n = (size_t)h->B * P.cap[s];
-    v.push_back({P.ag_id[s], n * 2}); v.push_back({P.ag_pos[s], n * 2}); v.push_back({P.ag_e[s], n * 8});
-    v.push_back({P.ag_prow[s], n * 4});
-    if (P.reward_mode == PPG_REWARD_SPARSE_KICKBACK) v.push_back({P.ag_par[s], n * 2});
-    if (P.variant == PPG_VARIANT_ECO) {
-      v.push_back({P.ag_age[s], n * 2}); v.push_back({P.ag_seq[s], n * 2}); v.push_back({P.ag_spd[s], n * 8}); v.push_back({P.ag_dead[s], n});
-      if (P.trait_mode == PPG_TRAIT_CADENCE) v.push_back({P.ag_acc[s], n * 8});
-      if (P.lin_on) {
-        const size_t m = (size_t)h->B * P.n_possible[s];
-        v.push_back({P.lin_parent[s], m * 2}); v.push_back({P.lin_live[s], m * 2}); v.push_back({P.lin_prev[s], m * 2}); v.push_back({P.lin_alive[s], m});
-      }
-    }
-    if (P.variant == PPG_VARIANT_STAG) {
-      v.push_back({P.ag_age[s], n * 2});
-      if (s == 0) { v.push_back({P.ag_face, n}); v.push_back({P.ag_trait, n * 8}); }
-    }
-  }
-  if (P.variant == PPG_VARIANT_STAG) v.push_back({P.shdr, sizeof(StagHdr) * (size_t)h->B});
-  if (P.variant == PPG_VARIANT_ECO) {
-    v.push_back({P.ehdr, sizeof(EcoHdr) * (size_t)h->B});
-    if (P.ep_sums) v.push_back({P.ep_sums, (size_t)h->B * PPG_EP_STRIDE * 8});
-    v.push_back({P.gh_n, (size_t)h->B}); v.push_back({P.gh_cell, (size_t)h->B * PPG_MAX_GHOSTS * 2}); v.push_back({P.gh_val, (size_t)h->B * PPG_MAX_GHOSTS * 4});
-  }
-  v.push_back({P.gr_pos, (size_t)h->B * std::max(1, P.n_grass) * 2});
-  v.push_back({P.gr_e, (size_t)h->B * std::max(1, P.n_grass) * 8});
-  v.push_back({P.counters, (size_t)h->B * PPG_N_STATS * 4});
+  for_each_state_array(h, [&](auto*& p, size_t n) { if (n) v.push_back({p, n * sizeof *p}); });
   return v;
 }
 
@@ -1171,14 +1186,24 @@ int ppg_agent_state(ppg_handle h, const ppg_agent_state_args* a, void* cuda_stre
   return PPG_OK;
 }
 
-int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, int32_t* xy_pred, double* energy_pred,
-                 int32_t* ids_prey, int32_t* xy_prey, double* energy_prey, int32_t* xy_grass, double* energy_grass) {
-  if (!h || env < 0 || env >= h->B || !n_live) return PPG_ERR_INVALID;
+// Start of every per-env reader: the env index is checked, a reader the handle lacks fails with the message
+// `unsupported` (nullptr: supported), every queued call has finished, and the env's header is copied to *hd (if given).
+static int read_begin(ppg_handle h, int32_t env, const char* unsupported, EnvHdr* hd) {
+  if (env < 0 || env >= h->B) return PPG_ERR_INVALID;
+  if (unsupported) { h->err = unsupported; return PPG_ERR_STATE; }
   CK(cudaSetDevice(h->device));
   CK(cudaDeviceSynchronize());
-  const StepParams& P = h->P;
+  if (hd) CK(cudaMemcpy(hd, h->P.hdr + env, sizeof *hd, cudaMemcpyDeviceToHost));
+  return PPG_OK;
+}
+
+int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, int32_t* xy_pred, double* energy_pred,
+                 int32_t* ids_prey, int32_t* xy_prey, double* energy_prey, int32_t* xy_grass, double* energy_grass) {
+  if (!h || !n_live) return PPG_ERR_INVALID;
   EnvHdr hd;
-  CK(cudaMemcpy(&hd, P.hdr + env, sizeof hd, cudaMemcpyDeviceToHost));
+  int rc = read_begin(h, env, nullptr, &hd);
+  if (rc) return rc;
+  const StepParams& P = h->P;
   int32_t* ids[2] = {ids_pred, ids_prey};
   int32_t* xy[2] = {xy_pred, xy_prey};
   double* en[2] = {energy_pred, energy_prey};
@@ -1187,12 +1212,9 @@ int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, 
     n_live[s] = n;
     std::vector<uint16_t> id(std::max(n, 1)), pos(std::max(n, 1));
     std::vector<double> e(std::max(n, 1));
-    const size_t b = (size_t)env * P.cap[s];
-    if (n) {
-      CK(cudaMemcpy(id.data(), P.ag_id[s] + b, n * 2, cudaMemcpyDeviceToHost));
-      CK(cudaMemcpy(pos.data(), P.ag_pos[s] + b, n * 2, cudaMemcpyDeviceToHost));
-      CK(cudaMemcpy(e.data(), P.ag_e[s] + b, n * 8, cudaMemcpyDeviceToHost));
-    }
+    CK(read_list(id.data(), P.ag_id[s], P, env, s, n));
+    CK(read_list(pos.data(), P.ag_pos[s], P, env, s, n));
+    CK(read_list(e.data(), P.ag_e[s], P, env, s, n));
     // report in agent_positions insertion order = ascending id (BASE:190-200,401)
     std::vector<int> order(n);
     for (int i = 0; i < n; ++i) order[i] = i;
@@ -1221,57 +1243,42 @@ int ppg_read_env(ppg_handle h, int32_t env, int32_t* n_live, int32_t* ids_pred, 
 
 int ppg_read_env_eco(ppg_handle h, int32_t env, int32_t* age_pred, double* speed_pred, int32_t* age_prey, double* speed_prey,
                      uint8_t* dead_prey, int32_t* active_num) {
-  if (!h || env < 0 || env >= h->B) return PPG_ERR_INVALID;
-  if (h->P.variant != PPG_VARIANT_ECO) { h->err = "ppg_read_env_eco: not an ECO handle"; return PPG_ERR_STATE; }
-  CK(cudaSetDevice(h->device));
-  CK(cudaDeviceSynchronize());
-  const StepParams& P = h->P;
+  if (!h) return PPG_ERR_INVALID;
   EnvHdr hd;
+  int rc = read_begin(h, env, h->P.variant != PPG_VARIANT_ECO ? "ppg_read_env_eco: not an ECO handle" : nullptr, &hd);
+  if (rc) return rc;
+  const StepParams& P = h->P;
   EcoHdr eh;
-  CK(cudaMemcpy(&hd, P.hdr + env, sizeof hd, cudaMemcpyDeviceToHost));
   CK(cudaMemcpy(&eh, P.ehdr + env, sizeof eh, cudaMemcpyDeviceToHost));
   int32_t* age[2] = {age_pred, age_prey};
   double* sp[2] = {speed_pred, speed_prey};
   for (int s = 0; s < 2; ++s) {  // the device list is in ascending id order = the order of ppg_read_env
-    const int n = hd.n_list[s];
-    if (!n) continue;
-    std::vector<uint16_t> a(n);
-    std::vector<double> v(n);
-    std::vector<uint8_t> d(n);
-    const size_t b = (size_t)env * P.cap[s];
-    CK(cudaMemcpy(a.data(), P.ag_age[s] + b, n * 2, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(v.data(), P.ag_spd[s] + b, n * 8, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(d.data(), P.ag_dead[s] + b, n, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < n; ++i) {
-      if (age[s]) age[s][i] = a[i];
-      if (sp[s]) sp[s][i] = v[i];
-      if (s == 1 && dead_prey) dead_prey[i] = d[i];
-    }
+    if (age[s]) CK(read_list(age[s], P.ag_age[s], P, env, s, hd.n_list[s]));
+    if (sp[s]) CK(read_list(sp[s], P.ag_spd[s], P, env, s, hd.n_list[s]));
   }
+  if (dead_prey) CK(read_list(dead_prey, P.ag_dead[1], P, env, 1, hd.n_list[1]));
   if (active_num) { active_num[0] = eh.active[0]; active_num[1] = eh.active[1]; }
   return PPG_OK;
 }
 
 int ppg_read_env_acc(ppg_handle h, int32_t env, double* acc_pred, double* acc_prey) {
-  if (!h || env < 0 || env >= h->B) return PPG_ERR_INVALID;
-  if (h->P.variant != PPG_VARIANT_ECO || h->P.trait_mode != PPG_TRAIT_CADENCE) { h->err = "ppg_read_env_acc: not a cadence handle"; return PPG_ERR_STATE; }
-  CK(cudaSetDevice(h->device));
-  CK(cudaDeviceSynchronize());
+  if (!h) return PPG_ERR_INVALID;
+  const bool cad = h->P.variant == PPG_VARIANT_ECO && h->P.trait_mode == PPG_TRAIT_CADENCE;
   EnvHdr hd;
-  CK(cudaMemcpy(&hd, h->P.hdr + env, sizeof hd, cudaMemcpyDeviceToHost));
+  int rc = read_begin(h, env, cad ? nullptr : "ppg_read_env_acc: not a cadence handle", &hd);
+  if (rc) return rc;
   double* out[2] = {acc_pred, acc_prey};
   for (int s = 0; s < 2; ++s)
-    if (hd.n_list[s] && out[s]) CK(cudaMemcpy(out[s], h->P.ag_acc[s] + (size_t)env * h->P.cap[s], sizeof(double) * hd.n_list[s], cudaMemcpyDeviceToHost));
+    if (out[s]) CK(read_list(out[s], h->P.ag_acc[s], h->P, env, s, hd.n_list[s]));
   return PPG_OK;
 }
 
 int ppg_read_episode_eco(ppg_handle h, int32_t env, double* sums, int32_t* spawned) {
-  if (!h || env < 0 || env >= h->B) return PPG_ERR_INVALID;
-  if (h->P.variant != PPG_VARIANT_ECO || !h->P.ep_sums) { h->err = "ppg_read_episode_eco: needs an ECO handle created with track_episode_sums"; return PPG_ERR_STATE; }
-  CK(cudaSetDevice(h->device));
-  CK(cudaDeviceSynchronize());
+  if (!h) return PPG_ERR_INVALID;
+  const bool tracked = h->P.variant == PPG_VARIANT_ECO && h->P.ep_sums;
   EnvHdr hd;
-  CK(cudaMemcpy(&hd, h->P.hdr + env, sizeof hd, cudaMemcpyDeviceToHost));
+  int rc = read_begin(h, env, tracked ? nullptr : "ppg_read_episode_eco: needs an ECO handle created with track_episode_sums", &hd);
+  if (rc) return rc;
   if (sums) CK(cudaMemcpy(sums, h->P.ep_sums + (size_t)env * PPG_EP_STRIDE, 4 * sizeof(double), cudaMemcpyDeviceToHost));
   // ids are handed out in order and never reused (ECO:260-272): spawned = ids used - founders of the running episode
   const bool rf = ppg_random_founders(h->P.trait_mode);
@@ -1280,45 +1287,28 @@ int ppg_read_episode_eco(ppg_handle h, int32_t env, double* sums, int32_t* spawn
 }
 
 int ppg_read_episode_events_eco(ppg_handle h, int32_t env, double* events) {
-  if (!h || env < 0 || env >= h->B || !events) return PPG_ERR_INVALID;
-  if (h->P.variant != PPG_VARIANT_ECO || !h->P.ep_sums) { h->err = "ppg_read_episode_events_eco: needs an ECO handle created with track_episode_sums"; return PPG_ERR_STATE; }
-  CK(cudaSetDevice(h->device));
-  CK(cudaDeviceSynchronize());
+  if (!h || !events) return PPG_ERR_INVALID;
+  const bool tracked = h->P.variant == PPG_VARIANT_ECO && h->P.ep_sums;
+  int rc = read_begin(h, env, tracked ? nullptr : "ppg_read_episode_events_eco: needs an ECO handle created with track_episode_sums", nullptr);
+  if (rc) return rc;
   CK(cudaMemcpy(events, h->P.ep_sums + (size_t)env * PPG_EP_STRIDE + PPG_EP_BLOCKED_CAPACITY, 6 * sizeof(double), cudaMemcpyDeviceToHost));
   return PPG_OK;
 }
 
 int ppg_read_env_stag(ppg_handle h, int32_t env, int32_t* age_pred, int32_t* facing_pred, double* trait_pred, int32_t* age_prey,
                       int64_t* capture, double* capture_real) {
-  if (!h || env < 0 || env >= h->B) return PPG_ERR_INVALID;
-  if (h->P.variant != PPG_VARIANT_STAG) { h->err = "ppg_read_env_stag: not a STAG handle"; return PPG_ERR_STATE; }
-  CK(cudaSetDevice(h->device));
-  CK(cudaDeviceSynchronize());
-  const StepParams& P = h->P;
+  if (!h) return PPG_ERR_INVALID;
   EnvHdr hd;
+  int rc = read_begin(h, env, h->P.variant != PPG_VARIANT_STAG ? "ppg_read_env_stag: not a STAG handle" : nullptr, &hd);
+  if (rc) return rc;
+  const StepParams& P = h->P;
   StagHdr sh;
-  CK(cudaMemcpy(&hd, P.hdr + env, sizeof hd, cudaMemcpyDeviceToHost));
   CK(cudaMemcpy(&sh, P.shdr + env, sizeof sh, cudaMemcpyDeviceToHost));
   int32_t* age[2] = {age_pred, age_prey};
-  for (int s = 0; s < 2; ++s) {  // the device list is in insertion order = the order of ppg_read_env
-    const int n = hd.n_list[s];
-    if (!n) continue;
-    std::vector<uint16_t> a(n);
-    const size_t b = (size_t)env * P.cap[s];
-    CK(cudaMemcpy(a.data(), P.ag_age[s] + b, n * 2, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < n; ++i)
-      if (age[s]) age[s][i] = a[i];
-    if (s == 0) {
-      std::vector<uint8_t> f(n);
-      std::vector<double> t(n);
-      CK(cudaMemcpy(f.data(), P.ag_face + b, n, cudaMemcpyDeviceToHost));
-      CK(cudaMemcpy(t.data(), P.ag_trait + b, n * 8, cudaMemcpyDeviceToHost));
-      for (int i = 0; i < n; ++i) {
-        if (facing_pred) facing_pred[i] = f[i];
-        if (trait_pred) trait_pred[i] = t[i];
-      }
-    }
-  }
+  for (int s = 0; s < 2; ++s)  // the device list is in insertion order = the order of ppg_read_env
+    if (age[s]) CK(read_list(age[s], P.ag_age[s], P, env, s, hd.n_list[s]));
+  if (facing_pred) CK(read_list(facing_pred, P.ag_face, P, env, 0, hd.n_list[0]));
+  if (trait_pred) CK(read_list(trait_pred, P.ag_trait, P, env, 0, hd.n_list[0]));
   if (capture) for (int k = 0; k < 12; ++k) capture[k] = sh.capture[k];
   if (capture_real) for (int k = 0; k < 3; ++k) capture_real[k] = sh.capture_real[k];
   return PPG_OK;
