@@ -458,6 +458,47 @@ typedef struct ppg_agent_state_args {
 int ppg_agent_state(ppg_handle h, const ppg_agent_state_args* a, void* cuda_stream);
 
 /*
+ * Row links between consecutive outputs (what a recurrent actor needs to carry each agent's hidden state from its row in one
+ * output to its row in the next).  Off by default: while off nothing is launched or allocated.  While on, every output
+ * (ppg_step, ppg_step_ordered, ppg_step_host, ppg_reset without a mask, every step of ppg_rollout_random; the two-kernel and
+ * the one-kernel step alike) is followed by one more kernel on the same stream that writes, for every row r of species s of
+ * that output:
+ *
+ *   prev_row[s][r] (int32): for an old row (r in [old_off[e], old_off[e+1])) that is not flagged PPG_ROW_FOUNDER, in an env
+ *     whose output does not have PPG_ENV_RESET, the row of the previous output from which the step took this agent's action:
+ *     the row of the same (env, row_agent) (STAG: the same flat id) in the previous output.  Every other row gets -1:
+ *     newborn rows, FOUNDER rows and every row of an env reset by this output (automatic, masked or full reset).  Rows at or
+ *     beyond the output's row count are not written.
+ *   For two consecutive outputs t and t+1 it is exactly the inverse of ppg_gae's next_row:
+ *     prev_row[t+1][r'] == r  <=>  next_row[t][r] == r'.
+ *   "Previous output": the output before this one, as ppg_get_buffers showed it.  For the first output after ppg_restore it is
+ *     the output ppg_restore leaves in the buffers (the snapshot's live agents, laid out by the restore): the rows the restored
+ *     lists point at, from which that step reads its actions.  Switched on at any point, links hold from the next output on.
+ *     A masked ppg_reset only schedules resets and changes nothing here.
+ *
+ * Kernel: one warp per env.  Per species it looks each old, non-FOUNDER row's id up in an id -> row table of the env saved
+ * after the previous output, writes prev_row, then (after __syncwarp) saves the table anew from the env's agent lists
+ * (ids, the row each agent's next action is read from, the list length): after an output they hold exactly (id, row in this
+ * output) of every agent that can act next.  The table is the open-addressing hash of ppg_gae (4 bytes x the next power of
+ * two >= 2 * cap_live[s] per env and species): it grows with cap_live, never with n_possible.  ppg_track_links and
+ * ppg_restore fill the tables from the lists (same kernel, save only), so nothing of this is in the snapshot blob.  No
+ * atomics on results; launched with plain stream order after the observation kernel, it never triggers dependent launches,
+ * so with the launch chain on the next step does not rewrite the lists while it reads them.  Malformed state does not fault:
+ * the kernel ORs the bits below into a sticky device word of the handle (cleared when the state is allocated; the caller may
+ * clear it) and leaves the affected rows at -1.
+ */
+#define PPG_LINK_ERR_MISSING 0x1u  /* an old, non-FOUNDER row's id is not in its env's table */
+#define PPG_LINK_ERR_OVERFLOW 0x2u /* a table ran full while being saved */
+
+/* Switches links on (on != 0) or off.  The first switch-on allocates prev_row (row capacity) and the tables; switching on
+ * while off fills the tables from the current lists (one kernel launch on cuda_stream); switching on while on changes
+ * nothing.  Switching off keeps the allocation.  PPG_ERR_CUDA if the allocation fails. */
+int ppg_track_links(ppg_handle h, int32_t on, void* cuda_stream);
+/* prev_row[2] receives the device arrays [row_capacity[s]], *error the device word of PPG_LINK_ERR_* bits; valid until
+ * ppg_destroy.  PPG_ERR_STATE while links are off, and before the first output after the switch-on or after ppg_restore. */
+int ppg_get_links(ppg_handle h, int32_t** prev_row, uint32_t** error);
+
+/*
  * Episode returns and agent lifetimes on the device (RLlib's episode_return_mean, episode_len_mean,
  * module_episode_returns_mean; the per-life records the evolutionary analyses read).  Off by default: while off nothing is
  * launched, allocated or changed.  While on, every output (ppg_reset without a mask, ppg_step, ppg_step_ordered,

@@ -18,7 +18,7 @@ SYMBOLS = [
     "ppg_read_env", "ppg_read_env_eco", "ppg_read_env_stag", "ppg_stats", "ppg_stats_device", "ppg_stats_clear", "ppg_launch_count", "ppg_last_error",
     "ppg_profile_begin", "ppg_profile_end", "ppg_profile_env_cycles", "ppg_rollout_random", "ppg_selftest_pow", "ppg_read_episode_eco", "ppg_read_episode_events_eco", "ppg_read_env_acc", "ppg_set_pdl_chain",
     "ppg_world_state", "ppg_track_returns", "ppg_get_returns", "ppg_episode_stats_device", "ppg_episode_stats_clear",
-    "ppg_gae", "ppg_agent_state",
+    "ppg_gae", "ppg_agent_state", "ppg_track_links", "ppg_get_links",
 ]
 
 _lib = None
@@ -74,6 +74,8 @@ def load():
     L.ppg_episode_stats_clear.argtypes = [vp, vp]
     L.ppg_gae.argtypes = [vp, C.POINTER(PpgGaeArgs), vp]
     L.ppg_agent_state.argtypes = [vp, C.POINTER(PpgAgentStateArgs), vp]
+    L.ppg_track_links.argtypes = [vp, i32, vp]
+    L.ppg_get_links.argtypes = [vp, C.POINTER(vp * 2), C.POINTER(vp)]
     L.ppg_stats.argtypes = [vp, vp, vp]
     L.ppg_stats_device.argtypes = [vp, C.POINTER(vp), vp]
     L.ppg_stats_clear.argtypes = [vp, vp]

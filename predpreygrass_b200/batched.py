@@ -417,6 +417,29 @@ class BatchedPredPreyGrass:
         _lib.check(self.L.ppg_agent_state(self.h, C.byref(a), self._stream()), self.h)
         return out
 
+    # ------------------------------------------------------------------ row links (include/ppg.h ppg_track_links)
+    def track_links(self, on=True):
+        """Switch row links on or off.  Switched on, every output from the next one on is linked to the output before it:
+        prev_row() then maps each of its rows to the row of the same agent in the previous output."""
+        _lib.check(self.L.ppg_track_links(self.h, 1 if on else 0, self._stream()), self.h)
+
+    def _links(self):
+        rows, err = (C.c_void_p * 2)(), C.c_void_p()
+        _lib.check(self.L.ppg_get_links(self.h, C.byref(rows), C.byref(err)), self.h)
+        return rows, err
+
+    def prev_row(self):
+        """(pred, prey) int32 CUDA views [cap] aligned with the rows of the last output: the row of the previous output this
+        row's agent acted from, -1 for newborn and founder rows (first n rows valid; valid until the next output).  PpgError
+        while links are off, and before the first output after track_links() or restore()."""
+        rows, _ = self._links()
+        return tuple(_view(rows[s], (self.row_capacity[s],), torch.int32, self.device) for s in range(2))
+
+    def links_error(self):
+        """int32 CUDA view [1] of the sticky PPG_LINK_ERR_* word (config.LINK_ERR_*); a caller may zero it"""
+        _, err = self._links()
+        return _view(err.value, (1,), torch.int32, self.device)
+
     def gae(self, gamma, lam, row_agent, flags, reward, value, old_off, new_off, new_cnt, env_flags, adv, value_target, next_row,
             error):
         """GAE advantages and value targets of a recorded rollout (include/ppg.h ppg_gae): one kernel launch on the current

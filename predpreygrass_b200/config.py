@@ -217,6 +217,7 @@ class PpgAgentStateArgs(C.Structure):
 
 
 GAE_ERR_ID, GAE_ERR_LINK, GAE_ERR_RANGE = 0x1, 0x2, 0x4  # include/ppg.h PPG_GAE_ERR_*
+LINK_ERR_MISSING, LINK_ERR_OVERFLOW = 0x1, 0x2  # include/ppg.h PPG_LINK_ERR_*
 
 
 def _round32(n):

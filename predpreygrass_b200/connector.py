@@ -18,6 +18,11 @@ environment step stays in the CUDA kernels.
 `RolloutBuffer` records T+1 outputs of a handle (`DeviceRollout.rollout()` fills it) and computes PPO's GAE advantages and
 value targets over them with one `ppg_gae` kernel launch (include/ppg.h); `columns()` hands out the transitions under
 RLlib's names, `advantages` and `value_targets` included.
+
+Recurrent policies: `DeviceRollout(..., recurrent=True)` switches the env's row links on (include/ppg.h ppg_track_links) and
+carries each agent's hidden state from its row in one output to its row in the next with one gather per species;
+`RolloutBuffer(..., keep_state=True)` records the state each action was computed from and marks each agent's life segment
+(`seq_id`, `seq_pos`) so a learner can cut BPTT sequences.
 """
 import torch
 
@@ -42,6 +47,24 @@ class LinearPolicy(torch.nn.Module):
 
     def forward(self, obs):
         return self.lin(obs.flatten(1))
+
+
+class GRUPolicy(torch.nn.Module):
+    """the smallest recurrent policy: a linear encoder, a GRU cell, a logits head (a stand-in that exercises the plumbing of
+    DeviceRollout(recurrent=True)).  forward(obs [n, C, R, R], state_in [n, state_size]) -> (logits, state_out)"""
+
+    def __init__(self, n_in, n_out, device, state_size=16, seed=0):
+        super().__init__()
+        torch.manual_seed(seed)
+        self.state_size = state_size
+        self.enc = torch.nn.Linear(n_in, state_size)
+        self.cell = torch.nn.GRUCell(state_size, state_size)
+        self.head = torch.nn.Linear(state_size, n_out)
+        self.to(device)
+
+    def forward(self, obs, state_in):
+        h = self.cell(torch.relu(self.enc(obs.flatten(1))), state_in)
+        return self.head(h), h
 
 
 class ConvPolicy(torch.nn.Module):
@@ -71,13 +94,23 @@ class DeviceRollout:
 
     policies: (predator_module, prey_module); a module maps float32 [n, C, R, R] to logits [n, n_logits].  For the STAG
     predator (`MultiDiscrete([n_moves, 2])`, STAG:1813-1816) the logits are n_moves + 2 wide: move logits, then join_hunt logits.
+
+    recurrent=True: each module has a `state_size` attribute H and is called as module(obs, state_in) -> (logits, state_out)
+    with state_in float32 [n, H].  The runner switches the env's row links on and keeps each species' state_out of the last
+    forward; the next state_in of a row is the state_out of the row its agent had in the previous output (env.prev_row()),
+    zeros for founders and newborns.  `state_in` holds the (pred, prey) states of the last act().
     """
 
-    def __init__(self, env, policies, stream=None, sample=True, seed=0):
+    def __init__(self, env, policies, stream=None, sample=True, seed=0, recurrent=False):
         self.env, self.policies, self.stream, self.sample = env, policies, stream, sample
         self.gen = torch.Generator(device=env.device).manual_seed(seed)
         self.variant = env.cfg.variant
         self.last = None
+        self.recurrent = recurrent
+        if recurrent:
+            env.track_links(True)
+            self.state_out = [None, None]  # state_out of the last forward per species, rows of the output it ran on
+            self.state_in = (None, None)
 
     def _ctx(self):
         return torch.cuda.stream(self.stream) if self.stream is not None else torch.cuda.stream(torch.cuda.current_stream(self.env.device))
@@ -95,13 +128,20 @@ class DeviceRollout:
         -> per species (n, actions int64 [n], logp or None)"""
         env, out = self.env, self.env.out
         n = out.counts()  # 16 bytes device -> host: the row counts of the last output
+        if self.recurrent:
+            self.state_in = self._next_state_in(n)
         res = []
         for s in range(2):
             k = n[s]
             if k == 0:
+                if self.recurrent:
+                    self.state_out[s] = self.state_in[s]
                 res.append((0, None, None))
                 continue
-            logits = self.policies[s](out.obs[s][:k])
+            if self.recurrent:
+                logits, self.state_out[s] = self.policies[s](out.obs[s][:k], self.state_in[s])
+            else:
+                logits = self.policies[s](out.obs[s][:k])
             if self.variant == VARIANT_STAG and s == 0:
                 nm = env.n_actions(0)
                 mv, lp1 = self._pick(logits[:, :nm])
@@ -114,6 +154,20 @@ class DeviceRollout:
             res.append((k, a, lp))
         return res
 
+    def _next_state_in(self, n):
+        """(pred, prey) float32 [n_s, H]: the state_out of each row's agent in the previous output, zeros where unlinked"""
+        res, prev = [], None
+        for s in range(2):
+            H, so = self.policies[s].state_size, self.state_out[s]
+            if so is None or so.shape[0] == 0 or n[s] == 0:  # nothing to carry: the first output, or no rows before
+                res.append(torch.zeros((n[s], H), dtype=torch.float32, device=self.env.device))
+                continue
+            if prev is None:
+                prev = self.env.prev_row()
+            pr = prev[s][: n[s]].to(torch.int64)
+            res.append(torch.where((pr >= 0)[:, None], so[pr.clamp(min=0)], 0.0))
+        return tuple(res)
+
     @torch.no_grad()
     def step(self):
         with self._ctx():
@@ -123,22 +177,30 @@ class DeviceRollout:
     @torch.no_grad()
     def rollout(self, buffer, value_fns):
         """fills `buffer` (a RolloutBuffer of this env, empty or just carried): T times act -> record -> step, then records
-        output T.  value_fns: (predator, prey); each maps the observation rows float32 [n, C, R, R] to values [n]."""
+        output T.  value_fns: (predator, prey); each maps the observation rows float32 [n, C, R, R] to values [n]; a recurrent
+        runner calls them as value_fn(obs, state_in) and hands state_in to the buffer (recorded with keep_state)."""
         if buffer.env is not self.env:
             raise ValueError("rollout: the buffer belongs to another env")
         with self._ctx():
             for _ in range(buffer.T):
                 acted = self.act()
                 buffer.record(self._values(acted, value_fns), actions=tuple(a for _, a, _ in acted),
-                              logp=None if not self.sample else tuple(lp for _, _, lp in acted))
+                              logp=None if not self.sample else tuple(lp for _, _, lp in acted),
+                              **({"state_in": self.state_in} if self.recurrent else {}))
                 self.env.step()
                 self.last = acted
             n = self.env.out.counts()
-            buffer.record(self._values(tuple((n[s], None, None) for s in range(2)), value_fns))
+            if self.recurrent:
+                self.state_in = self._next_state_in(n)
+            buffer.record(self._values(tuple((n[s], None, None) for s in range(2)), value_fns),
+                          **({"state_in": self.state_in} if self.recurrent else {}))
         return buffer
 
     def _values(self, acted, value_fns):
         out = self.env.out
+        if self.recurrent:
+            return tuple(value_fns[s](out.obs[s][:k], self.state_in[s]).reshape(-1) if k else torch.zeros(0, device=self.env.device)
+                         for s, (k, _, _) in enumerate(acted))
         return tuple(value_fns[s](out.obs[s][:k]).reshape(-1) if k else torch.zeros(0, device=self.env.device)
                      for s, (k, _, _) in enumerate(acted))
 
@@ -200,13 +262,15 @@ class RolloutBuffer:
     valid), old_off [T+1, B+1], new_off, new_cnt and env_flags [T+1, B]; actions and logp of the rows of output t [T, cap];
     the observation rows [n_t, C, R, R] of each output (keep_obs=False skips them).  `values` is public: a learner may
     overwrite it, e.g. with the value predictions of updated weights, and call compute() again.  Per step, record() only copies
-    into these slabs, except that with keep_obs it clones each output's observation rows (one allocation per species)."""
+    into these slabs, except that with keep_obs it clones each output's observation rows (one allocation per species).
+    keep_state=True: record() also takes state_in = (pred, prey) [n_s, H], the recurrent state each row's action was computed
+    from, and clones it the same way; columns() then adds state_in, seq_id and seq_pos."""
 
-    def __init__(self, env, n_steps, keep_obs=True):
+    def __init__(self, env, n_steps, keep_obs=True, keep_state=False):
         T = int(n_steps)
         if T < 1:
             raise ValueError("RolloutBuffer: n_steps must be >= 1")
-        self.env, self.T, self.keep_obs = env, T, keep_obs
+        self.env, self.T, self.keep_obs, self.keep_state = env, T, keep_obs, keep_state
         d, B, cap = env.device, env.n_envs, env.row_capacity
 
         def slab(rows, n, dtype, fill=0):
@@ -229,19 +293,23 @@ class RolloutBuffer:
         self.next_row = slab(T, cap, torch.int32, -1)
         self.error = torch.zeros(1, dtype=torch.int32, device=d)
         self.obs = [[None, None] for _ in range(T + 1)]
+        self.state = [[None, None] for _ in range(T + 1)]
         self.n = [(0, 0)] * (T + 1)  # rows of each output, from the length of its values
         self.t = 0                   # outputs recorded
         self.has_logp = False
         self._carried = False
         self._computed = False
 
-    def record(self, values, actions=None, logp=None):
+    def record(self, values, actions=None, logp=None, state_in=None):
         """Records the env's current output into slot t: values = (v_pred, v_prey), float32 [n_s] for every row of the output
         (terminated and truncated rows included); actions / logp: (pred, prey) [n_s] of the rows of this output, for slots
-        0..T-1.  Tensor.copy_ on the current stream, no host synchronisation."""
+        0..T-1; state_in (with keep_state; a carried slot keeps its state without it): (pred, prey) float32 [n_s, H].
+        Tensor.copy_ on the current stream, no host synchronisation."""
         t, T, out = self.t, self.T, self.env.out
         if t > T:
             raise RuntimeError(f"RolloutBuffer.record: all {T + 1} outputs are recorded (compute, columns, then carry)")
+        if self.keep_state and state_in is None and not self._carried:
+            raise ValueError("RolloutBuffer.record: keep_state needs state_in")
         n = tuple(int(values[s].shape[0]) for s in range(2))
         for s in range(2):
             if n[s] > self.env.row_capacity[s]:
@@ -256,6 +324,8 @@ class RolloutBuffer:
                 self.new_off[s][t].copy_(out.new_off[s])
                 self.new_cnt[s][t].copy_(out.new_cnt[s])
                 self.obs[t][s] = out.obs[s][:k].clone() if self.keep_obs else None
+            if self.keep_state and state_in is not None:
+                self.state[t][s] = state_in[s][:k].clone()
             self.values[s][t, :k].copy_(values[s])
             if t < T and actions is not None and actions[s] is not None:
                 self.actions[s][t, :k].copy_(actions[s])
@@ -283,7 +353,11 @@ class RolloutBuffer:
         """{"predator": columns, "prey": columns}: one entry per transition (row (t, r) with next_row >= 0), ordered by t, then
         row, under RLlib's names: obs, actions, action_logp (None unless recorded), rewards, terminateds, truncateds (of the
         successor row, by the rule of include/ppg.h), vf_preds, advantages, value_targets, eps_id (env index) and agent_index
-        (agent id).  Synchronises once; raises PpgError if the kernel flagged malformed slabs."""
+        (agent id).  With keep_state also state_in (the recorded state of the row), seq_id (int64: one id per agent life
+        segment inside the rollout, the flat index t0 * cap + r0 of the segment's first row) and seq_pos (int32: the
+        transition's position in its segment), derived from the links compute() produced; a learner cuts BPTT chunks of
+        length L where seq_pos % L == 0 and starts each from state_in there.  Synchronises once; raises PpgError if the
+        kernel flagged malformed slabs."""
         from ._lib import PpgError
 
         if not self._computed:
@@ -329,6 +403,16 @@ class RolloutBuffer:
                         parts.append(self.obs[t][s][r_i[k:k + per_t[t]]])
                     k += per_t[t]
                 obs = torch.cat(parts) if parts else self.obs[0][s][:0]
+            extra = {}
+            if self.keep_state:
+                seg_id, seg_pos = self._segments(s)
+                parts, k = [], 0
+                for t in range(T):
+                    if per_t[t]:
+                        parts.append(self.state[t][s][r_i[k:k + per_t[t]]])
+                    k += per_t[t]
+                extra = {"state_in": torch.cat(parts) if parts else self.state[0][s][:0],
+                         "seq_id": seg_id.flatten()[i], "seq_pos": seg_pos.flatten()[i]}
             res[name] = {
                 "obs": obs,
                 "actions": self.actions[s].flatten()[i].to(torch.int64),
@@ -341,8 +425,28 @@ class RolloutBuffer:
                 "value_targets": self.value_targets[s].flatten()[i],
                 "eps_id": env_i,
                 "agent_index": self.row_agent[s].flatten()[i].to(torch.int64),
+                **extra,
             }
         return res
+
+    def _segments(self, s):
+        """[T, cap] segment id and position of every row of outputs 0..T-1, forward along next_row: a row another row links
+        to continues that row's segment, every other row starts one"""
+        T, cap, d = self.T, self.env.row_capacity[s], self.env.device
+        ar = torch.arange(cap, device=d)
+        seg_id = torch.empty((T, cap), dtype=torch.int64, device=d)
+        seg_pos = torch.zeros((T, cap), dtype=torch.int32, device=d)
+        seg_id[0] = ar
+        n_t = self.n_rows[:, s] + self.n_rows[:, s + 2]
+        for t in range(T - 1):
+            nr = self.next_row[s][t].to(torch.int64)
+            dst = torch.where((nr >= 0) & (ar < n_t[t]), nr, cap)  # unlinked rows scatter into a spill slot
+            sid = torch.cat([(t + 1) * cap + ar, ar[:1]])
+            spos = torch.zeros(cap + 1, dtype=torch.int32, device=d)
+            sid.scatter_(0, dst, seg_id[t])
+            spos.scatter_(0, dst, seg_pos[t] + 1)
+            seg_id[t + 1], seg_pos[t + 1] = sid[:cap], spos[:cap]
+        return seg_id, seg_pos
 
     def carry(self):
         """makes output T slot 0 of the next rollout (its columns, values and observation rows); the next record() adds the
@@ -354,8 +458,10 @@ class RolloutBuffer:
             for sl in (self.row_agent, self.row_env, self.flags, self.reward, self.values, self.old_off, self.new_off, self.new_cnt):
                 sl[s][0].copy_(sl[s][T])
             self.obs[0][s] = self.obs[T][s]
+            self.state[0][s] = self.state[T][s]
         self.env_flags[0].copy_(self.env_flags[T])
         self.n_rows[0].copy_(self.n_rows[T])
         self.n[0] = self.n[T]
         self.obs[1:] = [[None, None] for _ in range(T)]
+        self.state[1:] = [[None, None] for _ in range(T)]
         self.t, self._carried, self._computed, self.has_logp = 0, True, False, False

@@ -53,6 +53,8 @@ cudaError_t launch_gae(const GaeParams& p, cudaStream_t stream);
 int gae_warps(int log2_h);
 // ppg_agent_state.cu
 cudaError_t launch_agent_state(const AgentStateParams& p, cudaStream_t stream);
+// ppg_links.cu
+cudaError_t launch_links(const LinksParams& p, cudaStream_t stream);
 }  // namespace ppg
 
 namespace ppg { int g_pdl_chain = -1; }
@@ -92,6 +94,11 @@ struct ppg_handle_s {
   bool R_alloc = false;
   double* d_ep_partial = nullptr;        // ppg_episode_stats_device scratch and result
   double* d_ep_stats = nullptr;
+  // row links (ppg_track_links): allocated at the first switch-on; ready once an output was linked since the tables were
+  // last filled by the switch-on or a restore
+  bool links_on = false, links_ready = false;
+  LinksParams Lk;
+  bool Lk_alloc = false;
   int64_t launch_count = 0;
   std::vector<void*> allocs;
   unsigned long long* d_stats = nullptr;
@@ -766,6 +773,12 @@ static int run_step_kernel(ppg_handle h, const int32_t* a0, const int32_t* a1, c
     CK(launch_returns(h->R, st));
     h->launch_count++;
   }
+  if (h->links_on) {
+    h->Lk.save_only = 0;
+    CK(launch_links(h->Lk, st));
+    h->launch_count++;
+    h->links_ready = true;
+  }
   // the images now hold this output's world, except that an env idle since a ppg_restore still has the pre-restore one:
   // after restoring idle envs only a full reset (a0 == NULL, every env dumps its image) makes them valid again
   if (a0 == nullptr || h->img != ppg_handle_s::IMG_RESTORED_IDLE) h->img = ppg_handle_s::IMG_VALID;
@@ -1003,6 +1016,12 @@ int ppg_restore(ppg_handle h, const void* blob, size_t bytes, void* cuda_stream)
     CK(cudaMemsetAsync(h->R.env_valid, 0, (size_t)h->B, st));
     CK(cudaMemsetAsync(h->R.env_return, 0xFF, (size_t)h->B * 2 * sizeof(double), st));  // all-ones bits: NaN
   }
+  if (h->links_on) {  // the link tables are not in the blob: saved from the restored lists
+    h->Lk.save_only = 1;
+    CK(launch_links(h->Lk, st));
+    h->launch_count++;
+    h->links_ready = false;
+  }
   CK(cudaStreamSynchronize(st));
   h->h_n_rows_valid = false;
   return PPG_OK;
@@ -1068,6 +1087,51 @@ int ppg_episode_stats_clear(ppg_handle h, void* cuda_stream) {
   CK(cudaSetDevice(h->device));
   CK(launch_episode_stats_clear(h->R.env_acc, h->B, static_cast<cudaStream_t>(cuda_stream)));
   h->launch_count++;
+  return PPG_OK;
+}
+
+int ppg_track_links(ppg_handle h, int32_t on, void* cuda_stream) {
+  if (!h) return PPG_ERR_INVALID;
+  if (!on) { h->links_on = h->links_ready = false; return PPG_OK; }
+  if (h->links_on) return PPG_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+  CK(cudaSetDevice(h->device));
+  LinksParams& L = h->Lk;
+  const StepParams& P = h->P;
+  if (!h->Lk_alloc) {
+    memset(&L, 0, sizeof L);
+    L.hdr = P.hdr;
+    for (int s = 0; s < 2; ++s) {
+      L.ag_id[s] = P.ag_id[s]; L.ag_prow[s] = P.ag_prow[s]; L.row_agent[s] = P.row_agent[s]; L.flags[s] = P.flags[s];
+      L.old_off[s] = P.old_off[s]; L.new_off[s] = P.new_off[s]; L.new_cnt[s] = P.new_cnt[s];
+      L.cap[s] = P.cap[s];
+      L.log2_h[s] = 1;
+      while ((1 << L.log2_h[s]) < 2 * P.cap[s]) ++L.log2_h[s];  // load factor <= 1/2 with cap_live list entries per env
+      CK(dalloc(h, &L.prev_row[s], (size_t)h->bufs.row_capacity[s]));
+      CK(dalloc(h, &L.tab[s], (size_t)h->B << L.log2_h[s], false));
+      CK(cudaMemset(L.tab[s], 0xFF, ((size_t)h->B << L.log2_h[s]) * sizeof(uint32_t)));  // LINK_EMPTY
+      CK(dalloc(h, &L.base[s], (size_t)h->B));
+    }
+    L.env_flags = P.env_flags;
+    L.B = h->B;
+    CK(dalloc(h, &L.error, 1));
+    h->Lk_alloc = true;
+  }
+  L.save_only = 1;
+  CK(launch_links(L, st));
+  h->launch_count++;
+  h->links_on = true;
+  h->links_ready = false;
+  return PPG_OK;
+}
+
+int ppg_get_links(ppg_handle h, int32_t** prev_row, uint32_t** error) {
+  if (!h || !prev_row || !error) return PPG_ERR_INVALID;
+  if (!h->links_on) { h->err = "ppg_get_links: links are off (ppg_track_links)"; return PPG_ERR_STATE; }
+  if (!h->links_ready) { h->err = "ppg_get_links: no output since links were switched on or since ppg_restore"; return PPG_ERR_STATE; }
+  prev_row[0] = h->Lk.prev_row[0];
+  prev_row[1] = h->Lk.prev_row[1];
+  *error = h->Lk.error;
   return PPG_OK;
 }
 

@@ -300,6 +300,12 @@ struct AgentStateParams {
   int n_grass, B;
 };
 
+// Link tables of ppg_gae_kernel and ppg_links_kernel: per env (and species) an open-addressing hash with linear probing over
+// 1 << log2_h words id << 16 | j, where j is the position of the id's row among the env's rows of one output.  Its size
+// follows cap_live, never n_possible.  LINK_EMPTY is no such word: id 0xFFFF is never valid (n_possible <= 65535).
+constexpr uint32_t LINK_EMPTY = 0xFFFFFFFFu;
+__device__ __forceinline__ uint32_t link_slot(int id, int log2_h) { return ((uint32_t)id * 0x9E3779B1u) >> (32 - log2_h); }
+
 // ppg_gae_kernel (ppg_gae.cu): links the rows of a rollout and runs the GAE recursion (include/ppg.h ppg_gae).
 struct GaeParams {
   ppg_gae_args a;
@@ -307,6 +313,28 @@ struct GaeParams {
   int n_possible[2];
   int B;
   int log2_h;         // link table: 1 << log2_h entries per warp and buffer
+};
+
+// ppg_links_kernel (ppg_links.cu): the row of the previous output behind every old row of the last output (include/ppg.h
+// ppg_track_links).  tab[s] / base[s] are saved from the agent lists after every output and read after the next one.
+struct LinksParams {
+  const EnvHdr* hdr;
+  const uint16_t* ag_id[2];
+  const int32_t* ag_prow[2];
+  const int32_t* row_agent[2];
+  const uint8_t* flags[2];
+  const int32_t* old_off[2];
+  const int32_t* new_off[2];
+  const int32_t* new_cnt[2];
+  const uint8_t* env_flags;
+  int32_t* prev_row[2];  // [row_capacity[s]]
+  uint32_t* tab[2];      // [B][1 << log2_h[s]] link table of the output the lists were saved from
+  int4* base[2];         // [B] that output's old_off[e], old row count, new_off[e] (row of position j, see ppg_links.cu)
+  uint32_t* error;       // [1] sticky PPG_LINK_ERR_* bits
+  int cap[2];            // cap_live[s]: list pitch
+  int log2_h[2];
+  int B;
+  int save_only;         // 1: only save the tables (switch-on, ppg_restore); prev_row is not written
 };
 
 // Launch with programmatic stream serialization (PDL): the grid's CTAs may be scheduled as soon as every CTA of the kernel

@@ -4,9 +4,8 @@
 // t = T to 0.  At output t it reads the env's rows of t; it looks every live row up, by id, in the link table of output t+1
 // and, for a hit, evaluates the recursion from the successor row's reward, flags, value, advantage and link (written by the
 // same warp one iteration earlier); and it inserts the old, non-FOUNDER rows of t into the other table, which serves output
-// t-1.  A table is an open-addressing hash (linear probing) of (id << 16 | row - old_off) words in the warp's shared-memory
-// slice, so its size follows cap_live, never n_possible.  __syncwarp separates the outputs: it orders the warp's global
-// writes of output t+1 before the reads of output t.  Every value is one chain of fp32 operations with no reduction, so the
+// t-1.  A table is the link table of ppg_device.cuh (id << 16 | row - old_off words) in the warp's shared-memory slice.
+// __syncwarp separates the outputs: it orders the warp's global writes of output t+1 before the reads of output t.  Every value is one chain of fp32 operations with no reduction, so the
 // result does not depend on the schedule.  The kernel never executes griddepcontrol.launch_dependents.
 #include <cuda_runtime.h>
 
@@ -19,9 +18,6 @@ namespace ppg {
 
 constexpr int GAE_WARPS = 8;  // warps per CTA at most; fewer when a warp's two tables need more than GAE_SMEM_MAX / 8
 constexpr int GAE_SMEM_MAX = 227 * 1024;
-constexpr uint32_t GAE_EMPTY = 0xFFFFFFFFu;  // id 0xFFFF is never valid (n_possible <= 65535)
-
-__device__ __forceinline__ uint32_t gae_slot(int id, int log2_h) { return ((uint32_t)id * 0x9E3779B1u) >> (32 - log2_h); }
 
 __global__ void __launch_bounds__(GAE_WARPS * 32) ppg_gae_kernel(const __grid_constant__ GaeParams p) {
   extern __shared__ uint32_t gae_smem[];
@@ -50,7 +46,7 @@ __global__ void __launch_bounds__(GAE_WARPS * 32) ppg_gae_kernel(const __grid_co
     for (int t = T; t >= 0; --t) {
       uint32_t* mine = tab + (t & 1) * H;
       const uint32_t* succ = tab + ((t + 1) & 1) * H;
-      for (int k = lane; k < H; k += 32) mine[k] = GAE_EMPTY;
+      for (int k = lane; k < H; k += 32) mine[k] = LINK_EMPTY;
       __syncwarp();
       const int o0 = old_off[(size_t)t * (B + 1) + e], o1 = old_off[(size_t)t * (B + 1) + e + 1];
       const int n0 = new_off[(size_t)t * B + e], nc = new_cnt[(size_t)t * B + e];
@@ -78,18 +74,18 @@ __global__ void __launch_bounds__(GAE_WARPS * 32) ppg_gae_kernel(const __grid_co
         bool ins = t > 0 && id_ok && j < n_old && !(f & (PPG_ROW_FOUNDER | PPG_ROW_NEWBORN));
         if (ins) {
           const uint32_t w = (uint32_t)id << 16 | (uint32_t)j;
-          uint32_t k = gae_slot(id, p.log2_h);
+          uint32_t k = link_slot(id, p.log2_h);
           int probe = 0;
-          while (atomicCAS(&mine[k], GAE_EMPTY, w) != GAE_EMPTY && ++probe < H) k = (k + 1) & (H - 1);
+          while (atomicCAS(&mine[k], LINK_EMPTY, w) != LINK_EMPTY && ++probe < H) k = (k + 1) & (H - 1);
           if (probe >= H) { err |= PPG_GAE_ERR_RANGE; ins = false; }
         }
         inserted += __popc(__ballot_sync(0xFFFFFFFFu, ins));
         int rn = -1;
         if (lookup && id_ok && !(f & (PPG_ROW_TERMINATED | PPG_ROW_TRUNCATED))) {
-          uint32_t k = gae_slot(id, p.log2_h);
+          uint32_t k = link_slot(id, p.log2_h);
           for (int probe = 0; probe < H; ++probe) {
             const uint32_t w = succ[k];
-            if (w == GAE_EMPTY) break;
+            if (w == LINK_EMPTY) break;
             if ((int)(w >> 16) == id) { rn = old0_next + (int)(w & 0xFFFFu); break; }
             k = (k + 1) & (H - 1);
           }
