@@ -12,8 +12,7 @@
 #include "ppg_device.cuh"
 
 namespace ppg {
-cudaError_t launch_step_base(const StepParams& p, int warps_per_cta, int n_cta, size_t smem, cudaStream_t stream);
-cudaError_t step_base_occupancy(int warps_per_cta, int map_bytes, bool bulk, bool split, size_t smem, int* blocks_per_sm);
+StepKernel step_kernel_base(const StepParams& p, int warps_per_cta);
 cudaError_t launch_prepare_offsets(const EnvHdr* hdr, int B, int n0, int n1, unsigned long long* cntA, unsigned long long* sum1,
                                    unsigned long long* sum2, int32_t* totals4, unsigned epoch, int hdr_founders, cudaStream_t s);
 cudaError_t launch_init_hdr(EnvHdr* hdr, int B, unsigned long long seed, cudaStream_t s);
@@ -29,13 +28,11 @@ cudaError_t launch_stats(const uint32_t* counters, const EnvHdr* hdr, int B, uns
 cudaError_t launch_obs(const StepParams& p, int n_cta, bool overlap, cudaStream_t stream);
 cudaError_t obs_occupancy(const StepParams& p, int* blocks_per_sm);
 // ppg_eco.cu
-cudaError_t launch_step_eco(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream);
-cudaError_t step_eco_occupancy(int map_bytes, bool split, int kind, size_t smem, int* blocks_per_sm);
+StepKernel step_kernel_eco(const StepParams& p);
 cudaError_t launch_set_tape_reals(EcoHdr* ehdr, int B, const long long* real_off, cudaStream_t s);
 cudaError_t launch_eco_founders(const StepParams& p, cudaStream_t s);
 // ppg_stag.cu
-cudaError_t launch_step_stag(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream);
-cudaError_t step_stag_occupancy(int map_bytes, bool split, size_t smem, int* blocks_per_sm);
+StepKernel step_kernel_stag(const StepParams& p);
 cudaError_t launch_set_tape_reals_stag(StagHdr* shdr, int B, const long long* real_off, cudaStream_t s);
 cudaError_t launch_random_actions_stag(const int32_t* n_rows, const int32_t* re0, const int32_t* ra0, const int32_t* re1, const int32_t* ra1,
                                        int32_t* a0, int32_t* a1, unsigned long long seed, unsigned call, unsigned env_base, int t2_pred,
@@ -73,6 +70,7 @@ struct ppg_handle_s {
   std::vector<int32_t> walls;  // copy of ppg_config.wall_cells
   int warps_per_cta = 4, n_cta = 0;
   size_t smem_bytes = 0;
+  StepKernel step_kernel = {nullptr, 0};
   unsigned long long launches_step = 0;  // step-kernel launches so far (epoch)
   unsigned long long ticket_next = 0;    // value the device ticket counter has after all launches so far
   unsigned long long obs_ticket_next = 0;  // same for the observation kernel's counter
@@ -551,11 +549,10 @@ static int upload_tables(ppg_handle h) {
   return PPG_OK;
 }
 
-// 4. launch geometry of the step and observation kernels; every PPG_* experiment switch of a handle except PPG_OBS_BULK
-//    (layout_smem) is read here.  *env_order: the step kernel orders the envs of the next launch big-first (P.perm).
-static int launch_geometry(ppg_handle h, bool* env_order) {
+// 4. the step's paths; with launch_grid, every PPG_* experiment switch of a handle except PPG_OBS_BULK (layout_smem) is read
+//    here.  *env_order: the step kernel orders the envs of the next launch big-first (P.perm).
+static int launch_paths(ppg_handle h, bool* env_order) {
   StepParams& P = h->P;
-  const int B = h->B;
   const bool eco = P.variant == PPG_VARIANT_ECO, stag = P.variant == PPG_VARIANT_STAG;
   int W = 1;
   if (const char* ev = getenv("PPG_WARPS_PER_CTA")) W = atoi(ev);
@@ -568,27 +565,9 @@ static int launch_geometry(ppg_handle h, bool* env_order) {
   if (W != 1 || P.obs_bulk || P.CH >= (int)DSC_COPY) P.obs_split = 0;
   h->warps_per_cta = W;
   h->smem_bytes = (size_t)W * P.smem_per_env;
-  // persistent warps: as many CTAs as fit on the device, never more than there are envs
-  int per_sm = 0, n_sm = 0;
-  if (eco) CK(step_eco_occupancy(P.map_bytes, P.obs_split != 0, P.trait_mode != PPG_TRAIT_SPEED ? 1 : (P.lin_on ? 2 : 0), h->smem_bytes, &per_sm));
-  else if (stag) CK(step_stag_occupancy(P.map_bytes, P.obs_split != 0, h->smem_bytes, &per_sm));
-  else CK(step_base_occupancy(W, P.map_bytes, P.obs_bulk != 0, P.obs_split != 0, h->smem_bytes, &per_sm));
-  CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device));
-  if (per_sm < 1) { h->err = "step kernel does not fit on an SM"; return PPG_ERR_INVALID; }
-  h->n_cta = std::min((B + W - 1) / W, per_sm * n_sm);
-  if (const char* ev = getenv("PPG_MAX_CTAS")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev)));
   // big-envs-first order of the next launch: only where no env ever waits for another one (publish_begin)
   *env_order = !eco && P.obs_split;
   if (const char* ev = getenv("PPG_ENV_ORDER")) *env_order = *env_order && atoi(ev) != 0;
-  if (P.obs_split) {
-    if (const char* ev = getenv("PPG_OBS_OVERLAP")) h->obs_overlap = atoi(ev) != 0;
-    CK(obs_occupancy(P, &per_sm));
-    if (per_sm < 1) { h->err = "observation kernel does not fit on an SM"; return PPG_ERR_INVALID; }
-    h->n_cta_obs = std::min(B, per_sm * n_sm);
-    if (const char* ev = getenv("PPG_OBS_CTAS_PER_SM")) h->n_cta_obs = std::max(1, std::min(h->n_cta_obs, atoi(ev) * n_sm));
-    // overlap: leave room on every SM for observation CTAs next to the step kernel's persistent warps
-    if (const char* ev = getenv("PPG_STEP_CTAS_PER_SM")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev) * n_sm));
-  }
   return PPG_OK;
 }
 
@@ -649,14 +628,48 @@ static int allocate(ppg_handle h, bool env_order) {
   return PPG_OK;
 }
 
+// 6. the step kernel (its choice depends on the allocated state: ECO's episode sums) and the grids of the step and observation
+//    kernels
+static int launch_grid(ppg_handle h) {
+  StepParams& P = h->P;
+  const int B = h->B, W = h->warps_per_cta;
+  h->step_kernel = P.variant == PPG_VARIANT_ECO ? step_kernel_eco(P) : P.variant == PPG_VARIANT_STAG ? step_kernel_stag(P) : step_kernel_base(P, W);
+  const StepKernel& k = h->step_kernel;
+  if (k.fn == nullptr) { h->err = "no step kernel for this configuration"; return PPG_ERR_INVALID; }
+  // opt in to the slice's dynamic shared memory (above 48 KB); the attribute only grows, so it holds for every handle of the
+  // process that launches this kernel on this device
+  cudaFuncAttributes fa;
+  CK(cudaFuncGetAttributes(&fa, k.fn));
+  if ((size_t)fa.maxDynamicSharedSizeBytes < h->smem_bytes)
+    CK(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+  // persistent warps: as many CTAs as fit on the device, never more than there are envs
+  int per_sm = 0, n_sm = 0;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k.fn, k.threads, h->smem_bytes));
+  CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, h->device));
+  if (per_sm < 1) { h->err = "step kernel does not fit on an SM"; return PPG_ERR_INVALID; }
+  h->n_cta = std::min((B + W - 1) / W, per_sm * n_sm);
+  if (const char* ev = getenv("PPG_MAX_CTAS")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev)));
+  if (P.obs_split) {
+    if (const char* ev = getenv("PPG_OBS_OVERLAP")) h->obs_overlap = atoi(ev) != 0;
+    CK(obs_occupancy(P, &per_sm));
+    if (per_sm < 1) { h->err = "observation kernel does not fit on an SM"; return PPG_ERR_INVALID; }
+    h->n_cta_obs = std::min(B, per_sm * n_sm);
+    if (const char* ev = getenv("PPG_OBS_CTAS_PER_SM")) h->n_cta_obs = std::max(1, std::min(h->n_cta_obs, atoi(ev) * n_sm));
+    // overlap: leave room on every SM for observation CTAs next to the step kernel's persistent warps
+    if (const char* ev = getenv("PPG_STEP_CTAS_PER_SM")) h->n_cta = std::max(1, std::min(h->n_cta, atoi(ev) * n_sm));
+  }
+  return PPG_OK;
+}
+
 static int init_handle(ppg_handle h) {
   CK(cudaSetDevice(h->device));
   set_step_params(h);
   bool env_order = false;
   int rc = layout_smem(h);
   if (!rc) rc = upload_tables(h);
-  if (!rc) rc = launch_geometry(h, &env_order);
+  if (!rc) rc = launch_paths(h, &env_order);
   if (!rc) rc = allocate(h, env_order);
+  if (!rc) rc = launch_grid(h);
   if (rc) return rc;
   CK(launch_init_hdr(h->P.hdr, h->B, h->cfg.seed, 0));
   h->launch_count++;
@@ -755,9 +768,7 @@ static int run_step_kernel(ppg_handle h, const int32_t* a0, const int32_t* a1, c
     for (int k = 0; k < 3; ++k) { CK(cudaEventCreate(&pe[k])); h->prof_events.push_back(pe[k]); }
     CK(cudaEventRecord(pe[0], st));
   }
-  if (P.variant == PPG_VARIANT_ECO) CK(launch_step_eco(P, h->n_cta, h->smem_bytes, st));
-  else if (P.variant == PPG_VARIANT_STAG) CK(launch_step_stag(P, h->n_cta, h->smem_bytes, st));
-  else CK(launch_step_base(P, h->warps_per_cta, h->n_cta, h->smem_bytes, st));
+  CK(pdl_launch(h->step_kernel.fn, dim3((unsigned)h->n_cta), dim3((unsigned)h->step_kernel.threads), h->smem_bytes, st, P));
   h->launches_step++;
   h->launch_count++;
   if (h->profiling) CK(cudaEventRecord(pe[1], st));

@@ -70,8 +70,6 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
   const RowDesc D = carve_desc(sbase, p);
   const unsigned sb32 = (unsigned)__cvta_generic_to_shared(sbase);
   const int G = p.G, GG = p.GG, PP = p.P, PS = p.PS;
-  const unsigned epoch = p.epoch;
-  const int par = (int)(epoch & 1u);
   const int mode_r = p.reward_mode;
   const bool dense = mode_r == PPG_REWARD_DENSE || mode_r == PPG_REWARD_DENSE_ADDITIVE;
   const bool kick = mode_r == PPG_REWARD_SPARSE_KICKBACK;
@@ -92,32 +90,17 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
     }
   }
   unsigned rowctr = 0;
-  const int n_old_total[2] = {p.totals[(par ^ 1) * 4 + 0], p.totals[(par ^ 1) * 4 + 1]};
-  const int n_blk = (p.B + 31) >> 5, n_grp = (p.B + 1023) >> 10;
+  EnvLoop L = env_loop(p, SPLIT);  // SPLIT exists for W == 1 only
   __syncwarp();
 
-  // W == 1: envs come from the ticket counter; after the first one the ticket is drawn by lane 0 while the previous env is
-  // still being finished (`env_next`: late enough that the schedule stays dynamic, early enough that the atomic's round
-  // trip is never waited for).  Tickets are handed out in env order to warps that are running, so an env that waits for
-  // the publication of a lower env (ECO's episode-end rows, the one-kernel step) always waits for a running warp.
-  // ticket -> env: big envs first when the previous launch left an order (publish_begin), else index order
-  const int32_t* const perm = (W == 1 && SPLIT && p.perm[par ^ 1] != nullptr && p.perm_tag[par ^ 1] == epoch - 1u) ? p.perm[par ^ 1] : nullptr;
-  // static_first: the first ticket of a warp is its CTA index — 2960 atomics on one address at kernel start cost the last
-  // warp ~7 us; the counter then hands out the tickets from min(grid, B) on
-  const int t_first = p.static_first ? min((int)gridDim.x, p.B) : 0;
-  int env_next = 0;
-  if (W == 1 && lane == 0) {
-    env_next = p.static_first ? min((int)blockIdx.x, p.B) : (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-    if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-  }
-  unsigned long long pend = 0ULL;  // lane 0: completion-queue slot + 1 of the env whose hand-over is still owed (queue_push)
-  int pend_env = 0;
+  // W == 1: envs come from the ticket counter (EnvLoop)
+  if (W == 1 && lane == 0) next_ticket(p, L, true);
   SPAN_MARK(base, 1)
   for (;;) {
     PHASE_DECL
     int env = 0;  // PHASE: ticket+hdr
     if (W == 1) {
-      env = __shfl_sync(FULL, env_next, 0);
+      env = __shfl_sync(FULL, L.env_next, 0);
       if (env >= p.B) break;
     } else {
       // the W warps of a CTA take W consecutive envs and start them together: warps of one CTA then run the
@@ -138,7 +121,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
     int next_live[2] = {0, 0};
     int mode = 0;  // 0 idle, 1 reset, 2 step
     unsigned env_flags = 0;
-    unsigned st_starved[2] = {0, 0}, st_eaten = 0, st_grass = 0, st_fallback = 0;
+    EnvStats st = {};
     int cur[2] = {0, 0};
     bool over = false, trunc = false;
 
@@ -171,22 +154,8 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
       const int g = lane + 32 * q;
       if (g < p.n_grass) { gp_r[q] = p.gr_pos[(size_t)env * p.n_grass + g]; ge_r[q] = p.gr_e[(size_t)env * p.n_grass + g]; }
     }
-    // first old row of this env: the previous launch published how many rows every env needs now
-    if (!prefix_before(p.cntA[par ^ 1], p.sum1[par ^ 1], p.sum2[par ^ 1], 0, env, epoch - 1u, false, lane, old_base[0], old_base[1])) {
-      if (lane == 0) atomicOr(p.error, 2u);  // the host did not prepare the counts of the previous output
-    }
-    // hand-over of the PREVIOUS env of this warp: its stores were issued a round trip ago, the fence finds them acknowledged
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
+    mode = env_begin<SPLIT>(p, L, env, h.state, p.n_init, old_base, next_live, lane);
     PHASE_MARK(1)
-    if (h.state & ST_NEEDS_RESET) mode = 1;
-    else if (h.state & ST_IDLE) mode = 0;
-    else mode = 2;
-    if (mode != 2) {
-      // reset / idle envs know their counts up front (founders, no births): publish them before doing any work, so
-      // that later envs waiting for their newborn-row prefix never wait for a reset
-      if (mode == 1) { next_live[0] = p.n_init[0]; next_live[1] = p.n_init[1]; }
-      publish_counts(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane);
-    }
 
     if (PPG_UNLIKELY(mode == 1)) {  // PHASE: reset
       // ------------------------------------------------------------------ reset() (BASE:129-217)
@@ -480,7 +449,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
               S.map[0][cell] = 0;  // BASE:293
               S.flg[0][slot] = F_DIED;
             }
-            st_starved[0]++;
+            st.starved[0]++;
             __syncwarp();
             continue;
           }
@@ -507,7 +476,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
               S.map[1][cell] = 0;  // BASE:335
               S.flg[1][q] = F_DIED | F_CAUGHT;
             }
-            st_eaten++;
+            st.eaten++;
             __syncwarp();
           }
         }
@@ -545,7 +514,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
             S.flg[1][slot] |= F_ATE;
             if (vt_valid) { S.vt[1][1 + slot] = (float)en; S.vt[2][g] = 0.f; }
           }
-          st_grass += __popc(__ballot_sync(FULL, eat));
+          st.grass += __popc(__ballot_sync(FULL, eat));
           __syncwarp();
           continue;
         }
@@ -563,7 +532,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
               S.map[1][cl] = 0;
               S.flg[1][sl] = F_DIED;
             }
-            st_starved[1]++;
+            st.starved[1]++;
             __syncwarp();
             continue;
           }
@@ -578,7 +547,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
               S.flg[1][sl] |= F_ATE;
               if (vt_valid) { S.vt[1][1 + sl] = (float)en; S.vt[2][gg] = 0.f; }
             }
-            st_grass++;
+            st.grass++;
             __syncwarp();
           }
         }
@@ -618,7 +587,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
               }
             }
             if (PPG_UNLIKELY(sx < 0)) {
-              st_fallback++;
+              st.fallback++;
               if (p.tape_cells != nullptr && h.tape_pos < h.tape_end) {
                 const int c = p.tape_cells[h.tape_pos++];  // recorded np.random.randint choice (BASE:764)
                 sx = c / G; sy = c % G;
@@ -699,17 +668,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
 
     PHASE_MARK(11)
     // ---------------------------------------------------------------- publish the counts  // PHASE: publish
-    // four atomics back to back, nobody waits for them here: the warp's next env, this env's slot in the completion queue,
-    // and the two accumulators of the row allocation (results looked at after the rows are written)
-#if PPG_TICKET_EARLY
-    if (W == 1 && lane == 0) {
-      env_next = t_first + (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-      if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-    }
-#endif
-    unsigned long long q_slot = 0ULL, pubA = 0ULL, pubB = 0ULL;
-    if (SPLIT) q_slot = queue_reserve(p, lane);
-    if (mode == 2) publish_begin(p, env, par, epoch, next_live, births, lane, pubA, pubB, (n_old_total[0] + n_old_total[1]) / p.B * 5 / 4);
+    env_publish<SPLIT>(p, L, env, mode, next_live, births, (L.n_old_total[0] + L.n_old_total[1]) / p.B * 5 / 4, W == 1, lane);
 
     PHASE_MARK(12)
     // ------------------------------------------------- rows: metadata, observations, state write-back  // PHASE: rows pass1
@@ -726,18 +685,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
       for (int pass = 0; pass < 2; ++pass) {  // 0: rows of the agents that acted, 1: newborn rows
       if (pass == 1) {
         if (births[0] + births[1] == 0) break;
-        if (!SPLIT) {
-          // newborn rows: their first row depends on the births of every env before this one; by now
-          // (all other work of this env is done) the predecessors have normally published theirs
-          int nb0 = 0, nb1 = 0;
-          if (!prefix_before(p.cntB[par], p.sum1[par], p.sum2[par], 2, env, epoch, true, lane, nb0, nb1)) {
-            if (lane == 0) atomicOr(p.error, 1u);
-          }
-          new_base[0] = n_old_total[0] + nb0;
-          new_base[1] = n_old_total[1] + nb1;
-        }
-        // SPLIT: nobody waits — the observation kernel (which runs after every env has published its births) places the
-        // newborn rows and writes their labels (nb_info)
+        if (!SPLIT) newborn_base(p, L, env, lane, new_base);
       }
 #pragma unroll 1
       for (int s = 0; s < 2; ++s) {
@@ -824,13 +772,7 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
       }
       }
       PHASE_MARK(14)
-      if (mode == 2) publish_end(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane, pubA, pubB);
-      if (lane < 2) {  // PHASE: tail
-        const int nb = lane == 0 ? births[0] : births[1];
-        if (!SPLIT) p.new_off[lane][env] = nb > 0 ? (lane == 0 ? new_base[0] : new_base[1]) : 0;
-        p.new_cnt[lane][env] = nb;
-      }
-      if (SPLIT) dump_image(sbase, p, env, mode, keep, old_base, n, births, lane);  // before the maps are un-written
+      env_rows_done<SPLIT>(p, L, sbase, env, mode, keep, old_base, n, births, new_base, next_live, lane);  // PHASE: tail
       PHASE_MARK(15)
       // leave the maps empty for the next env of this warp: un-write every cell that can hold an entry
       // (a non-zero owner entry always has its owner standing on it)
@@ -865,57 +807,16 @@ __global__ void __launch_bounds__(W * 32, PPG_MIN_CTAS / W) ppg_step_base_kernel
       PHASE_MARK(16)
       if (over) h.state = p.autoreset ? ST_NEEDS_RESET : ST_IDLE;  // idle: final state stays readable
       if (lane == 0) p.hdr[env] = h;
-      // per-env counters (PPG_STAT_*): lane k adds statistic k (selects, no divergent switch)
-      if (lane < PPG_N_STATS) {
-        unsigned add = 0;
-        if (mode == 2) {
-          add = lane == PPG_STAT_ENV_STEPS ? 1u : add;
-          add = lane == PPG_STAT_AGENT_STEPS ? (unsigned)(n[0] + n[1]) : add;
-          add = lane == PPG_STAT_EPISODES ? (unsigned)over : add;
-          add = lane == PPG_STAT_EPISODE_STEPS ? (over ? h.step : 0u) : add;
-          add = lane == PPG_STAT_BIRTHS_PRED ? (unsigned)births[0] : add;
-          add = lane == PPG_STAT_BIRTHS_PREY ? (unsigned)births[1] : add;
-          add = lane == PPG_STAT_STARVED_PRED ? st_starved[0] : add;
-          add = lane == PPG_STAT_STARVED_PREY ? st_starved[1] : add;
-          add = lane == PPG_STAT_EATEN_PREY ? st_eaten : add;
-          add = lane == PPG_STAT_GRASS_EATEN ? st_grass : add;
-          add = lane == PPG_STAT_TRUNCATED ? (unsigned)trunc : add;
-          add = lane == PPG_STAT_SPAWN_FALLBACK ? st_fallback : add;
-        }
-        if (lane == PPG_STAT_ROWS_PRED) add = n[0] + births[0];
-        if (lane == PPG_STAT_ROWS_PREY) add = n[1] + births[1];
-        if (add) atomicAdd(p.counters + (size_t)env * PPG_N_STATS + lane, add);  // RED: nobody waits for the old value
-      }
+      add_stats(p, env, mode, n, births, over, trunc, h.step, st, lane);
     } else {
-      if (lane < 2) {
-        p.new_off[lane][env] = 0;
-        p.new_cnt[lane][env] = 0;
-      }
-      if (SPLIT) dump_image(sbase, p, env, 0, false, old_base, n, births, lane);  // header only: no rows
+      env_idle<SPLIT>(p, sbase, env, old_base, lane);
     }
-    if (lane == 0) {
-      p.env_cycles[env] = make_uint4((unsigned)(clock64() - t_env0), (unsigned)mode | ((unsigned)(births[0] + births[1]) << 8) | ((unsigned)(n[0] + n[1]) << 16), t_ns0, smid());
-      p.env_flags[env] = (uint8_t)env_flags;
-      p.env_status[env] = h.status;
-      p.env_step[env] = h.step;
-      p.env_count[2 * env] = mode == 0 ? h.n_list[0] : cur[0];
-      p.env_count[2 * env + 1] = mode == 0 ? h.n_list[1] : cur[1];
-    }
-    if (SPLIT && lane == 0) { pend = q_slot + 1ULL; pend_env = env; }  // handed over from the top of the loop (queue_push)
-    __syncwarp();
-#if !PPG_PUSH_DEFER
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
-#endif
-#if !PPG_TICKET_EARLY
-    if (W == 1 && lane == 0) {
-      env_next = t_first + (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-      if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-    }
-#endif
+    const int count[2] = {mode == 0 ? h.n_list[0] : cur[0], mode == 0 ? h.n_list[1] : cur[1]};
+    env_end<SPLIT>(p, L, env, mode, n, births, env_flags, h, t_env0, t_ns0, count, true, lane);
     PHASE_MARK(17)
     PHASE_FLUSH(base)
   }
-  if (SPLIT) queue_push(p, pend, pend_env, lane);
+  if (SPLIT) queue_push(p, L.pend, L.pend_env, lane);
   if (lane == 0) bulk_wait_read<0>();  // shared memory must stay valid until the engine has read it
   SPAN_MARK(base, 2)
 }
@@ -1070,52 +971,21 @@ __global__ void ppg_stats_kernel(const uint32_t* __restrict__ counters, const En
 // ------------------------------------------------------------------------------------------------
 // launch wrappers used by ppg_api.cu
 // ------------------------------------------------------------------------------------------------
-template <int W, typename MapT, bool BULK, bool SPLIT>
-static cudaError_t launch_w(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  static size_t attr_bytes = 0;  // opt in to > 48 KB of dynamic shared memory (grows monotonically)
-  if (smem > attr_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(ppg_step_base_kernel<W, MapT, BULK, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    attr_bytes = smem;
-  }
-  return pdl_launch(ppg_step_base_kernel<W, MapT, BULK, SPLIT>, dim3((unsigned)n_cta), dim3(W * 32), smem, stream, p);
-}
-
-template <int W, typename MapT, bool BULK, bool SPLIT>
-static cudaError_t occupancy_w(size_t smem, int* blocks_per_sm) {
-  cudaError_t e = cudaFuncSetAttribute(ppg_step_base_kernel<W, MapT, BULK, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, ppg_step_base_kernel<W, MapT, BULK, SPLIT>, W * 32, smem);
-}
-
 // SPLIT (two-kernel step) exists for one warp per CTA and direct stores only (ppg_create enforces it)
-#define PPG_DISPATCH(FN, ...)                                                                     \
-  do {                                                                                            \
-    const bool m8 = map_bytes == 1;                                                               \
-    if (split) return m8 ? FN<1, uint8_t, false, true>(__VA_ARGS__) : FN<1, uint16_t, false, true>(__VA_ARGS__); \
-    if (warps_per_cta == 1) {                                                                     \
-      if (bulk) return m8 ? FN<1, uint8_t, true, false>(__VA_ARGS__) : FN<1, uint16_t, true, false>(__VA_ARGS__); \
-      return m8 ? FN<1, uint8_t, false, false>(__VA_ARGS__) : FN<1, uint16_t, false, false>(__VA_ARGS__);       \
-    }                                                                                             \
-    if (warps_per_cta == 4) {                                                                     \
-      if (bulk) return m8 ? FN<4, uint8_t, true, false>(__VA_ARGS__) : FN<4, uint16_t, true, false>(__VA_ARGS__); \
-      return m8 ? FN<4, uint8_t, false, false>(__VA_ARGS__) : FN<4, uint16_t, false, false>(__VA_ARGS__);       \
-    }                                                                                             \
-    if (warps_per_cta == 8) {                                                                     \
-      if (bulk) return m8 ? FN<8, uint8_t, true, false>(__VA_ARGS__) : FN<8, uint16_t, true, false>(__VA_ARGS__); \
-      return m8 ? FN<8, uint8_t, false, false>(__VA_ARGS__) : FN<8, uint16_t, false, false>(__VA_ARGS__);       \
-    }                                                                                             \
-    return cudaErrorInvalidValue;                                                                 \
-  } while (0)
-
-cudaError_t launch_step_base(const StepParams& p, int warps_per_cta, int n_cta, size_t smem, cudaStream_t stream) {
-  const int map_bytes = p.map_bytes;
-  const bool bulk = p.obs_bulk != 0, split = p.obs_split != 0;
-  PPG_DISPATCH(launch_w, p, n_cta, smem, stream);
+template <typename MapT>
+static StepKernel base_kernel(const StepParams& p, int warps_per_cta) {
+  const bool bulk = p.obs_bulk != 0;
+  if (p.obs_split) return {ppg_step_base_kernel<1, MapT, false, true>, 32};
+  switch (warps_per_cta) {
+    case 1: return {bulk ? ppg_step_base_kernel<1, MapT, true, false> : ppg_step_base_kernel<1, MapT, false, false>, 32};
+    case 4: return {bulk ? ppg_step_base_kernel<4, MapT, true, false> : ppg_step_base_kernel<4, MapT, false, false>, 4 * 32};
+    case 8: return {bulk ? ppg_step_base_kernel<8, MapT, true, false> : ppg_step_base_kernel<8, MapT, false, false>, 8 * 32};
+    default: return {nullptr, 0};
+  }
 }
 
-cudaError_t step_base_occupancy(int warps_per_cta, int map_bytes, bool bulk, bool split, size_t smem, int* blocks_per_sm) {
-  PPG_DISPATCH(occupancy_w, smem, blocks_per_sm);
+StepKernel step_kernel_base(const StepParams& p, int warps_per_cta) {
+  return p.map_bytes == 1 ? base_kernel<uint8_t>(p, warps_per_cta) : base_kernel<uint16_t>(p, warps_per_cta);
 }
 
 cudaError_t launch_prepare_offsets(const EnvHdr* hdr, int B, int n0, int n1, unsigned long long* cntA, unsigned long long* sum1,

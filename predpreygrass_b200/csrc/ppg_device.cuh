@@ -337,6 +337,13 @@ struct LinksParams {
   int save_only;         // 1: only save the tables (switch-on, ppg_restore); prev_row is not written
 };
 
+// A step kernel instantiation and its block size: ppg_create picks the handle's one (step_kernel_base / _eco / _stag), sizes the
+// grid with its occupancy, and every step launches it.
+struct StepKernel {
+  void (*fn)(StepParams);
+  int threads;
+};
+
 // Launch with programmatic stream serialization (PDL): the grid's CTAs may be scheduled as soon as every CTA of the kernel
 // before it in the stream has executed griddepcontrol.launch_dependents (or exited), which hides the launch ramp of the 2960
 // one-warp CTAs of a step kernel behind the tail of the observation kernel.  The kernel MUST execute griddepcontrol.wait before

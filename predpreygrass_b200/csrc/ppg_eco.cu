@@ -224,8 +224,6 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
   const RowDesc D = carve_desc(sbase, p);
   const unsigned sb32 = (unsigned)__cvta_generic_to_shared(sbase);
   const int G = p.G, GG = p.GG, PP = p.P, PS = p.PS;
-  const unsigned epoch = p.epoch;
-  const int par = (int)(epoch & 1u);
   const unsigned lt_mask = (1u << lane) - 1u;
   const int AR = p.action_range, AD = (p.action_range - 1) / 2;
 
@@ -233,17 +231,12 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
   for (int i = lane; i < p.init_bytes / 16; i += 32)
     reinterpret_cast<uint4*>(sbase + p.so_map[0])[i] = __ldg(reinterpret_cast<const uint4*>(p.init_image) + i);
   unsigned rowctr = 0;
-  const int n_old_total[2] = {p.totals[(par ^ 1) * 4 + 0], p.totals[(par ^ 1) * 4 + 1]};
-  const int n_blk = (p.B + 31) >> 5, n_grp = (p.B + 1023) >> 10;
+  EnvLoop L = env_loop(p, false);  // an env at its episode end may wait for the births of lower envs: index order
   __syncwarp();
 
-  // envs come from the ticket counter; after the first one the ticket is drawn while the previous env is being finished (ppg_base.cu)
-  int env_next = 0;
-  if (lane == 0) env_next = (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-  unsigned long long pend = 0ULL;  // lane 0: completion-queue slot + 1 of the env whose hand-over is still owed (queue_push)
-  int pend_env = 0;
+  if (lane == 0) next_ticket(p, L, true);
   for (;;) {
-    const int env = __shfl_sync(FULL, env_next, 0);
+    const int env = __shfl_sync(FULL, L.env_next, 0);
     if (env >= p.B) break;
 
     int n[2] = {0, 0};
@@ -253,7 +246,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
     int next_live[2] = {0, 0};
     int mode = 0;
     unsigned env_flags = 0;
-    unsigned st_starved[2] = {0, 0}, st_eaten = 0, st_grass = 0, st_fallback = 0;
+    EnvStats st = {};
     bool over = false, trunc = false, done = false, have_new_base = false;
     int n_gh = 0;  // ghost cells loaded into the pseudo-slots cap[1]-1, cap[1]-2, ...
     double ep_dist[2] = {0.0, 0.0}, ep_cost[2] = {0.0, 0.0};  // this step's distance moved / locomotion energy per species (per lane)
@@ -296,20 +289,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
     // founders of the episode a reset starts: constant for ECO, drawn per episode by the trait variants (MR:189-192)
     int nf[2] = {p.n_init[0], p.n_init[1]};
     if (ppg_random_founders(tm) && ((unsigned)h.pad[1] & 0x80000000u)) { nf[0] = h.pad[0] & 0xFFFF; nf[1] = (h.pad[0] >> 16) & 0x7FFF; }
-    if (!prefix_before(p.cntA[par ^ 1], p.sum1[par ^ 1], p.sum2[par ^ 1], 0, env, epoch - 1u, false, lane, old_base[0], old_base[1])) {
-      if (lane == 0) atomicOr(p.error, 2u);
-    }
-    // hand-over of the PREVIOUS env of this warp, after this env's first loads were issued (queue_push, ppg_step_common.cuh)
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
-    if (h.state & ST_NEEDS_RESET) mode = 1;
-    else if (h.state & ST_IDLE) mode = 0;
-    else mode = 2;
-    if (mode != 2) {
-      // reset / idle envs know their counts up front (founders, no births): publish them before doing any work, so
-      // that later envs waiting for their newborn-row prefix never wait for a reset
-      if (mode == 1) { next_live[0] = nf[0]; next_live[1] = nf[1]; }
-      publish_counts(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane);
-    }
+    mode = env_begin<SPLIT>(p, L, env, h.state, nf, old_base, next_live, lane);
     const unsigned genv = (unsigned)(env + p.env_base);
 
     if (PPG_UNLIKELY(mode == 1)) {
@@ -701,7 +681,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
               SEL(S.flg)[slot] = F_DIED;  // also drops FC (dead_prey.discard, ECO:768-769) and F_CAUGHT (reward 0, ECO:772)
               if (LIN) lineage_set_alive(p, env, s, SEL(S.id)[slot], 0);  // ECO:770
             }
-            if (s == 0) { eh.active[0] -= 1; st_starved[0]++; } else { eh.active[1] -= 1; st_starved[1]++; }
+            if (s == 0) { eh.active[0] -= 1; st.starved[0]++; } else { eh.active[1] -= 1; st.starved[1]++; }
             __syncwarp();
           }
         }
@@ -724,7 +704,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
             S.gE[gg - 1] = 0.0;
             S.flg[1][sl] = (uint8_t)(f | F_ATE);
           }
-          st_grass++;
+          st.grass++;
           __syncwarp();
         }
       }
@@ -754,7 +734,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
             S.gE[g - 1] = rem > 0.0 ? rem : 0.0;
             S.flg[1][slot] |= F_ATE;
           }
-          st_grass += __popc(__ballot_sync(FULL, eat));
+          st.grass += __popc(__ballot_sync(FULL, eat));
           __syncwarp();
           continue;
         }
@@ -777,7 +757,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
               S.gE[gg - 1] = rem > 0.0 ? rem : 0.0;
               S.flg[1][sl] = (uint8_t)(f | F_ATE);
             }
-            st_grass++;
+            st.grass++;
             __syncwarp();
           }
         }
@@ -878,7 +858,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
                 S.flg[1][q] = (uint8_t)((qf & F_ATE) | F_DIED | F_CAUGHT);
               }
               eh.active[1] -= 1;  // also for a prey that already starved or aged out this step (quirk 4)
-              st_eaten++;
+              st.eaten++;
               __syncwarp();
             }
           }
@@ -960,7 +940,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
               }
             }
             if (PPG_UNLIKELY(sx < 0)) {
-              st_fallback++;
+              st.fallback++;
               if (p.tape_cells != nullptr && h.tape_pos < h.tape_end) {
                 const int c = p.tape_cells[h.tape_pos++];
                 sx = c / G; sy = c % G;
@@ -1008,12 +988,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
               __syncwarp();
             } else if (maybe_done) {
               if (!have_new_base) {
-                int nb0 = 0, nb1 = 0;
-                if (!prefix_before(p.cntB[par], p.sum1[par], p.sum2[par], 2, env, epoch, true, lane, nb0, nb1)) {
-                  if (lane == 0) atomicOr(p.error, 1u);
-                }
-                new_base[0] = n_old_total[0] + nb0;
-                new_base[1] = n_old_total[1] + nb1;
+                newborn_base(p, L, env, lane, new_base);
                 have_new_base = true;
               }
               rowctr = emit_row_now<MapT, false, true>(sbase, p, p.obs[s] + (size_t)(SEL(new_base) + cs - SEL(n)) * p.elems[s], CELLXY(sx, sy), s,
@@ -1049,14 +1024,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
       env_flags = PPG_ENV_IDLE;
     }
 
-    // four atomics back to back, nobody waits for them here (ppg_base.cu): the warp's next env, this env's slot in the
-    // completion queue, the two accumulators of the row allocation
-#if PPG_TICKET_EARLY
-    if (lane == 0) env_next = (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-#endif
-    unsigned long long q_slot = 0ULL, pubA = 0ULL, pubB = 0ULL;
-    if (SPLIT) q_slot = queue_reserve(p, lane);
-    if (mode == 2) publish_begin(p, env, par, epoch, next_live, births, lane, pubA, pubB, 0);
+    env_publish<SPLIT>(p, L, env, mode, next_live, births, 0, true, lane);
 
     // ------------------------------------------------- rows: metadata, observations, state write-back
     if (lane == 0) {
@@ -1070,15 +1038,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
       for (int pass = 0; pass < 2; ++pass) {  // 0: rows of the agents that acted, 1: newborn rows
         if (pass == 1) {
           if (births[0] + births[1] == 0) break;
-          // SPLIT: the observation kernel places the newborn rows (nobody waits here)
-          if (!SPLIT && !have_new_base) {
-            int nb0 = 0, nb1 = 0;
-            if (!prefix_before(p.cntB[par], p.sum1[par], p.sum2[par], 2, env, epoch, true, lane, nb0, nb1)) {
-              if (lane == 0) atomicOr(p.error, 1u);
-            }
-            new_base[0] = n_old_total[0] + nb0;
-            new_base[1] = n_old_total[1] + nb1;
-          }
+          if (!SPLIT && !have_new_base) newborn_base(p, L, env, lane, new_base);
         }
 #pragma unroll 1
         for (int s = 0; s < 2; ++s) {
@@ -1174,13 +1134,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
           }
         }
       }
-      if (mode == 2) publish_end(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane, pubA, pubB);
-      if (lane < 2) {
-        const int nb = lane == 0 ? births[0] : births[1];
-        if (!SPLIT) p.new_off[lane][env] = nb > 0 ? (lane == 0 ? new_base[0] : new_base[1]) : 0;
-        p.new_cnt[lane][env] = nb;
-      }
-      if (SPLIT) dump_image(sbase, p, env, mode, keep, old_base, n, births, lane);  // before the maps are un-written
+      env_rows_done<SPLIT>(p, L, sbase, env, mode, keep, old_base, n, births, new_base, next_live, lane);
       // ghost cells of the next step: loaded ghosts whose entry nobody overwrote or zeroed, and prey that aged out this
       // step and were written back as carcasses (their entry outlives them).  Only a finite intake cap can create them.
       {
@@ -1244,54 +1198,13 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_eco_kernel(const __gr
       }
       if (over) h.state = p.autoreset ? ST_NEEDS_RESET : ST_IDLE;
       if (lane == 0) { p.hdr[env] = h; p.ehdr[env] = eh; }
-      if (lane < PPG_N_STATS) {
-        unsigned add = 0;
-        if (mode == 2) {
-          switch (lane) {
-            case PPG_STAT_ENV_STEPS: add = 1; break;
-            case PPG_STAT_AGENT_STEPS: add = n[0] + n[1]; break;
-            case PPG_STAT_EPISODES: add = over; break;
-            case PPG_STAT_EPISODE_STEPS: add = over ? h.step : 0; break;
-            case PPG_STAT_BIRTHS_PRED: add = births[0]; break;
-            case PPG_STAT_BIRTHS_PREY: add = births[1]; break;
-            case PPG_STAT_STARVED_PRED: add = st_starved[0]; break;
-            case PPG_STAT_STARVED_PREY: add = st_starved[1]; break;
-            case PPG_STAT_EATEN_PREY: add = st_eaten; break;
-            case PPG_STAT_GRASS_EATEN: add = st_grass; break;
-            case PPG_STAT_TRUNCATED: add = trunc; break;
-            case PPG_STAT_SPAWN_FALLBACK: add = st_fallback; break;
-            default: break;
-          }
-        }
-        if (lane == PPG_STAT_ROWS_PRED) add = n[0] + births[0];
-        if (lane == PPG_STAT_ROWS_PREY) add = n[1] + births[1];
-        if (add) atomicAdd(p.counters + (size_t)env * PPG_N_STATS + lane, add);  // RED: nobody waits for the old value
-      }
+      add_stats(p, env, mode, n, births, over, trunc, h.step, st, lane);
     } else {
-      if (lane < 2) {
-        p.new_off[lane][env] = 0;
-        p.new_cnt[lane][env] = 0;
-      }
-      if (SPLIT) dump_image(sbase, p, env, 0, false, old_base, n, births, lane);  // header only: no rows
+      env_idle<SPLIT>(p, sbase, env, old_base, lane);
     }
-    if (lane == 0) {
-      p.env_cycles[env] = make_uint4((unsigned)(clock64() - t_env0), (unsigned)mode | ((unsigned)(births[0] + births[1]) << 8) | ((unsigned)(n[0] + n[1]) << 16), t_ns0, smid());
-      p.env_flags[env] = (uint8_t)env_flags;
-      p.env_status[env] = h.status;
-      p.env_step[env] = h.step;
-      p.env_count[2 * env] = eh.active[0];
-      p.env_count[2 * env + 1] = eh.active[1];
-    }
-    if (SPLIT && lane == 0) { pend = q_slot + 1ULL; pend_env = env; }  // handed over from the top of the loop (queue_push)
-    __syncwarp();
-#if !PPG_PUSH_DEFER
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
-#endif
-#if !PPG_TICKET_EARLY
-    if (lane == 0) env_next = (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-#endif
+    env_end<SPLIT>(p, L, env, mode, n, births, env_flags, h, t_env0, t_ns0, eh.active, true, lane);
   }
-  if (SPLIT) queue_push(p, pend, pend_env, lane);
+  if (SPLIT) queue_push(p, L.pend, L.pend_env, lane);
 }
 
 // trait variants: founders of the episode a scheduled reset will start (see draw_next_founders), after ppg_reset marked the envs
@@ -1312,59 +1225,29 @@ __global__ void ppg_set_tape_reals_kernel(EcoHdr* ehdr, int B, const long long* 
   ehdr[e].real_end = real_off ? real_off[e + 1] : 0;
 }
 
-template <typename MapT, bool SPLIT, int KIND>
-static cudaError_t launch_eco_t(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  static size_t attr_bytes = 0;
-  if (smem > attr_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(ppg_step_eco_kernel<1, MapT, SPLIT, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    attr_bytes = smem;
-  }
-  return pdl_launch(ppg_step_eco_kernel<1, MapT, SPLIT, KIND>, dim3((unsigned)n_cta), dim3(32), smem, stream, p);
-}
-
-template <int KIND>
-static cudaError_t launch_eco_v(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  if (p.obs_split) return p.map_bytes == 1 ? launch_eco_t<uint8_t, true, KIND>(p, n_cta, smem, stream) : launch_eco_t<uint16_t, true, KIND>(p, n_cta, smem, stream);
-  return p.map_bytes == 1 ? launch_eco_t<uint8_t, false, KIND>(p, n_cta, smem, stream) : launch_eco_t<uint16_t, false, KIND>(p, n_cta, smem, stream);
-}
-template <int KIND>
-static cudaError_t launch_eco_split(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  return p.map_bytes == 1 ? launch_eco_t<uint8_t, true, KIND>(p, n_cta, smem, stream) : launch_eco_t<uint16_t, true, KIND>(p, n_cta, smem, stream);
-}
-cudaError_t launch_step_eco(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  if (p.trait_mode != PPG_TRAIT_SPEED && p.obs_split) {
+template <typename MapT>
+static StepKernel eco_kernel(const StepParams& p) {
+  const bool split = p.obs_split != 0;
+  if (p.trait_mode != PPG_TRAIT_SPEED) {
+    if (!split) return {ppg_step_eco_kernel<1, MapT, false, 1>, 32};
     switch (p.trait_mode) {
-      case PPG_TRAIT_METABOLIC: return launch_eco_split<10 + PPG_TRAIT_METABOLIC>(p, n_cta, smem, stream);
-      case PPG_TRAIT_INVESTMENT: return launch_eco_split<10 + PPG_TRAIT_INVESTMENT>(p, n_cta, smem, stream);
-      case PPG_TRAIT_COOPERATION: return launch_eco_split<10 + PPG_TRAIT_COOPERATION>(p, n_cta, smem, stream);
-      case PPG_TRAIT_CADENCE: return launch_eco_split<10 + PPG_TRAIT_CADENCE>(p, n_cta, smem, stream);
-      default: break;
+      case PPG_TRAIT_METABOLIC: return {ppg_step_eco_kernel<1, MapT, true, 10 + PPG_TRAIT_METABOLIC>, 32};
+      case PPG_TRAIT_INVESTMENT: return {ppg_step_eco_kernel<1, MapT, true, 10 + PPG_TRAIT_INVESTMENT>, 32};
+      case PPG_TRAIT_COOPERATION: return {ppg_step_eco_kernel<1, MapT, true, 10 + PPG_TRAIT_COOPERATION>, 32};
+      case PPG_TRAIT_CADENCE: return {ppg_step_eco_kernel<1, MapT, true, 10 + PPG_TRAIT_CADENCE>, 32};
+      default: return {nullptr, 0};
     }
   }
-  if (p.trait_mode != PPG_TRAIT_SPEED) return launch_eco_v<1>(p, n_cta, smem, stream);
-  if (p.lin_on) return launch_eco_v<2>(p, n_cta, smem, stream);
+  if (p.lin_on) return {split ? ppg_step_eco_kernel<1, MapT, true, 2> : ppg_step_eco_kernel<1, MapT, false, 2>, 32};
   // the shipped config reaches none of the carcass / ghost-cell / juvenile / episode-sum code: the kernel without it (KIND 3)
-  const bool lean = p.obs_split && p.trait_mode == PPG_TRAIT_SPEED && !(p.bite_cap_prey < HUGE_VAL) && p.carcass_age < 0 && p.ep_sums == nullptr;
-  if (const char* ev = getenv("PPG_ECO_LEAN")) { if (atoi(ev) == 0) return launch_eco_v<0>(p, n_cta, smem, stream); }
-  return lean ? launch_eco_split<3>(p, n_cta, smem, stream) : launch_eco_v<0>(p, n_cta, smem, stream);
+  bool lean = split && !(p.bite_cap_prey < HUGE_VAL) && p.carcass_age < 0 && p.ep_sums == nullptr;
+  if (const char* ev = getenv("PPG_ECO_LEAN")) lean = lean && atoi(ev) != 0;
+  if (lean) return {ppg_step_eco_kernel<1, MapT, true, 3>, 32};
+  return {split ? ppg_step_eco_kernel<1, MapT, true, 0> : ppg_step_eco_kernel<1, MapT, false, 0>, 32};
 }
 
-template <typename MapT, bool SPLIT, int KIND>
-static cudaError_t occupancy_eco_t(size_t smem, int* blocks_per_sm) {
-  cudaError_t e = cudaFuncSetAttribute(ppg_step_eco_kernel<1, MapT, SPLIT, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, ppg_step_eco_kernel<1, MapT, SPLIT, KIND>, 32, smem);
-}
-
-template <int KIND>
-static cudaError_t occupancy_eco_v(int map_bytes, bool split, size_t smem, int* blocks_per_sm) {
-  if (split) return map_bytes == 1 ? occupancy_eco_t<uint8_t, true, KIND>(smem, blocks_per_sm) : occupancy_eco_t<uint16_t, true, KIND>(smem, blocks_per_sm);
-  return map_bytes == 1 ? occupancy_eco_t<uint8_t, false, KIND>(smem, blocks_per_sm) : occupancy_eco_t<uint16_t, false, KIND>(smem, blocks_per_sm);
-}
-cudaError_t step_eco_occupancy(int map_bytes, bool split, int kind, size_t smem, int* blocks_per_sm) {
-  if (kind == 1) return occupancy_eco_v<1>(map_bytes, split, smem, blocks_per_sm);
-  return kind == 2 ? occupancy_eco_v<2>(map_bytes, split, smem, blocks_per_sm) : occupancy_eco_v<0>(map_bytes, split, smem, blocks_per_sm);
+StepKernel step_kernel_eco(const StepParams& p) {
+  return p.map_bytes == 1 ? eco_kernel<uint8_t>(p) : eco_kernel<uint16_t>(p);
 }
 
 cudaError_t launch_eco_founders(const StepParams& p, cudaStream_t s) {

@@ -167,8 +167,6 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
   const RowDesc D = carve_desc(sbase, p);
   const unsigned sb32 = (unsigned)__cvta_generic_to_shared(sbase);
   const int G = p.G, GG = p.GG, PP = p.P, PS = p.PS;
-  const unsigned epoch = p.epoch;
-  const int par = (int)(epoch & 1u);
   const unsigned lt_mask = (1u << lane) - 1u;
   const int T2[2] = {p.n_possible_t[0][0], p.n_possible_t[1][0]};  // first flat id of type 2 per species
 
@@ -176,26 +174,15 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
   for (int i = lane; i < p.init_bytes / 16; i += 32)
     reinterpret_cast<uint4*>(sbase + p.so_map[0])[i] = __ldg(reinterpret_cast<const uint4*>(p.init_image) + i);
   unsigned rowctr = 0;
-  const int n_old_total[2] = {p.totals[(par ^ 1) * 4 + 0], p.totals[(par ^ 1) * 4 + 1]};
-  const int n_blk = (p.B + 31) >> 5, n_grp = (p.B + 1023) >> 10;
+  EnvLoop L = env_loop(p, SPLIT);
   __syncwarp();
 
   // owner map of a prey slot's grid channel (STAG:2082-2092)
   auto prey_map = [&](int slot) -> MapT* { return (int)S.id[1][slot] >= T2[1] ? X.map3 : S.map[1]; };
 
-  // envs come from the ticket counter; after the first one the ticket is drawn while the previous env is being finished (ppg_base.cu)
-  // ticket -> env: big envs first when the previous launch left an order (publish_begin), else index order
-  const int32_t* const perm = (SPLIT && p.perm[par ^ 1] != nullptr && p.perm_tag[par ^ 1] == epoch - 1u) ? p.perm[par ^ 1] : nullptr;
-  const int t_first = p.static_first ? min((int)gridDim.x, p.B) : 0;  // first ticket of a warp = its CTA index (ppg_base.cu)
-  int env_next = 0;
-  if (lane == 0) {
-    env_next = p.static_first ? min((int)blockIdx.x, p.B) : (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-    if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-  }
-  unsigned long long pend = 0ULL;  // lane 0: completion-queue slot + 1 of the env whose hand-over is still owed (queue_push)
-  int pend_env = 0;
+  if (lane == 0) next_ticket(p, L, true);
   for (;;) {
-    const int env = __shfl_sync(FULL, env_next, 0);
+    const int env = __shfl_sync(FULL, L.env_next, 0);
     if (env >= p.B) break;
 
     int n[2] = {0, 0};
@@ -206,7 +193,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
     int live[2] = {0, 0};
     int mode = 0;
     unsigned env_flags = 0;
-    unsigned st_starved[2] = {0, 0}, st_eaten = 0, st_grass = 0, st_fallback = 0, st_attempts = 0;
+    EnvStats st = {};
     bool over = false, trunc = false, done = false;
 
     const long long t_env0 = clock64();
@@ -238,18 +225,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
       const int g = lane + 32 * q;
       if (g < p.n_grass) { gp_r[q] = p.gr_pos[(size_t)env * p.n_grass + g]; ge_r[q] = p.gr_e[(size_t)env * p.n_grass + g]; }
     }
-    if (!prefix_before(p.cntA[par ^ 1], p.sum1[par ^ 1], p.sum2[par ^ 1], 0, env, epoch - 1u, false, lane, old_base[0], old_base[1])) {
-      if (lane == 0) atomicOr(p.error, 2u);
-    }
-    // hand-over of the PREVIOUS env of this warp, after this env's first loads were issued (queue_push, ppg_step_common.cuh)
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
-    if (h.state & ST_NEEDS_RESET) mode = 1;
-    else if (h.state & ST_IDLE) mode = 0;
-    else mode = 2;
-    if (mode != 2) {
-      if (mode == 1) { next_live[0] = p.n_init[0]; next_live[1] = p.n_init[1]; }
-      publish_counts(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane);
-    }
+    mode = env_begin<SPLIT>(p, L, env, h.state, p.n_init, old_base, next_live, lane);
     const unsigned genv = (unsigned)(env + p.env_base);
 
     if (PPG_UNLIKELY(mode == 1)) {
@@ -554,7 +530,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
             ++c;
           }
         c = __reduce_add_sync(FULL, c);
-        if (s == 0) st_starved[0] += c; else st_starved[1] += c;
+        if (s == 0) st.starved[0] += c; else st.starved[1] += c;
       }
       __syncwarp();
 
@@ -611,7 +587,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
         const bool clash = eat && S.gtag[g - 1] != (uint8_t)lane;
         if (!__any_sync(FULL, clash)) {
           if (eat) graze(slot, g);
-          st_grass += __popc(__ballot_sync(FULL, eat));
+          st.grass += __popc(__ballot_sync(FULL, eat));
           __syncwarp();
           continue;
         }
@@ -621,7 +597,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
           const int l = __ffs(em) - 1;
           em &= em - 1;
           if (lane == l) graze(slot, g);
-          st_grass++;
+          st.grass++;
           __syncwarp();
         }
       }
@@ -694,7 +670,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
               }
               sh.capture_real[0] = prob; sh.capture_real[1] = ratio; sh.capture_real[2] += prob;  // STAG:1176-1179
               sh.capture[8] += 1;
-              st_attempts++;
+              st.attempts++;
               const double join_cost = p.join_cost;
               if (!success) {
                 if (join_cost != 0.0) {  // STAG:1185-1192
@@ -756,7 +732,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
                     ++c;
                   }
                 }
-                st_starved[0] += __reduce_add_sync(FULL, c);
+                st.starved[0] += __reduce_add_sync(FULL, c);
                 __syncwarp();
               }
               if (captured) {  // prey termination (STAG:1419-1440)
@@ -764,7 +740,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
                   (ptype ? X.map3 : S.map[1])[pcell] = 0;
                   S.flg[1][prey] = F_DIED | F_CAUGHT;
                 }
-                st_eaten++;
+                st.eaten++;
                 __syncwarp();
               }
             }
@@ -772,7 +748,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
               const int g = S.map[2][pcell];
               if (g != 0) {
                 if (lane == 0) graze(prey, g);
-                st_grass++;
+                st.grass++;
               }
               __syncwarp();
             }
@@ -834,7 +810,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
             }
             if (sx < 0) {
               if (count_free_cells<MapT>(sbase, p, nl[0], nl[1], lane) == 0) { h.status |= PPG_STATUS_NO_SPAWN_CELL; continue; }  // no draw (STAG:1041-1044)
-              st_fallback++;
+              st.fallback++;
               int c;
               if (stag_take_int(p, h, c)) { sx = c / G; sy = c % G; }
               else {
@@ -897,17 +873,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
       env_flags = PPG_ENV_IDLE;
     }
 
-    // four atomics back to back, nobody waits for them here (ppg_base.cu): the warp's next env, this env's slot in the
-    // completion queue, the two accumulators of the row allocation
-#if PPG_TICKET_EARLY
-    if (lane == 0) {
-      env_next = t_first + (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-      if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-    }
-#endif
-    unsigned long long q_slot = 0ULL, pubA = 0ULL, pubB = 0ULL;
-    if (SPLIT) q_slot = queue_reserve(p, lane);
-    if (mode == 2) publish_begin(p, env, par, epoch, next_live, births, lane, pubA, pubB, (n_old_total[0] + n_old_total[1]) / p.B * 5 / 4);
+    env_publish<SPLIT>(p, L, env, mode, next_live, births, (L.n_old_total[0] + L.n_old_total[1]) / p.B * 5 / 4, true, lane);
 
     // ------------------------------------------------- rows: metadata, observations, state write-back
     if (lane == 0) {
@@ -921,14 +887,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
       for (int pass = 0; pass < 2; ++pass) {  // 0: rows of the agents that acted, 1: newborn rows
         if (pass == 1) {
           if (births[0] + births[1] == 0) break;
-          if (!SPLIT) {  // SPLIT: the observation kernel places the newborn rows (nobody waits here)
-            int nb0 = 0, nb1 = 0;
-            if (!prefix_before(p.cntB[par], p.sum1[par], p.sum2[par], 2, env, epoch, true, lane, nb0, nb1)) {
-              if (lane == 0) atomicOr(p.error, 1u);
-            }
-            new_base[0] = n_old_total[0] + nb0;
-            new_base[1] = n_old_total[1] + nb1;
-          }
+          if (!SPLIT) newborn_base(p, L, env, lane, new_base);
         }
 #pragma unroll 1
         for (int s = 0; s < 2; ++s) {
@@ -1007,13 +966,7 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
           }
         }
       }
-      if (mode == 2) publish_end(p, env, par, epoch, next_live, births, n_blk, n_grp, n_old_total, lane, pubA, pubB);
-      if (lane < 2) {
-        const int nb = lane == 0 ? births[0] : births[1];
-        if (!SPLIT) p.new_off[lane][env] = nb > 0 ? (lane == 0 ? new_base[0] : new_base[1]) : 0;
-        p.new_cnt[lane][env] = nb;
-      }
-      if (SPLIT) dump_image(sbase, p, env, mode, keep, old_base, n, births, lane);  // before the maps are un-written
+      env_rows_done<SPLIT>(p, L, sbase, env, mode, keep, old_base, n, births, new_base, next_live, lane);
       // leave the maps empty for the next env of this warp: every loaded or born slot un-writes its cell in its channel
       #pragma unroll 1
       for (int i = lane; i < n[0] + births[0]; i += 32) S.map[0][CELLP((unsigned)S.pos[0][i])] = 0;
@@ -1033,60 +986,13 @@ __global__ void __launch_bounds__(W * 32, 16 / W) ppg_step_stag_kernel(const __g
       }
       if (over) h.state = p.autoreset ? ST_NEEDS_RESET : ST_IDLE;
       if (lane == 0) { p.hdr[env] = h; p.shdr[env] = sh; }
-      if (lane < PPG_N_STATS) {
-        unsigned add = 0;
-        if (mode == 2) {
-          switch (lane) {
-            case PPG_STAT_ENV_STEPS: add = 1; break;
-            case PPG_STAT_AGENT_STEPS: add = n[0] + n[1]; break;
-            case PPG_STAT_EPISODES: add = over; break;
-            case PPG_STAT_EPISODE_STEPS: add = over ? h.step : 0; break;
-            case PPG_STAT_BIRTHS_PRED: add = births[0]; break;
-            case PPG_STAT_BIRTHS_PREY: add = births[1]; break;
-            case PPG_STAT_STARVED_PRED: add = st_starved[0]; break;
-            case PPG_STAT_STARVED_PREY: add = st_starved[1]; break;
-            case PPG_STAT_EATEN_PREY: add = st_eaten; break;
-            case PPG_STAT_GRASS_EATEN: add = st_grass; break;
-            case PPG_STAT_TRUNCATED: add = trunc; break;
-            case PPG_STAT_SPAWN_FALLBACK: add = st_fallback; break;
-            case PPG_STAT_CAPTURE_ATTEMPTS: add = st_attempts; break;
-            default: break;
-          }
-        }
-        if (lane == PPG_STAT_ROWS_PRED) add = n[0] + births[0];
-        if (lane == PPG_STAT_ROWS_PREY) add = n[1] + births[1];
-        if (add) atomicAdd(p.counters + (size_t)env * PPG_N_STATS + lane, add);  // RED: nobody waits for the old value
-      }
+      add_stats(p, env, mode, n, births, over, trunc, h.step, st, lane);
     } else {
-      if (lane < 2) {
-        p.new_off[lane][env] = 0;
-        p.new_cnt[lane][env] = 0;
-      }
-      if (SPLIT) dump_image(sbase, p, env, 0, false, old_base, n, births, lane);  // header only: no rows
+      env_idle<SPLIT>(p, sbase, env, old_base, lane);
     }
-    if (lane == 0) {
-      p.env_cycles[env] = make_uint4((unsigned)(clock64() - t_env0), (unsigned)mode | ((unsigned)(births[0] + births[1]) << 8) | ((unsigned)(n[0] + n[1]) << 16), t_ns0, smid());
-      p.env_flags[env] = (uint8_t)env_flags;
-      p.env_status[env] = h.status;
-      p.env_step[env] = h.step;
-      if (mode != 0) {  // an idle env keeps the counts of its last step
-        p.env_count[2 * env] = live[0];
-        p.env_count[2 * env + 1] = live[1];
-      }
-    }
-    if (SPLIT && lane == 0) { pend = q_slot + 1ULL; pend_env = env; }  // handed over from the top of the loop (queue_push)
-    __syncwarp();
-#if !PPG_PUSH_DEFER
-    if (SPLIT) queue_push(p, pend, pend_env, lane);
-#endif
-#if !PPG_TICKET_EARLY
-    if (lane == 0) {
-      env_next = t_first + (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
-      if (perm != nullptr && env_next < p.B) env_next = perm[env_next];
-    }
-#endif
+    env_end<SPLIT>(p, L, env, mode, n, births, env_flags, h, t_env0, t_ns0, live, mode != 0, lane);  // an idle env keeps the counts of its last step
   }
-  if (SPLIT) queue_push(p, pend, pend_env, lane);
+  if (SPLIT) queue_push(p, L.pend, L.pend_env, lane);
 }
 
 // reals cursor of the replay tape
@@ -1125,32 +1031,13 @@ __global__ void ppg_random_actions_stag_kernel(const int32_t* __restrict__ n_row
   }
 }
 
-template <typename MapT, bool SPLIT>
-static cudaError_t launch_stag_t(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  static size_t attr_bytes = 0;
-  if (smem > attr_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(ppg_step_stag_kernel<1, MapT, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    attr_bytes = smem;
-  }
-  return pdl_launch(ppg_step_stag_kernel<1, MapT, SPLIT>, dim3((unsigned)n_cta), dim3(32), smem, stream, p);
+template <typename MapT>
+static StepKernel stag_kernel(const StepParams& p) {
+  return {p.obs_split ? ppg_step_stag_kernel<1, MapT, true> : ppg_step_stag_kernel<1, MapT, false>, 32};
 }
 
-cudaError_t launch_step_stag(const StepParams& p, int n_cta, size_t smem, cudaStream_t stream) {
-  if (p.obs_split) return p.map_bytes == 1 ? launch_stag_t<uint8_t, true>(p, n_cta, smem, stream) : launch_stag_t<uint16_t, true>(p, n_cta, smem, stream);
-  return p.map_bytes == 1 ? launch_stag_t<uint8_t, false>(p, n_cta, smem, stream) : launch_stag_t<uint16_t, false>(p, n_cta, smem, stream);
-}
-
-template <typename MapT, bool SPLIT>
-static cudaError_t occupancy_stag_t(size_t smem, int* blocks_per_sm) {
-  cudaError_t e = cudaFuncSetAttribute(ppg_step_stag_kernel<1, MapT, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, ppg_step_stag_kernel<1, MapT, SPLIT>, 32, smem);
-}
-
-cudaError_t step_stag_occupancy(int map_bytes, bool split, size_t smem, int* blocks_per_sm) {
-  if (split) return map_bytes == 1 ? occupancy_stag_t<uint8_t, true>(smem, blocks_per_sm) : occupancy_stag_t<uint16_t, true>(smem, blocks_per_sm);
-  return map_bytes == 1 ? occupancy_stag_t<uint8_t, false>(smem, blocks_per_sm) : occupancy_stag_t<uint16_t, false>(smem, blocks_per_sm);
+StepKernel step_kernel_stag(const StepParams& p) {
+  return p.map_bytes == 1 ? stag_kernel<uint8_t>(p) : stag_kernel<uint16_t>(p);
 }
 
 cudaError_t launch_set_tape_reals_stag(StagHdr* shdr, int B, const long long* real_off, cudaStream_t s) {

@@ -1,7 +1,7 @@
-// ppg_step_common.cuh — device code shared by the step kernels of all env variants (ppg_base.cu, ppg_eco.cu):
+// ppg_step_common.cuh — device code shared by the step kernels of all env variants (ppg_base.cu, ppg_eco.cu, ppg_stag.cu):
 // the per-env shared-memory view, the observation-row writers (two-level gather: padded byte maps -> fp32
-// value tables), the deterministic cross-env row allocation (hierarchical epoch-tagged counts) and the
-// Philox placement / free-cell draws.  See DESIGN.md §3.
+// value tables), the deterministic cross-env row allocation (hierarchical epoch-tagged counts), the
+// Philox placement / free-cell draws and the env loop around the variants' simulation.  See DESIGN.md §3.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -13,14 +13,6 @@ namespace ppg {
 // rarely taken branches (reset, replay tapes, explicit action order, fall-backs): kept out of the fall-through path, the step
 // kernels are bound by instruction delivery (DESIGN.md §3)
 #define PPG_UNLIKELY(x) __builtin_expect(!!(x), 0)
-
-// experiment switches of the env loop (defaults = what is shipped and measured)
-#ifndef PPG_TICKET_EARLY
-#define PPG_TICKET_EARLY 1  // draw the warp's next ticket while the current env is being finished
-#endif
-#ifndef PPG_PUSH_DEFER
-#define PPG_PUSH_DEFER 1    // hand an env to the observation kernel from the top of the next env (fence under the loads)
-#endif
 
 // shared-memory atomics by 32-bit shared address: one ATOMS / RED instruction instead of the generic-pointer atomicAdd's
 // address-space dispatch (~15 instructions per call in the SASS of the previous build)
@@ -780,6 +772,175 @@ __device__ __forceinline__ void queue_push(const StepParams& p, unsigned long lo
     st_volatile(p.queue + (pend - 1ULL), TAG(p.epoch, pend_env));
     pend = 0ULL;
   }
+}
+
+// ------------------------------------------------------------------------------------------------
+// the env loop of a persistent step warp (DESIGN.md §3.4-3.5); the variant's simulation runs between env_begin and
+// env_publish, its rows between env_publish and env_rows_done
+// ------------------------------------------------------------------------------------------------
+// Envs come from the ticket counter; after the first one lane 0 draws the warp's next ticket while the current env is still
+// being finished (env_publish: late enough that the schedule stays dynamic, early enough that the atomic's round trip is never
+// waited for).  Tickets are handed out in env order to warps that are running, so an env that waits for the publication of a
+// lower env (ECO's episode-end rows, the one-kernel step) always waits for a running warp.
+struct EnvLoop {
+  unsigned epoch;
+  int par;                  // epoch & 1: the parity of the count words this launch publishes
+  int n_blk, n_grp;         // 32-env blocks, 1024-env groups
+  int n_old_total[2];       // rows of the previous output
+  bool order;               // the kernel may take its envs out of index order (perm, static_first)
+  const int32_t* perm;      // ticket -> env: big envs first when the previous launch left an order (publish_begin), else index order
+  int env_next;             // lane 0: the warp's next env
+  unsigned long long q_slot, pubA, pubB;  // lane 0: the env's completion-queue slot and row-allocation atomics (env_publish)
+  unsigned long long pend;  // lane 0: completion-queue slot + 1 of the env whose hand-over is still owed (queue_push)
+  int pend_env;
+};
+
+// order: only for kernels in which no env ever waits for another one (publish_begin)
+__device__ __forceinline__ EnvLoop env_loop(const StepParams& p, bool order) {
+  EnvLoop L;
+  L.order = order;
+  L.epoch = p.epoch;
+  L.par = (int)(L.epoch & 1u);
+  L.n_blk = (p.B + 31) >> 5;
+  L.n_grp = (p.B + 1023) >> 10;
+  L.n_old_total[0] = p.totals[(L.par ^ 1) * 4 + 0];
+  L.n_old_total[1] = p.totals[(L.par ^ 1) * 4 + 1];
+  L.perm = (order && p.perm[L.par ^ 1] != nullptr && p.perm_tag[L.par ^ 1] == L.epoch - 1u) ? p.perm[L.par ^ 1] : nullptr;
+  L.env_next = 0;
+  L.pend = 0ULL;
+  L.pend_env = 0;
+  return L;
+}
+
+// lane 0: draws the warp's next env (first: the warp's first one).  static_first: the first ticket of a warp is its CTA index —
+// 2960 atomics on one address at kernel start cost the last warp ~7 us; the counter then hands out the tickets from min(grid, B) on.
+__device__ __forceinline__ void next_ticket(const StepParams& p, EnvLoop& L, bool first) {
+  const int t = !(L.order && p.static_first) ? (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base)
+                : first ? min((int)blockIdx.x, p.B) : min((int)gridDim.x, p.B) + (int)(atomicAdd(p.ticket, 1ULL) - p.ticket_base);
+  L.env_next = L.perm != nullptr && t < p.B ? L.perm[t] : t;
+}
+
+// Start of an env whose header and first list entries have been requested: its first old row (the previous launch published
+// how many rows every env needs now), the hand-over of the warp's previous env (its stores were issued a round trip ago, the
+// fence finds them acknowledged) and the mode (0 idle, 1 reset, 2 step).  Reset / idle envs know their counts up front
+// (`founders`, no births) and publish them before doing any work, so that later envs waiting for their newborn-row prefix
+// never wait for a reset.
+template <bool SPLIT>
+__device__ __forceinline__ int env_begin(const StepParams& p, EnvLoop& L, int env, unsigned state, const int founders[2], int old_base[2],
+                                         int next_live[2], int lane) {
+  if (!prefix_before(p.cntA[L.par ^ 1], p.sum1[L.par ^ 1], p.sum2[L.par ^ 1], 0, env, L.epoch - 1u, false, lane, old_base[0], old_base[1])) {
+    if (lane == 0) atomicOr(p.error, 2u);  // the host did not prepare the counts of the previous output
+  }
+  if (SPLIT) queue_push(p, L.pend, L.pend_env, lane);
+  const int mode = (state & ST_NEEDS_RESET) ? 1 : ((state & ST_IDLE) ? 0 : 2);
+  if (mode != 2) {
+    const int births[2] = {0, 0};
+    if (mode == 1) { next_live[0] = founders[0]; next_live[1] = founders[1]; }
+    publish_counts(p, env, L.par, L.epoch, next_live, births, L.n_blk, L.n_grp, L.n_old_total, lane);
+  }
+  return mode;
+}
+
+// After the simulation: four atomics back to back, nobody waits for them here — the warp's next env (`tickets`), this env's
+// slot in the completion queue and the two accumulators of the row allocation (results looked at in env_rows_done).
+// `big`: the big-env bound of publish_begin.
+template <bool SPLIT>
+__device__ __forceinline__ void env_publish(const StepParams& p, EnvLoop& L, int env, int mode, const int next_live[2], const int births[2],
+                                            int big, bool tickets, int lane) {
+  if (tickets && lane == 0) next_ticket(p, L, false);
+  L.q_slot = L.pubA = L.pubB = 0ULL;
+  if (SPLIT) L.q_slot = queue_reserve(p, lane);
+  if (mode == 2) publish_begin(p, env, L.par, L.epoch, next_live, births, lane, L.pubA, L.pubB, big);
+}
+
+// one-kernel step: the first newborn row of the env depends on the births of every env before it; by now (all other work of
+// the env is done) the predecessors have normally published theirs.  The two-kernel step never waits: the observation kernel
+// places the newborn rows (nb_info).
+__device__ __forceinline__ void newborn_base(const StepParams& p, const EnvLoop& L, int env, int lane, int new_base[2]) {
+  int nb0 = 0, nb1 = 0;
+  if (!prefix_before(p.cntB[L.par], p.sum1[L.par], p.sum2[L.par], 2, env, L.epoch, true, lane, nb0, nb1)) {
+    if (lane == 0) atomicOr(p.error, 1u);
+  }
+  new_base[0] = L.n_old_total[0] + nb0;
+  new_base[1] = L.n_old_total[1] + nb1;
+}
+
+// After the rows of a reset or stepped env: the rest of its publication, its newborn-row range and (two-kernel step) its image,
+// dumped before the caller un-writes the maps.
+template <bool SPLIT>
+__device__ __forceinline__ void env_rows_done(const StepParams& p, const EnvLoop& L, unsigned char* sbase, int env, int mode, bool keep,
+                                              const int old_base[2], const int n[2], const int births[2], const int new_base[2],
+                                              const int next_live[2], int lane) {
+  if (mode == 2) publish_end(p, env, L.par, L.epoch, next_live, births, L.n_blk, L.n_grp, L.n_old_total, lane, L.pubA, L.pubB);
+  if (lane < 2) {
+    const int nb = lane == 0 ? births[0] : births[1];
+    if (!SPLIT) p.new_off[lane][env] = nb > 0 ? (lane == 0 ? new_base[0] : new_base[1]) : 0;
+    p.new_cnt[lane][env] = nb;
+  }
+  if (SPLIT) dump_image(sbase, p, env, mode, keep, old_base, n, births, lane);
+}
+
+// an idle env: no rows, a header-only image
+template <bool SPLIT>
+__device__ __forceinline__ void env_idle(const StepParams& p, unsigned char* sbase, int env, const int old_base[2], int lane) {
+  if (lane < 2) {
+    p.new_off[lane][env] = 0;
+    p.new_cnt[lane][env] = 0;
+  }
+  const int none[2] = {0, 0};
+  if (SPLIT) dump_image(sbase, p, env, 0, false, old_base, none, none, lane);
+}
+
+// counters of one env-step behind PPG_STAT_*
+struct EnvStats {
+  unsigned starved[2], eaten, grass, fallback;
+  unsigned attempts;  // STAG's capture attempts, 0 elsewhere
+};
+
+// lane k adds statistic k (selects, no divergent switch)
+__device__ __forceinline__ void add_stats(const StepParams& p, int env, int mode, const int n[2], const int births[2], bool over, bool trunc,
+                                          unsigned step, const EnvStats& st, int lane) {
+  if (lane < PPG_N_STATS) {
+    unsigned add = 0;
+    if (mode == 2) {
+      add = lane == PPG_STAT_ENV_STEPS ? 1u : add;
+      add = lane == PPG_STAT_AGENT_STEPS ? (unsigned)(n[0] + n[1]) : add;
+      add = lane == PPG_STAT_EPISODES ? (unsigned)over : add;
+      add = lane == PPG_STAT_EPISODE_STEPS ? (over ? step : 0u) : add;
+      add = lane == PPG_STAT_BIRTHS_PRED ? (unsigned)births[0] : add;
+      add = lane == PPG_STAT_BIRTHS_PREY ? (unsigned)births[1] : add;
+      add = lane == PPG_STAT_STARVED_PRED ? st.starved[0] : add;
+      add = lane == PPG_STAT_STARVED_PREY ? st.starved[1] : add;
+      add = lane == PPG_STAT_EATEN_PREY ? st.eaten : add;
+      add = lane == PPG_STAT_GRASS_EATEN ? st.grass : add;
+      add = lane == PPG_STAT_TRUNCATED ? (unsigned)trunc : add;
+      add = lane == PPG_STAT_SPAWN_FALLBACK ? st.fallback : add;
+      add = lane == PPG_STAT_CAPTURE_ATTEMPTS ? st.attempts : add;
+    }
+    if (lane == PPG_STAT_ROWS_PRED) add = n[0] + births[0];
+    if (lane == PPG_STAT_ROWS_PREY) add = n[1] + births[1];
+    if (add) atomicAdd(p.counters + (size_t)env * PPG_N_STATS + lane, add);  // RED: nobody waits for the old value
+  }
+}
+
+// End of an env: its per-env outputs, then its hand-over to the observation kernel is owed (made from the top of the warp's next
+// env or after the loop, queue_push).  `count`: the agent counts the env reports, written unless `write_count` is false.
+template <bool SPLIT>
+__device__ __forceinline__ void env_end(const StepParams& p, EnvLoop& L, int env, int mode, const int n[2], const int births[2],
+                                        unsigned env_flags, const EnvHdr& h, long long t_env0, unsigned t_ns0, const int count[2],
+                                        bool write_count, int lane) {
+  if (lane == 0) {
+    p.env_cycles[env] = make_uint4((unsigned)(clock64() - t_env0), (unsigned)mode | ((unsigned)(births[0] + births[1]) << 8) | ((unsigned)(n[0] + n[1]) << 16), t_ns0, smid());
+    p.env_flags[env] = (uint8_t)env_flags;
+    p.env_status[env] = h.status;
+    p.env_step[env] = h.step;
+    if (write_count) {
+      p.env_count[2 * env] = count[0];
+      p.env_count[2 * env + 1] = count[1];
+    }
+  }
+  if (SPLIT && lane == 0) { L.pend = L.q_slot + 1ULL; L.pend_env = env; }
+  __syncwarp();
 }
 
 }  // namespace ppg

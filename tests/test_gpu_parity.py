@@ -34,9 +34,17 @@ def test_replay_4096_envs_300_steps():
     assert st["env_steps"] > 4096 * 250
 
 
-@pytest.mark.parametrize("mode", ["sparse", "dense", "additive", "kickback"])
-def test_reward_modes_crowded(mode):
+@pytest.mark.parametrize("mode,switches", [pytest.param(m, {}, id=m) for m in ("sparse", "dense", "additive", "kickback")] + [
+    # the one-kernel step's CTA-ganged warps and rows through the bulk-copy engine (DESIGN.md §4 experiment switches)
+    pytest.param("kickback", {"PPG_WARPS_PER_CTA": "4"}, id="kickback-warps4"),
+    pytest.param("dense", {"PPG_WARPS_PER_CTA": "8"}, id="dense-warps8"),
+    pytest.param("sparse", {"PPG_OBS_BULK": "1"}, id="sparse-bulk"),
+    pytest.param("additive", {"PPG_OBS_BULK": "1", "PPG_WARPS_PER_CTA": "4"}, id="additive-bulk-warps4"),
+])
+def test_reward_modes_crowded(mode, switches, monkeypatch):
     """crowded 6x6 world: births every step, blocked moves, co-located agents, spawn fallback draws"""
+    for k, v in switches.items():
+        monkeypatch.setenv(k, v)  # read when the handle is created
     cfg = make_config(CROWDED, reward_mode=mode, cap_live=(64, 64), seed=3)
     st = lockstep_parity(cfg, 256, 150, state_envs=(0, 17, 255))
     assert st["spawn_fallback"] > 0 and st["births_prey"] > 0 and st["truncated"] >= 0
